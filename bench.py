@@ -2,7 +2,7 @@
 """Headline benchmark: single-tile training rays/s (fwd + bwd + optimiser) of the ScaNeRF
 per-tile hot path at config/default.yaml shape, on N B200s (one tile per GPU, weak scaling).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One step = one pass of the hot path over one batch of 2^14 synthetic rays:
@@ -422,6 +422,42 @@ def bench_reference_drivers(cfg, steps=12):
         out["ratio"] = out["reference"]["ms_per_step"] / out["dropin"]["ms_per_step"]
     return out
 
+
+def dump_outputs(out_dir, timed_loss, cfg, dev, seed, batch, rows=1 << 20):
+    """--dump-outputs: writes <name>.npy (float32; row indices float64) so that two builds can be compared output for output.
+      loss.npy       the loss the last timed TileStep.step_device returned: what a caller of the timed path receives.
+      seeded_step.*  one more step_device on the last timed batch, by a tile built afresh from the benchmark's seed: its loss,
+                     the pose offsets, the decoder and a fixed, seeded sample of `rows` rows of the hash table and its Adam
+                     moments (GiBs in full at the headline size).
+    The timed tile's own parameters are not written: its backward accumulates with float atomics, whose order varies from run
+    to run, and the table's Adam (eps 1e-15) turns near-cancelling sums into updates of +-lr, so its state drifts apart between
+    two runs of one build within a few steps (B200, headline size, 2^20 sampled rows: after 1 step the table agrees within
+    1e-7, after 2 steps 2427 rows differ by up to 1e-4, after 30 steps most rows and every pose offset differ; the loss after
+    30 steps agrees within 1e-5 relative).  A step from the seeded state has the same inputs in every run."""
+    import numpy as np
+    import torch
+    step, _ = build_tile(cfg, dev, seed)
+    seeded_loss = step.step_device(*batch)
+    table = step.featureGrid.HE.features.detach()
+    flat = lambda t: t.reshape(-1, table.shape[-1])
+    n = flat(table).shape[0]
+    idx = np.sort(np.random.default_rng(0).choice(n, min(rows, n), replace=False))
+    idx_dev = torch.from_numpy(idx).to(table.device)
+    sel = lambda t: flat(t)[idx_dev]
+    arrays = {"loss": timed_loss, "seeded_step.loss": seeded_loss, "seeded_step.table_rows": idx.astype(np.float64),
+              "seeded_step.table": sel(table)}
+    opt = step.featureGrid_optimizer
+    if hasattr(opt, "params"):                                   # vdbAdam: [param, exp_avg, exp_avg_sq] per parameter
+        arrays["seeded_step.table_exp_avg"], arrays["seeded_step.table_exp_avg_sq"] = sel(opt.params[0][1]), sel(opt.params[0][2])
+    arrays["seeded_step.se3_refine"] = step.poses.se3_refine
+    for k, p in step.decoder.named_parameters():
+        arrays["seeded_step.decoder." + k] = p
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        if not isinstance(a, np.ndarray):
+            a = a.detach().float().cpu().numpy()
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
 # ----------------------------------------------------------------------------- main arm
 def main():
     ap = argparse.ArgumentParser()
@@ -433,9 +469,14 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-render", action="store_true")
     ap.add_argument("--no-variants", action="store_true", help="skip the warp-loss / C1 / reference-CUDA legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last timed step's loss, and what one step from the seeded tile computes "
+                         "on the last timed batch, to DIR/<name>.npy")
     args = ap.parse_args()
     cfg, name = WORKLOADS[args.workload], args.workload
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: the GPU path only (--impl ours)")
         return run_reference(args, cfg, name)
 
     import torch
@@ -443,6 +484,8 @@ def main():
     assert args.warmup >= 3, "timing rules: at least 3 warm-up steps"
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs: one GPU only (the tiles of a multi-GPU run train in an ADMM consensus)")
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (no CPU fallback in the product path)"
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
@@ -484,9 +527,11 @@ def main():
             sync_events.append((e0, e1))
         counter["i"] += 1
 
+    last_losses = []
+
     def run_device(batch):
         maybe_sync()
-        return [st.step_device(*b) for st, b in zip(steps, batch)]
+        last_losses[:] = [st.step_device(*b) for st, b in zip(steps, batch)]
 
     def run_e2e(batch):
         maybe_sync()
@@ -705,6 +750,8 @@ def main():
         line["cpu_baseline"] = {"value": rays / sec, "unit": "rays/s", "cores": cores, "kind": "port",
                                 "sample": f"{rays} rays x {cfg['S'] + cfg['S_bg']} samples of the same workload, fwd+bwd, "
                                           f"mean of {passes} passes ({passes * sec:.1f} s of CPU work)"}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last_losses[0], cfg, dev, rank, devb[-1])
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
