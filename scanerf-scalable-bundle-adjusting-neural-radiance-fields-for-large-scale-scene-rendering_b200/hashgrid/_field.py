@@ -4,6 +4,7 @@ autograd.Function over (features, decoder parameters, ray directions)."""
 import ctypes
 
 import torch
+from torch.utils.weak import WeakIdKeyDictionary
 
 import scanerf_b200_capi as capi
 from . import _gradmode
@@ -103,23 +104,26 @@ def decoder_apply(feats, rays_d, mask32, S, params, valid=None, ert=None):
     return DecoderFn.apply(feats, rays_d, mask32, S, valid, ert, *params)
 
 
-_small_levels_cache = {}
+# resolution tensor (by identity: the entry dies with the tensor) -> (its version counter when counted, count)
+_small_levels_cache = WeakIdKeyDictionary()
 SMALL_LEVEL_LOG2 = 22          # levels with at most this many grid vertices are reduced in one pass (tools/sweep_small_levels.py)
 
 
 def small_levels(resolution):
     """Number of leading levels whose grid has at most 2^22 vertices ((rx+1)(ry+1)(rz+1)): however large the hash table,
     such a level touches few entries, and the fused backward reduces it in one pass (snrf_field_encode_bwd_adam).
-    Read back from the device once per resolution tensor."""
-    key = (resolution.data_ptr(), tuple(resolution.shape))
-    n = _small_levels_cache.get(key)
-    if n is None:
-        r = resolution.detach().cpu().long() + 1
-        verts = r[:, 0] * r[:, 1] * r[:, 2]
-        n = 0
-        while n < verts.shape[0] and int(verts[n]) <= (1 << SMALL_LEVEL_LOG2):
-            n += 1
-        _small_levels_cache[key] = n
+    Read back from the device once per resolution tensor and in-place change of it."""
+    cacheable = not resolution.is_inference()          # (inference tensors have no version counter)
+    hit = _small_levels_cache.get(resolution) if cacheable else None
+    if hit is not None and hit[0] == resolution._version:
+        return hit[1]
+    r = resolution.detach().cpu().long() + 1
+    verts = r[:, 0] * r[:, 1] * r[:, 2]
+    n = 0
+    while n < verts.shape[0] and int(verts[n]) <= (1 << SMALL_LEVEL_LOG2):
+        n += 1
+    if cacheable:
+        _small_levels_cache[resolution] = (resolution._version, n)
     return n
 
 
