@@ -372,20 +372,9 @@ int snrf_bg_pts_inference_v2(const float* rays_o, const float* rays_d, const flo
                              const float* corners, const float* sizes, const int* resolution, const void* features_tables,
                              const float* params, float* diffuse, float* specular, float* alpha, int B, int S, int T,
                              int nb, void* stream);
-/* operand precision of the inference MLP: 1 (default) bf16x3 split, 0 plain bf16 */
-void snrf_infer_set_precision(int split);
-/* tuning hook: 128-sample tiles in flight per CTA for single-tile scenes (1 or 2, default 1: see csrc/infer.cu) */
-void snrf_infer_set_inflight(int tiles);
-/* tuning hook: tiles in flight per CTA of the single-tile decode pass (4 = default, 2 = the round-1 kernel) */
-void snrf_infer_set_decode_inflight(int n);
 /* tuning hook: log2 of the samples per chunk of the single-tile two-pass evaluation behind pts_inference / bg_pts_inference*
  * (20 .. 26): a chunk streams the table from HBM once, its scratch is 153 B per sample */
 void snrf_infer_set_chunk_log2(int bits);
-/* tuning hook: 1 (default) = the four-tile decode pass composes decoder layer 2 into its consumers (as snrf_decoder_set_fwd_fold) */
-void snrf_infer_set_fold(int on);
-/* tuning hook: 1 (default) = multi-pass paths (single-tile two-pass, multi-tile grouped), 0 = the fused kernel,
- * 2 = the grouped (compacting) path also for single-tile scenes */
-void snrf_infer_set_two_pass(int on);
 /* The multi-pass inference paths keep their scratch (features of one 4 Mi-sample chunk, <= 3.1 GB) in a private
  * stream-ordered pool between calls; this synchronises the device and returns that memory to the driver. */
 int snrf_infer_release_scratch(void);

@@ -64,7 +64,6 @@ template <bool SPLIT> constexpr int off_small() { return off_mask<SPLIT>() + 128
 template <bool SPLIT> constexpr int off_tiles() { return ((off_small<SPLIT>() + 64 + 1023) / 1024) * 1024; }
 template <bool SPLIT> constexpr int fwd_tiles() { return SPLIT ? 5 : 3; }     // operand tiles of one in-flight forward tile
 template <bool SPLIT> constexpr int fwd_smem() { return off_tiles<SPLIT>() + 2 * fwd_tiles<SPLIT>() * kTile + 1024; }   // two tiles in flight
-template <bool SPLIT> constexpr int fwd_smem_one() { return off_tiles<SPLIT>() + fwd_tiles<SPLIT>() * kTile + 1024; }   // one tile in flight
 template <bool SPLIT> constexpr int bwd_smem() { return off_tiles<SPLIT>() + 10 * kTile + 1024; }
 
 // TMEM columns: working accumulators, then (backward only) the persistent gradient accumulators

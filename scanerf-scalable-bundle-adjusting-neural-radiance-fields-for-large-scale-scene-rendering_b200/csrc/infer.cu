@@ -1,5 +1,5 @@
-// Render-side fused field evaluation: fp16 hash-table encode + decoder MLP on the tensor cores +
-// per-sample alpha and tile-overlap blending, one kernel, sm_100a.
+// Render-side field evaluation: fp16 hash-table encode + decoder MLP on the tensor cores + per-sample alpha and
+// tile-overlap blending, sm_100a.
 //
 // Replaces (behaviour, not code) the reference's per-thread-MLP kernels
 //   pts_inference        hashgrid/src/rendering_kernel.cu:467-621  (foreground, <= 4 overlapping tiles per sample)
@@ -7,12 +7,12 @@
 //   bg_pts_inference_v2  :1011-1171                                (background, one tile slot per call)
 // with get_multilevel_features<16> (:79-114) and Decoder::inference (hashgrid/include/decoder.h:169-218).
 //
-// The reference evaluates the 13 994-parameter MLP per thread out of global memory.  Here a CTA owns
-// 128 consecutive samples, walks the distinct tile ids present among them in ascending order (the
-// order in which the reference visits a sample's slots), stages that tile's weights once as bf16(x3)
-// operand tiles (decoder_core.cuh) and runs the layers as tcgen05 MMAs with the accumulators in TMEM;
-// rows whose sample does not belong to the current tile (or whose occupancy cell is empty) carry
-// zeros and are ignored in the epilogue.  Nothing but the three output rows per sample goes to HBM.
+// The reference evaluates the 13 994-parameter MLP per thread out of global memory.  Here the encode is a pass of
+// its own that writes level-major features, and the decoder runs on 128-sample tiles as tcgen05 MMAs with the
+// accumulators in TMEM and a scene tile's weights staged once per CTA as bf16x3 operand tiles (decoder_core.cuh).
+// launch() picks one of two implementations from the input:
+//   one scene tile (foreground, or one background slot)  -> launch_two_pass: every sample belongs to that tile;
+//   several scene tiles, or blended background          -> launch_work: the (sample, slot) pairs are grouped by tile.
 #include "decoder_core.cuh"
 #include <cuda_fp16.h>
 using namespace dec;
@@ -25,31 +25,6 @@ enum Mode { kFore = 0, kBackBlend = 1, kBackSlot = 2 };
 __device__ __forceinline__ uint32_t hash3(int x, int y, int z, uint32_t mask)
 {
     return (((uint32_t)x) ^ ((uint32_t)y * 2654435761u) ^ ((uint32_t)z * 805459861u)) & mask;
-}
-
-// Trilinear encode of 4 consecutive levels [l0, l0 + 4) from an fp16 table (rendering_kernel.cu:79-114): u in
-// [0,1]^3, v = u * (res - 1), corner order c = 4 dx + 2 dy + dz, accumulation in that order.  x[2 j], x[2 j + 1] =
-// the two features of level l0 + j.  (The four column groups of a row cover the 16 levels.)
-__device__ __forceinline__ void encode4(f3 u, const int* __restrict__ res, const __half2* __restrict__ table, uint32_t T, int l0, float* x)
-{
-    const uint32_t mask = T - 1u;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        const int l = l0 + j;
-        const float vx = u.x * (float)(res[3 * l] - 1), vy = u.y * (float)(res[3 * l + 1] - 1), vz = u.z * (float)(res[3 * l + 2] - 1);
-        const int ix = (int)vx, iy = (int)vy, iz = (int)vz;
-        const float ox = vx - (float)ix, oy = vy - (float)iy, oz = vz - (float)iz;
-        const __half2* tl = table + (size_t)l * T;
-        float2 f[8];
-#pragma unroll
-        for (int k = 0; k < 8; ++k) f[k] = __half22float2(__ldg(tl + hash3(ix + ((k >> 2) & 1), iy + ((k >> 1) & 1), iz + (k & 1), mask)));
-        const float ax = 1 - ox, ay = 1 - oy, az = 1 - oz;
-        const float w[8] = {ax * ay * az, ax * ay * oz, ax * oy * az, ax * oy * oz, ox * ay * az, ox * ay * oz, ox * oy * az, ox * oy * oz};
-        float a = 0.0f, b = 0.0f;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) { a += w[k] * f[k].x; b += w[k] * f[k].y; }
-        x[2 * j] = a; x[2 * j + 1] = b;
-    }
 }
 
 struct InferArgs {
@@ -68,195 +43,16 @@ struct InferArgs {
     uint32_t T;
 };
 
-template <bool SPLIT, int MODE, int NCG>
-__global__ void __launch_bounds__(kThreadsDec, 1)
-infer_kernel(InferArgs a, int num_tiles)
-{
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    unsigned char* smem = (unsigned char*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    __shared__ uint64_t bars[2];
-    __shared__ uint32_t tmem_slot;
-    __shared__ int next_ids[2];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-    if (warp == 0) umma::tmem_alloc<512>(&tmem_slot);
-    if (tid == 0) { umma::mbar_init(&bars[0], 1); umma::mbar_init(&bars[1], 1); umma::mbar_fence_init(); }
-    // NCG = 2 (a single scene tile: one set of weights, staged once): two 128-sample tiles in flight per CTA, so one
-    // group's table gathers and epilogues overlap the other's MMAs.  NCG = 4 (several scene tiles): one tile per CTA,
-    // weights re-staged whenever the walk reaches another scene tile.
-    if (NCG == 2) stage_all_weights<SPLIT>(smem, flat_params(a.params), nullptr, tid, kThreadsDec);
-    umma::fence_async_smem();
-    umma::tc_fence_before();
-    __syncthreads();
-    umma::tc_fence_after();
-    Ctx<SPLIT, NCG> c;
-    c.init(smem, bars, tmem_slot);
-    const int row = c.row, cg = c.cg;
-    int& next_id = next_ids[c.group];
-    unsigned char* T0 = smem + off_tiles<SPLIT>() + c.group * fwd_tiles<SPLIT>() * kTile;
-    unsigned char* T1 = T0 + kTile;
-    unsigned char* T2 = T1 + kTile;
-    unsigned char* LOa = SPLIT ? T2 + kTile : T1;
-    unsigned char* LOb = SPLIT ? LOa + kTile : T2;
-    const Tiles Tl{T0, T1, nullptr, T2, T1, nullptr, T2, nullptr, LOa, LOb};
-    int staged = NCG == 2 ? 0 : -1;
-    const long long total = (long long)a.B * a.S;
-    constexpr int NG = NCG == 2 ? 2 : 1;               // tiles in flight
-    constexpr int NX = 32 / NCG;                       // features per thread
-    const int shc = NCG == 4 ? cg - 2 : cg;            // SH chunk held by this thread (< 0: none)
-
-    for (int tile = NG * blockIdx.x + c.group; tile < num_tiles; tile += NG * gridDim.x) {
-        const long long n = (long long)tile * kRows + row;
-        const bool live = n < total;
-        const int ray = live ? (int)(n / a.S) : 0, k = live ? (int)(n % a.S) : 0;
-        short ids[kMaxPts] = {-1, -1, -1, -1};
-        float zv = -1.0f, step_len = 0.0f;
-        f3 o = mk3(0, 0, 0), d = mk3(0, 0, 1);
-        if (live) {
-            o = ld3(a.rays_o + 3 * (size_t)ray); d = ld3(a.rays_d + 3 * (size_t)ray);
-            zv = a.z_vals[n];
-            if (MODE == kFore) {
-                const short4 s4 = *reinterpret_cast<const short4*>(a.slots + (size_t)n * kMaxPts);
-                ids[0] = s4.x; ids[1] = s4.y; ids[2] = s4.z; ids[3] = s4.w;
-                step_len = a.dists[n];
-            } else {
-                const short* s = a.slots + (size_t)ray * kMaxPts;
-                if (MODE == kBackSlot) ids[0] = s[a.step];
-                else { ids[0] = s[0]; ids[1] = s[1]; ids[2] = s[2]; ids[3] = s[3]; }
-                step_len = (k == a.S - 1) ? 10000000.0f : a.z_vals[n + 1] - zv;
-            }
-            // slots after the first -1 are ignored (the reference breaks out of its slot loop there)
-#pragma unroll
-            for (int i = 1; i < kMaxPts; ++i) if (ids[i - 1] == -1) ids[i] = -1;
-        }
-        const f3 p = o + zv * d;
-        const f3 dn = d * rsqrtf(dot3(d, d));                 // normalize(): decoder.h:201, no epsilon
-        float sh[16];
-        if (shc >= 0) sh16(dn.x, dn.y, dn.z, sh);
-        const float dlen = sqrtf(dot3(d, d));
-        f3 acc_d = mk3(0, 0, 0), acc_s = mk3(0, 0, 0);
-        float acc_a = 0.0f, wsum = 0.0f;
-
-        int cur = -1;
-        while (true) {
-            // next tile id present in this CTA's samples, ascending
-            int mine = 0x7fffffff;
-#pragma unroll
-            for (int i = 0; i < kMaxPts; ++i) if (ids[i] > cur && ids[i] < mine) mine = ids[i];
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) mine = min(mine, __shfl_xor_sync(0xffffffffu, mine, off));
-            if (c.leader_warp && lane == 0) next_id = 0x7fffffff;
-            c.sync();
-            if (lane == 0 && mine != 0x7fffffff) atomicMin(&next_id, mine);
-            c.sync();
-            const int b = next_id;
-            c.sync();                                          // everyone has read next_id before it is reset
-            if (b == 0x7fffffff) break;
-            cur = b;
-            int slot = -1;
-#pragma unroll
-            for (int i = 0; i < kMaxPts; ++i) if (ids[i] == b && slot < 0) slot = i;
-            const bool member = slot >= 0;
-
-            // ---- geometry of this sample in tile b
-            const f3 bc = ld3(a.corners + 3 * b), bs = ld3(a.sizes + 3 * b);
-            f3 u = mk3(0, 0, 0);
-            float w = 0.0f;
-            bool active = false;
-            if (member) {
-                if (MODE == kFore) {
-                    const f3 q = mk3((p.x - bc.x) / bs.x, (p.y - bc.y) / bs.y, (p.z - bc.z) / bs.z);          // [0,1]
-                    const f3 dis = mk3((0.5f - fabsf(q.x - 0.5f)) * bs.x, (0.5f - fabsf(q.y - 0.5f)) * bs.y, (0.5f - fabsf(q.z - 0.5f)) * bs.z);
-                    if (dis.x != 0 && dis.z != 0) w = dis.x * dis.z;
-                    else if (dis.x != 0) w = dis.x;
-                    else if (dis.z != 0) w = dis.z;
-                    const int lx = a.grid_log2dim[3 * b], ly = a.grid_log2dim[3 * b + 1], lz = a.grid_log2dim[3 * b + 2];
-                    const int gx = min(max((int)(q.x * (float)(1 << lx)), 0), (1 << lx) - 1);
-                    const int gy = min(max((int)(q.y * (float)(1 << ly)), 0), (1 << ly) - 1);
-                    const int gz = min(max((int)(q.z * (float)(1 << lz)), 0), (1 << lz) - 1);
-                    active = a.grid_occ[a.grid_starts[b] + ((gx << (ly + lz)) | (gy << lz) | gz)] != 0;
-                    u = mk3(q.x * 0.5f + 0.25f, q.y * 0.5f + 0.25f, q.z * 0.5f + 0.25f);                       // [0.25, 0.75]
-                } else {
-                    // contraction of the 2x-normalised position (rendering_kernel.cu:1060-1095)
-                    float q[3] = {2.0f * (p.x - bc.x) / bs.x - 1.0f, 2.0f * (p.y - bc.y) / bs.y - 1.0f, 2.0f * (p.z - bc.z) / bs.z - 1.0f};
-                    float nrm = fabsf(q[0]);
-                    if (fabsf(q[1]) > nrm) nrm = fabsf(q[1]);
-                    if (fabsf(q[2]) > nrm) nrm = fabsf(q[2]);
-                    const float ratio = (2.0f - 1.0f / nrm) / nrm;
-                    u = mk3((q[0] * ratio + 2.0f) * 0.25f, (q[1] * ratio + 2.0f) * 0.25f, (q[2] * ratio + 2.0f) * 0.25f);
-                    w = MODE == kBackBlend ? a.blend[(size_t)ray * kMaxPts + slot] : 1.0f;
-                    active = true;
-                }
-            }
-            if (!c.any(active)) {                              // nobody needs the MLP for this tile
-                if (member) wsum += w;
-                continue;
-            }
-            if (staged != b) {
-                stage_all_weights<SPLIT>(smem, flat_params(a.params + (size_t)b * 13994), nullptr, tid, kThreadsDec);
-                staged = b;
-            }
-            float x[NX];                                       // this thread's features: levels (16 / NCG) cg ...
-            if (active) {
-#pragma unroll
-                for (int q = 0; q < NX / 8; ++q)
-                    encode4(u, a.resolution + (size_t)b * 48, a.tables + (size_t)b * 16 * a.T, a.T, (NX / 2) * cg + 4 * q, x + 8 * q);
-            } else {
-#pragma unroll
-                for (int j = 0; j < NX; ++j) x[j] = 0.0f;
-            }
-            store_input_row<SPLIT, NCG>(Tl, row, cg, x, sh + 8 * (shc & 1));
-            float head[10], zh[7];
-            forward_layers<SPLIT, false, NCG>(c, Tl, head, zh);
-            float zs[16];
-            if (cg == 0) {
-                umma::tmem_ld16(c.tmem + cDh + c.lane_addr, zs);
-                umma::tc_wait_ld();
-            }
-            if (active && cg == 0) {
-                // Decoder::inference activations (decoder.h:134-146): softplus without threshold, expf sigmoids
-                const float sigma = logf(1.0f + expf(zh[0]));
-                const f3 dif = mk3(1.0f / (1.0f + expf(-zh[1])), 1.0f / (1.0f + expf(-zh[2])), 1.0f / (1.0f + expf(-zh[3])));
-                const f3 tint = mk3(1.0f / (1.0f + expf(-zh[4])), 1.0f / (1.0f + expf(-zh[5])), 1.0f / (1.0f + expf(-zh[6])));
-                const f3 spe = mk3(tint.x / (1.0f + expf(-(zs[0] + c.bias[oB5 + 0]))), tint.y / (1.0f + expf(-(zs[1] + c.bias[oB5 + 1]))),
-                                   tint.z / (1.0f + expf(-(zs[2] + c.bias[oB5 + 2]))));
-                const float al = MODE == kFore ? 1.0f - expf(-1.0f * sigma * step_len * dlen) : 1.0f - expf(-1.0f * sigma * step_len);
-                acc_d = acc_d + (w * al) * dif;
-                acc_s = acc_s + (w * al) * spe;
-                acc_a += w * al;
-            }
-            if (member) wsum += w;
-        }
-        if (live && cg == 0) {
-            bool write = true;
-            if (MODE == kBackSlot) {
-                write = ids[0] != -1;                          // rays without a tile in this slot keep the caller's rows
-            } else if (wsum > 0) {
-                const float inv = 1.0f / wsum;                 // float3 /= float: multiply by the reciprocal
-                acc_d = acc_d * inv; acc_s = acc_s * inv; acc_a = acc_a * inv;
-            }
-            if (write) {
-                st3(a.out_diffuse + 3 * (size_t)n, acc_d);
-                st3(a.out_specular + 3 * (size_t)n, acc_s);
-                a.out_alpha[n] = acc_a;
-            }
-        }
-    }
-    umma::tc_fence_before();
-    __syncthreads();
-    if (warp == 0) umma::tmem_free<512>(tmem_slot);
-}
-
-
 // ------------------------------------------------------------------------------------------------------------------
-// Single-tile fast path: the same evaluation as infer_kernel, split into two passes over chunks of samples.
+// Single-tile path: three passes over chunks of samples.
 //   pass 0 (infer_geometry_kernel): per-sample table coordinate / weight / alpha scale / state, once.
 //   pass 1 (infer_encode_kernel): fp16 gathers, ONE LEVEL PER CTA ROW -> level-major features [16][Nc].
 //           The whole GPU walks one 64 MiB level slice at a time, which stays L2-resident: the table streams from HBM
-//           once per chunk, whereas the fused kernel (every level of a sample at once) pulls a 32-byte sector per
-//           corner from HBM -- ~4 KB per sample, the floor of a 1080p frame is then ~170 ms per pass.
-//   pass 2 (infer_decode_kernel): decoder layers on the tensor cores, two tiles in flight per CTA (no gathers here,
-//           so the L1 is not needed), inference activations, alpha, the reference's weight normalisation.
+//           once per chunk, whereas gathering every level of a sample at once pulls a 32-byte sector per corner from
+//           HBM -- ~4 KB per sample, the floor of a 1080p frame is then ~170 ms per pass.
+//   pass 2: decoder layers on the tensor cores (no gathers here, so the L1 is not needed), inference activations,
+//           alpha, the reference's weight normalisation.  infer_decode4_kernel (four tiles in flight per CTA) when
+//           S >= kMinS4, infer_decode_kernel (two tiles in flight) otherwise.
 // Per-sample state byte: 0 = write zeros (foreground sample outside occupied space), 1 = evaluate, 2 = leave the
 // caller's rows untouched (background ray without a tile in this slot).
 struct Geom {
@@ -353,8 +149,7 @@ infer_encode_kernel(InferArgs a, int Nc, const float4* __restrict__ uw, const un
 // Decoder layers + inference activations for one 128-row tile of precomputed level-major features (row r of this
 // thread at f0[level * stride]).  Returns false when no row of the tile is active (nothing evaluated); sigma / dif /
 // spe are valid for the active rows of column group 0.
-template <bool SPLIT>
-__device__ __forceinline__ bool eval_tile(Ctx<SPLIT, 2>& c, const Tiles& Tl, bool active, const float2* __restrict__ f0, size_t stride,
+__device__ __forceinline__ bool eval_tile(Ctx<true, 2>& c, const Tiles& Tl, bool active, const float2* __restrict__ f0, size_t stride,
                                           f3 d, float& sigma, f3& dif, f3& spe)
 {
     if (!c.any(active)) return false;
@@ -372,9 +167,9 @@ __device__ __forceinline__ bool eval_tile(Ctx<SPLIT, 2>& c, const Tiles& Tl, boo
 #pragma unroll
         for (int j = 0; j < 16; ++j) { x[j] = 0.0f; sh[j] = 0.0f; }
     }
-    store_input_row<SPLIT, 2>(Tl, c.row, cg, x, sh + 8 * cg);
+    store_input_row<true, 2>(Tl, c.row, cg, x, sh + 8 * cg);
     float head[10], zh[7];
-    forward_layers<SPLIT, false, 2>(c, Tl, head, zh);
+    forward_layers<true, false, 2>(c, Tl, head, zh);
     if (cg == 0) {
         float zs[16];
         umma::tmem_ld16(c.tmem + cDh + c.lane_addr, zs);
@@ -396,25 +191,25 @@ __device__ __forceinline__ bool eval_tile(Ctx<SPLIT, 2>& c, const Tiles& Tl, boo
     __shared__ uint64_t bars[2];                                                                                 \
     __shared__ uint32_t tmem_slot;                                                                               \
     const int tid = threadIdx.x, warp = tid >> 5;                                                                \
-    if (STAGE_PARAMS) stage_all_weights<SPLIT>(smem, flat_params(STAGE_PARAMS), nullptr, tid, kThreadsDec);       \
+    if (STAGE_PARAMS) stage_all_weights<true>(smem, flat_params(STAGE_PARAMS), nullptr, tid, kThreadsDec);        \
     if (warp == 0) umma::tmem_alloc<512>(&tmem_slot);                                                            \
     if (tid == 0) { umma::mbar_init(&bars[0], 1); umma::mbar_init(&bars[1], 1); umma::mbar_fence_init(); }       \
     umma::fence_async_smem();                                                                                    \
     umma::tc_fence_before();                                                                                     \
     __syncthreads();                                                                                             \
     umma::tc_fence_after();                                                                                      \
-    Ctx<SPLIT, 2> c;                                                                                             \
+    Ctx<true, 2> c;                                                                                              \
     c.init(smem, bars, tmem_slot);                                                                               \
     const int row = c.row, cg = c.cg;                                                                            \
-    unsigned char* T0 = smem + off_tiles<SPLIT>() + c.group * fwd_tiles<SPLIT>() * kTile;                        \
+    unsigned char* T0 = smem + off_tiles<true>() + c.group * fwd_tiles<true>() * kTile;                          \
     unsigned char* T1 = T0 + kTile;                                                                              \
     unsigned char* T2 = T1 + kTile;                                                                              \
-    unsigned char* LOa = SPLIT ? T2 + kTile : T1;                                                                \
-    unsigned char* LOb = SPLIT ? LOa + kTile : T2;                                                               \
+    unsigned char* LOa = T2 + kTile;                                                                             \
+    unsigned char* LOb = LOa + kTile;                                                                            \
     const Tiles Tl{T0, T1, nullptr, T2, T1, nullptr, T2, nullptr, LOa, LOb};                                     \
     (void)row; (void)cg;
 
-template <bool SPLIT, int MODE>
+template <int MODE>
 __global__ void __launch_bounds__(kThreadsDec, 1)
 infer_decode_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict__ feats_lm, const float2* __restrict__ aux,
                     const unsigned char* __restrict__ state, int num_tiles)
@@ -428,7 +223,7 @@ infer_decode_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict_
         float sigma = 0.0f;
         f3 dif = mk3(0, 0, 0), spe = mk3(0, 0, 0);
         const f3 d = active ? ld3(a.rays_d + 3 * (size_t)(n / a.S)) : mk3(0, 0, 1);
-        const bool done = eval_tile<SPLIT>(c, Tl, active, feats_lm + i, (size_t)Nc, d, sigma, dif, spe);
+        const bool done = eval_tile(c, Tl, active, feats_lm + i, (size_t)Nc, d, sigma, dif, spe);
         if (cg != 0) continue;
         if (done && active) {
             const float2 ws = aux[i];
@@ -455,8 +250,9 @@ infer_decode_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict_
 
 
 // The same decode pass with FOUR tiles in flight per CTA (decoder_core.cuh: forward_layers4 -- operand tiles in place, the
-// SH term of the first directional layer added per ray in fp32): one thread per sample row.  Needs a.S >= kMinS4.
-template <bool SPLIT, int MODE, bool FOLD>
+// SH term of the first directional layer added per ray in fp32, the activation-free layer 2 folded into its consumers):
+// one thread per sample row.  Needs a.S >= kMinS4.
+template <int MODE>
 __global__ void __launch_bounds__(kThreadsDec, 1)
 infer_decode4_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict__ feats_lm, const float2* __restrict__ aux,
                      const unsigned char* __restrict__ state, int num_tiles)
@@ -467,10 +263,10 @@ infer_decode4_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict
     __shared__ uint32_t tmem_slot;
     const int tid = threadIdx.x, warp = tid >> 5;
     const DecoderParams prm = flat_params(a.params);
-    stage_all_weights<SPLIT>(smem, prm, nullptr, tid, kThreadsDec);
-    float* w3sh = reinterpret_cast<float*>(smem + off_w3sh<SPLIT>());
+    stage_all_weights<true>(smem, prm, nullptr, tid, kThreadsDec);
+    float* w3sh = reinterpret_cast<float*>(smem + off_w3sh<true>());
     stage_w3sh(w3sh, prm, tid, kThreadsDec);
-    if (FOLD) stage_fold_weights4<SPLIT>(smem, prm, reinterpret_cast<float*>(smem + off_tiles4<SPLIT>()), tid, kThreadsDec);
+    stage_fold_weights4<true>(smem, prm, reinterpret_cast<float*>(smem + off_tiles4<true>()), tid, kThreadsDec);
     if (warp == 0) umma::tmem_alloc<512>(&tmem_slot);
     if (tid == 0) {
         for (int g = 0; g < kGroups4; ++g) umma::mbar_init(&bars[g], 1);
@@ -482,10 +278,10 @@ infer_decode4_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict
     umma::tc_fence_after();
     Ctx4 c;
     c.init(bars, tmem_slot);
-    unsigned char* P = smem + off_tiles4<SPLIT>() + c.group * 2 * kTile;
+    unsigned char* P = smem + off_tiles4<true>() + c.group * 2 * kTile;
     unsigned char* Q = P + kTile;
-    float* rb = reinterpret_cast<float*>(smem + off_raybias4<SPLIT>()) + c.group * kMaxRays4 * 64;
-    const float* bias = reinterpret_cast<const float*>(smem + off_bias<SPLIT>());
+    float* rb = reinterpret_cast<float*>(smem + off_raybias4<true>()) + c.group * kMaxRays4 * 64;
+    const float* bias = reinterpret_cast<const float*>(smem + off_bias<true>());
     const int row = c.row;
 
     for (int tile = kGroups4 * blockIdx.x + c.group; tile < num_tiles; tile += kGroups4 * gridDim.x) {
@@ -517,8 +313,8 @@ infer_decode4_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict
             const int nrays = (int)(last_n / a.S) - ray0 + 1;
             const int my_ray = active ? (int)(n / a.S) - ray0 : 0;
             float head[10], zh[7];
-            forward_layers4<SPLIT, FOLD>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
-                                         [&]() { ray_vectors4<true>(rb, w3sh, a.rays_d, ray0, nrays, c.gtid); });   // under the L1 MMAs
+            forward_layers4<true, true>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
+                                        [&]() { ray_vectors4<true>(rb, w3sh, a.rays_d, ray0, nrays, c.gtid); });   // under the L1 MMAs
             float zs[16];
             umma::tmem_ld16(c.tmem + c4Dh + c.lane_addr, zs);
             umma::tc_wait_ld();
@@ -713,7 +509,6 @@ work_encode_kernel(InferArgs a, Work w)
     }
 }
 
-template <bool SPLIT>
 __global__ void __launch_bounds__(kThreadsDec, 1)
 work_decode_kernel(InferArgs a, long long n0, Work w)
 {
@@ -726,7 +521,7 @@ work_decode_kernel(InferArgs a, long long n0, Work w)
         const int b = w.blk_tile[blk];
         if (b != staged) {                                     // CTA-uniform: both groups are done with the old weights
             __syncthreads();
-            stage_all_weights<SPLIT>(smem, flat_params(a.params + (size_t)b * 13994), nullptr, tid, kThreadsDec);
+            stage_all_weights<true>(smem, flat_params(a.params + (size_t)b * 13994), nullptr, tid, kThreadsDec);
             umma::fence_async_smem();
             __syncthreads();
             staged = b;
@@ -737,7 +532,7 @@ work_decode_kernel(InferArgs a, long long n0, Work w)
         float sigma = 0.0f;
         f3 dif = mk3(0, 0, 0), spe = mk3(0, 0, 0);
         const f3 d = active ? ld3(a.rays_d + 3 * (size_t)((n0 + i) / a.S)) : mk3(0, 0, 1);
-        const bool done = eval_tile<SPLIT>(c, Tl, active, w.feats + r, (size_t)w.max_rows, d, sigma, dif, spe);
+        const bool done = eval_tile(c, Tl, active, w.feats + r, (size_t)w.max_rows, d, sigma, dif, spe);
         if (done && active && cg == 0) {
             const float wgt = w.row_uw[r].w;
             const float wa = wgt * (1.0f - expf(-1.0f * sigma * w.row_scale[r]));
@@ -780,58 +575,21 @@ work_combine_kernel(InferArgs a, long long n0, int Nc, Work w)
     }
 }
 
-int g_chunk_log2 = 24;       // single-tile two-pass path: log2 of the samples per chunk (snrf_infer_set_chunk_log2; 22: 221 ms, 24: 218 ms per 1080p frame)
-int g_infer_fold = 1;        // the four-tile decode pass folds layer 2 into its consumers (decoder_core.cuh: forward_layers4<., FOLD>)
-int g_decode_inflight = 4;   // tiles in flight per CTA of the single-tile decode pass (4: infer_decode4_kernel, 2: infer_decode_kernel)
-int g_infer_split = 1;
-int g_infer_two_pass = 1;     // single-tile scenes: level-major encode pass + decoder pass (tuning hook)
-// Tiles in flight per CTA for single-tile scenes.  Measured on B200 (1920x1080, tools/render_one_frame.py): 1 tile in
-// flight 498 ms / frame, 2 tiles 765 ms -- the second tile's operand buffers take 80 KB away from the L1, and the table
-// gathers live on L1 hits between corners that share a sector.  Default 1; 2 stays selectable.
-int g_infer_inflight = 1;
+int g_chunk_log2 = 24;       // single-tile path: log2 of the samples per chunk (snrf_infer_set_chunk_log2; 22: 221 ms, 24: 218 ms per 1080p frame)
 
-// Scratch for the multi-pass paths comes from a private stream-ordered pool that keeps its memory across
+// Scratch for both paths comes from a private stream-ordered pool that keeps its memory across
 // synchronisations (the default pool hands it back to the driver at every sync; re-mapping 3 GB per call costs tens of
 // milliseconds).  snrf_infer_release_scratch() trims it.
 inline cudaError_t scratch_alloc(void** ptr, size_t bytes, cudaStream_t s) { return snrf_scratch_alloc(ptr, bytes, s); }
 
-template <int MODE, int NCG>
-int launch_ncg(const InferArgs& a, void* stream, const char* name)
-{
-    // shared memory not used for operand tiles stays L1: the table gathers need it (x-adjacent corners share sectors)
-    constexpr int smem_t = NCG == 2 ? fwd_smem<true>() : fwd_smem_one<true>();
-    constexpr int smem_f = NCG == 2 ? fwd_smem<false>() : fwd_smem_one<false>();
-    static bool configured = false;
-    if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(infer_kernel<true, MODE, NCG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_t);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_kernel<false, MODE, NCG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_f);
-        if (e != cudaSuccess) { snrf_set_error("%s: %s", name, cudaGetErrorString(e)); return (int)e; }
-        configured = true;
-    }
-    const long long total = (long long)a.B * a.S;
-    const int num_tiles = snrf_div_up(total, kRows);
-    const int per_cta = NCG == 2 ? 2 : 1;
-    cudaStream_t s = (cudaStream_t)stream;
-    int grid = snrf_sm_count();
-    if (grid > (num_tiles + per_cta - 1) / per_cta) grid = (num_tiles + per_cta - 1) / per_cta;
-    if (g_infer_split) infer_kernel<true, MODE, NCG><<<grid, kThreadsDec, smem_t, s>>>(a, num_tiles);
-    else infer_kernel<false, MODE, NCG><<<grid, kThreadsDec, smem_f, s>>>(a, num_tiles);
-    SNRF_RETURN_LAUNCH(name);
-}
-
-
-// single-tile fast path driver: chunks of samples, scratch from the stream-ordered allocator
+// single-tile driver: chunks of samples, scratch from the stream-ordered allocator
 template <int MODE>
 int launch_two_pass(const InferArgs& a, void* stream, const char* name)
 {
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(infer_decode_kernel<true, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<true>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode_kernel<false, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<false>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode4_kernel<true, MODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd4_smem<true>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode4_kernel<false, MODE, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd4_smem<false>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode4_kernel<true, MODE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd4_smem<true>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode4_kernel<false, MODE, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd4_smem<false>());
+        cudaError_t e = cudaFuncSetAttribute(infer_decode_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<true>());
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(infer_decode4_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd4_smem<true>());
         if (e != cudaSuccess) { snrf_set_error("%s: %s", name, cudaGetErrorString(e)); return (int)e; }
         configured = true;
     }
@@ -859,20 +617,13 @@ int launch_two_pass(const InferArgs& a, void* stream, const char* name)
         infer_encode_kernel<<<dim3(gx, 16), 256, 0, s>>>(a, Nc, uw, state, feats);
         const int num_tiles = snrf_div_up(Nc, kRows);
         int grid = sms;
-        if (g_decode_inflight == 4 && a.S >= kMinS4) {           // four tiles in flight per CTA
+        if (a.S >= kMinS4) {                                     // four tiles in flight per CTA
             if (grid > (num_tiles + 3) / 4) grid = (num_tiles + 3) / 4;
-            if (g_infer_fold) {
-                if (g_infer_split) infer_decode4_kernel<true, MODE, true><<<grid, kThreadsDec, fwd4_smem<true>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
-                else infer_decode4_kernel<false, MODE, true><<<grid, kThreadsDec, fwd4_smem<false>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
-            } else {
-                if (g_infer_split) infer_decode4_kernel<true, MODE, false><<<grid, kThreadsDec, fwd4_smem<true>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
-                else infer_decode4_kernel<false, MODE, false><<<grid, kThreadsDec, fwd4_smem<false>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
-            }
+            infer_decode4_kernel<MODE><<<grid, kThreadsDec, fwd4_smem<true>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
             continue;
         }
         if (grid > (num_tiles + 1) / 2) grid = (num_tiles + 1) / 2;
-        if (g_infer_split) infer_decode_kernel<true, MODE><<<grid, kThreadsDec, fwd_smem<true>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
-        else infer_decode_kernel<false, MODE><<<grid, kThreadsDec, fwd_smem<false>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
+        infer_decode_kernel<MODE><<<grid, kThreadsDec, fwd_smem<true>(), s>>>(a, n0, Nc, feats, aux, state, num_tiles);
     }
     e = cudaGetLastError();
     cudaFreeAsync(scratch, s);
@@ -886,8 +637,7 @@ int launch_work(const InferArgs& a, int nb, void* stream, const char* name)
 {
     static bool configured = false;
     if (!configured) {
-        cudaError_t e = cudaFuncSetAttribute(work_decode_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<true>());
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(work_decode_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<false>());
+        const cudaError_t e = cudaFuncSetAttribute(work_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, fwd_smem<true>());
         if (e != cudaSuccess) { snrf_set_error("%s: %s", name, cudaGetErrorString(e)); return (int)e; }
         configured = true;
     }
@@ -928,8 +678,7 @@ int launch_work(const InferArgs& a, int nb, void* stream, const char* name)
         int gx = snrf_div_up((long long)Nc * slots, 256);
         if (gx > sms * 32) gx = sms * 32;
         work_encode_kernel<<<dim3(gx, 16), 256, 0, s>>>(a, w);
-        if (g_infer_split) work_decode_kernel<true><<<sms, kThreadsDec, fwd_smem<true>(), s>>>(a, n0, w);
-        else work_decode_kernel<false><<<sms, kThreadsDec, fwd_smem<false>(), s>>>(a, n0, w);
+        work_decode_kernel<<<sms, kThreadsDec, fwd_smem<true>(), s>>>(a, n0, w);
         work_combine_kernel<MODE><<<gp < sms * 32 ? gp : sms * 32, 256, 0, s>>>(a, n0, Nc, w);
     }
     if (e == cudaSuccess) e = cudaGetLastError();
@@ -942,22 +691,14 @@ int launch_work(const InferArgs& a, int nb, void* stream, const char* name)
 template <int MODE>
 int launch(const InferArgs& a, int nb, void* stream, const char* name)
 {
-    if (g_infer_two_pass) return (nb == 1 && MODE != kBackBlend && g_infer_two_pass != 2) ? launch_two_pass<MODE>(a, stream, name) : launch_work<MODE>(a, nb, stream, name);
-    return (nb == 1 && g_infer_inflight == 2) ? launch_ncg<MODE, 2>(a, stream, name) : launch_ncg<MODE, 4>(a, stream, name);
+    return (nb == 1 && MODE != kBackBlend) ? launch_two_pass<MODE>(a, stream, name) : launch_work<MODE>(a, nb, stream, name);
 }
 
 }  // namespace
 
 // ------------------------------- C ABI --------------------------------------
-// tiles in flight per CTA of the single-tile decode pass: 4 (default) or 2 (round-1 kernel)
-SNRF_API void snrf_infer_set_decode_inflight(int n) { g_decode_inflight = n == 2 ? 2 : 4; }
-// tuning hook: log2 of the samples per chunk of the single-tile two-pass path (20 .. 26; scratch = 153 B per sample of a chunk)
+// tuning hook: log2 of the samples per chunk of the single-tile path (20 .. 26; scratch = 153 B per sample of a chunk)
 SNRF_API void snrf_infer_set_chunk_log2(int bits) { g_chunk_log2 = bits < 20 ? 20 : (bits > 26 ? 26 : bits); }
-// tuning hook: 1 (default) = the four-tile decode pass composes layer 2 into its consumers (four dependent stages per tile)
-SNRF_API void snrf_infer_set_fold(int on) { g_infer_fold = on ? 1 : 0; }
-SNRF_API void snrf_infer_set_precision(int split) { g_infer_split = split ? 1 : 0; }
-SNRF_API void snrf_infer_set_inflight(int tiles) { g_infer_inflight = tiles == 2 ? 2 : 1; }
-SNRF_API void snrf_infer_set_two_pass(int on) { g_infer_two_pass = on == 2 ? 2 : (on ? 1 : 0); }
 SNRF_API int snrf_infer_release_scratch(void) { return snrf_scratch_release(); }
 
 SNRF_API int snrf_pts_inference(const float* rays_o, const float* rays_d, const float* z_vals, const float* dists,

@@ -1,7 +1,7 @@
 """GPU: edge cases of the operator surface -- empty batches (every op is a no-op and raises nothing),
-ragged sizes (sample counts that are not multiples of the 128-row decode tile or of a warp), the two
-implementations of the field evaluation against each other on a ragged multi-tile batch, argument
-validation (dtype / device / shape errors are raised on the host, before any launch)."""
+ragged sizes (sample counts that are not multiples of a warp; the field evaluation's ragged batches are
+cases of test_render_gpu.py::test_pts_inference_against_cpu_restatement), argument validation
+(dtype / device / shape errors are raised on the host, before any launch)."""
 import numpy as np
 import pytest
 import torch
@@ -11,7 +11,6 @@ from test_render_gpu import dev, make_rays, make_scene
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-MISS = 1e7
 
 
 def z(*shape, dtype=torch.float32):
@@ -55,65 +54,22 @@ def test_empty_batches_are_noops():
     torch.cuda.synchronize()
 
 
-def _field_inputs(nb, B, S, seed):
-    """A ragged foreground batch: samples spread over the tiles, some unassigned (-1), some in two tiles."""
-    sc = dev(make_scene(nb, seed=seed))
-    o, d = (t.to(DEV) for t in make_rays(B, seed))
-    g = torch.Generator().manual_seed(seed)
-    zv = (torch.rand(B, S, generator=g) * 6.0).sort(-1)[0].to(DEV).contiguous()
-    di = (torch.rand(B, S, generator=g) * 0.1 + 0.01).to(DEV)
-    from hashgrid.lib import HASHGRID as H
-    isect = torch.full((B, nb, 2), MISS, device=DEV)
-    H.ray_block_intersection(o, d, sc["corners"], sc["sizes"], isect)
-    bi = torch.full((B, S, 4), -1, dtype=torch.int16, device=DEV)
-    H.prepare_points(zv, torch.ones(B, 1, dtype=torch.bool, device=DEV), isect, bi)
-    return sc, o, d, zv, di, bi
-
-
-@pytest.mark.parametrize("nb,B,S", [(1, 37, 19), (3, 211, 7), (3, 1, 1), (2, 130, 128)])
-def test_grouped_and_fused_field_evaluation_agree_on_ragged_batches(nb, B, S):
-    """B * S is not a multiple of the 128-row decode tile / 256-row block; both implementations must write
-    every sample (zeros where no tile is assigned) and agree to fp32 rounding of the slot sum."""
-    load_pkg()
-    import scanerf_b200_capi as capi
-    from hashgrid.lib import HASHGRID as H
-    sc, o, d, zv, di, bi = _field_inputs(nb, B, S, 11 + nb)
-    res = {}
-    for name, flag in (("grouped", 1), ("fused", 0)):
-        capi.lib().snrf_infer_set_two_pass(capi.c_int(flag))
-        outs = [torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 1), 7.0, device=DEV)]
-        H.pts_inference(o, d, zv, di, bi, sc["tables"], sc["params"], sc["res"], sc["occ"], sc["starts"], sc["l2d"], sc["corners"],
-                        sc["sizes"], *outs)
-        torch.cuda.synchronize()
-        res[name] = outs
-    capi.lib().snrf_infer_set_two_pass(capi.c_int(1))
-    for a, b in zip(res["grouped"], res["fused"]):
-        assert bool((a != 7.0).all()), "every sample row is written"
-        assert float((a - b).abs().max()) < 2e-6
-    none = (bi[..., 0] == -1)
-    assert float(res["grouped"][2][none].abs().max() if none.any() else 0.0) == 0.0, "unassigned samples give zeros"
-
-
 def test_background_slot_leaves_rows_of_rays_without_a_tile():
     load_pkg()
-    import scanerf_b200_capi as capi
     from hashgrid.lib import HASHGRID as H
     nb, B, S = 3, 77, 13
     sc = dev(make_scene(nb, seed=5))
     o, d = (t.to(DEV) for t in make_rays(B, 9))
     zv = (torch.rand(B, S, generator=torch.Generator().manual_seed(1)) * 30 + 1).sort(-1)[0].to(DEV).contiguous()
     ids = torch.randint(-1, nb, (B, 4), generator=torch.Generator().manual_seed(2)).to(torch.int16).to(DEV)
-    for flag in (1, 0):
-        capi.lib().snrf_infer_set_two_pass(capi.c_int(flag))
-        outs = [torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 1), 7.0, device=DEV)]
-        H.bg_pts_inference_v2(o, d, zv, ids, 2, sc["corners"], sc["sizes"], sc["res"], sc["tables"], sc["params"], *outs)
-        torch.cuda.synchronize()
-        skip = ids[:, 2] == -1
-        assert skip.any() and (~skip).any()
-        assert bool((outs[2][skip] == 7.0).all()) and bool((outs[0][skip] == 7.0).all())
-        assert bool((outs[2][~skip] != 7.0).all())
-        assert bool(((outs[2][~skip] >= 0) & (outs[2][~skip] <= 1)).all())
-    capi.lib().snrf_infer_set_two_pass(capi.c_int(1))
+    outs = [torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 1), 7.0, device=DEV)]
+    H.bg_pts_inference_v2(o, d, zv, ids, 2, sc["corners"], sc["sizes"], sc["res"], sc["tables"], sc["params"], *outs)
+    torch.cuda.synchronize()
+    skip = ids[:, 2] == -1
+    assert skip.any() and (~skip).any()
+    assert bool((outs[2][skip] == 7.0).all()) and bool((outs[0][skip] == 7.0).all())
+    assert bool((outs[2][~skip] != 7.0).all())
+    assert bool(((outs[2][~skip] >= 0) & (outs[2][~skip] <= 1)).all())
 
 
 def test_accumulate_ragged_sample_counts():

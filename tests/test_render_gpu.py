@@ -1,7 +1,7 @@
 """GPU: the multi-tile inference renderer ops (csrc/render.cu, csrc/infer.cu behind the reference's
 HASHGRID operator names) against the UNMODIFIED reference extension rebuilt into
 oracle/_ref/HASHGRID.so, stage by stage on the same inputs, plus CPU restatements of the simple
-stages and of the fused field evaluation (C hash-encode oracle + torch decoder restatement).
+stages and of the field evaluation in its three modes (C hash-encode oracle + torch decoder restatement).
 Bars: tile ids / tracing state / sample-to-tile assignment bit-exact; depths 1e-6; per-sample
 colours and alpha 1e-4 (the north star's composited-RGB tolerance)."""
 import numpy as np
@@ -60,21 +60,6 @@ def both(fn_name, ours, ref, make_args):
     return a, (b if ref is not None else None)
 
 
-@pytest.fixture(params=[(1, 1), (1, 0), (0, 1)], ids=["grouped", "grouped-unfolded", "fused"])
-def infer_path(request):
-    """The implementations of the field evaluation behind pts_inference / bg_pts_inference*: the grouped
-    multi-pass path (default; its four-tile decode pass with decoder layer 2 folded into its consumers, or not:
-    snrf_infer_set_fold) and the single fused kernel (snrf_infer_set_two_pass(0))."""
-    load_pkg()
-    import scanerf_b200_capi as capi
-    two_pass, fold = request.param
-    capi.lib().snrf_infer_set_two_pass(capi.c_int(two_pass))
-    capi.lib().snrf_infer_set_fold(capi.c_int(fold))
-    yield two_pass
-    capi.lib().snrf_infer_set_two_pass(capi.c_int(1))
-    capi.lib().snrf_infer_set_fold(capi.c_int(1))
-
-
 def _ops():
     load_pkg()
     from hashgrid.lib import HASHGRID as ours
@@ -82,7 +67,7 @@ def _ops():
 
 
 @pytest.mark.parametrize("nb,B", [(1, 500), (3, 6000)])
-def test_render_pipeline_stage_by_stage(nb, B, infer_path):
+def test_render_pipeline_stage_by_stage(nb, B):
     ours, ref = _ops()
     sc = dev(make_scene(nb))
     o, d = (t.to(DEV) for t in make_rays(B, nb * B))
@@ -208,38 +193,158 @@ def test_render_pipeline_stage_by_stage(nb, B, infer_path):
         assert torch.equal(a[6], r[6]) and torch.allclose(a[7], r[7], rtol=1e-6, atol=1e-6)
 
 
-def test_pts_inference_against_cpu_restatement(infer_path):
-    """Single tile, every cell occupied: per-sample outputs = alpha * decoder(encode(u)) with the
-    renderer's conventions (u = q/2 + 0.25, fp16 table, normalised d, no level mask)."""
+def _fma(a, b, c):
+    """float32 a * b + c with one rounding, as the kernels' contracted expressions (the product is exact in float64)."""
+    return (np.asarray(a, np.float64) * b + c).astype(np.float32)
+
+
+def _encode(u, table, res):
+    """The C oracle's hash encode (hash_encode_fwd) of table coordinates u [N,3] float32 -> [N,32], one level at a time
+    in the box [0, res - 1]: the oracle then locates the cell at v = u * (res - 1) as the kernels form it.  (Its
+    background mapping (x + 2) / 4 cannot hold every float32 u, and with these tables one ulp of u moves the
+    specular head by up to 1e-3.)"""
+    feats = np.empty((u.shape[0], 16, 2), np.float32)
+    for l in range(16):
+        r = res[l].astype(np.float32) - 1
+        feats[:, l:l + 1] = on.hash_encode_fwd(u * r, table[l:l + 1], res[l:l + 1], corner=np.zeros(3, np.float32), size=r)
+    return feats.reshape(-1, 32)
+
+
+def field_restatement(mode, sc, o, d, z, dist, slots, blend=None, step=0):
+    """CPU restatement of the field evaluation of pts_inference ("fore", rendering_kernel.cu:467-621),
+    bg_pts_inference ("blend", :871-1008) and bg_pts_inference_v2 ("slot", :1011-1171) on host tensors.
+
+    A sample visits its tile slots in order up to the first -1, each distinct tile once.  Foreground:
+    q = (p - corner) / size, face weight w from dis = (0.5 - |q - 0.5|) * size (dis.x * dis.z, else dis.x,
+    else dis.z, whichever are non-zero), added to the weight sum even where the occupancy cell is empty; the
+    field is evaluated only where it is set, at u = q / 2 + 0.25, and alpha = 1 - exp(-sigma * dist * |d|).
+    Background: contraction of the 2x-normalised position, w = the blend weight ("slot": the one slot `step`,
+    w = 1), alpha = 1 - exp(-sigma * step length), the last step 1e7, no |d|.  The sums are normalised by the
+    weight sum where it is positive, except for "slot".  The geometry is float32 in the kernel's order (with its
+    fused multiply-adds), the encode is the C oracle on the fp16 table (_encode), the decoder torch_ref.shallow_mlp
+    in float64.
+
+    Returns diffuse [B,S,3], specular [B,S,3], alpha [B,S,1] (float64), `keep` [B,S] (rows the op leaves
+    alone: "slot" rays without a tile in that slot) and `near` [B,S] (foreground samples within 1e-4 of a face of an
+    occupancy cell or of one of their tiles, where the kernel's FMA contraction may decide differently)."""
+    B, S = z.shape
+    N = B * S
+    f32 = lambda t: t.numpy().astype(np.float32)
+    o, d, z = f32(o), f32(d), f32(z)
+    corners, sizes = f32(sc["corners"]), f32(sc["sizes"])
+    ray, k = np.repeat(np.arange(B), S), np.tile(np.arange(S), B)
+    p = _fma(z.reshape(N, 1), d[ray], o[ray])
+    if mode == "fore":
+        ids = slots.numpy().reshape(N, 4).astype(np.int64)
+        scale = f32(dist).reshape(N) * np.sqrt((d[ray] * d[ray]).sum(-1))
+    else:
+        ids = slots.numpy().astype(np.int64)[ray]
+        if mode == "slot":
+            ids = np.concatenate([ids[:, step:step + 1], np.full((N, 3), -1)], 1)
+        znext = np.concatenate([z[:, 1:], z[:, -1:]], 1).reshape(N)
+        scale = np.where(k == S - 1, np.float32(1e7), znext - z.reshape(N))
+    wsum, acc, near = np.zeros(N), np.zeros((N, 7)), np.zeros(N, bool)
+    open_ = np.ones(N, bool)
+    for s in range(4):
+        open_ &= ids[:, s] >= 0
+        first = open_.copy()
+        for j in range(s):
+            first &= ids[:, j] != ids[:, s]
+        for b in np.unique(ids[first, s]):
+            n = np.nonzero(first & (ids[:, s] == b))[0]
+            bc, bs = corners[b], sizes[b]
+            if mode == "fore":
+                q = (p[n] - bc) / bs
+                dis = (np.float32(0.5) - np.abs(q - np.float32(0.5))) * bs
+                w = np.where((dis[:, 0] != 0) & (dis[:, 2] != 0), dis[:, 0] * dis[:, 2], np.where(dis[:, 0] != 0, dis[:, 0], dis[:, 2]))
+                l2 = sc["l2d"][b].numpy().astype(np.int64)
+                cell = q * (1 << l2).astype(np.float32)
+                g = np.clip(cell.astype(np.int64), 0, (1 << l2) - 1)
+                active = sc["occ"].numpy()[int(sc["starts"][b]) + ((g[:, 0] << (l2[1] + l2[2])) | (g[:, 1] << l2[2]) | g[:, 2])]
+                near[n] |= (np.abs(cell - np.round(cell)) * (bs / (1 << l2)) < 1e-4).any(-1)
+                u = _fma(q, 0.5, 0.25)
+            else:
+                q = np.float32(2) * (p[n] - bc) / bs - np.float32(1)
+                nrm = np.abs(q).max(-1, keepdims=True)
+                assert (nrm > 1).all(), "background samples lie outside the tile (u in [0, 1])"
+                u = _fma(q, (np.float32(2) - np.float32(1) / nrm) / nrm, 2) * np.float32(0.25)
+                w = blend.numpy()[ray[n], s] if mode == "blend" else np.ones(len(n), np.float32)
+                active = np.ones(len(n), bool)
+            wsum[n] += w
+            if not active.any():
+                continue
+            na = n[active]
+            feats = _encode(u[active], sc["tables"][b].float().numpy(), sc["res"][b].numpy())
+            mlp = {key: v.double() for key, v in sc["mlps"][b].items()}
+            h = tr.shallow_mlp(mlp, torch.from_numpy(feats).double(), torch.from_numpy(d[ray[na]]).double(),
+                               torch.ones(32, dtype=torch.float64))
+            wa = torch.from_numpy(w[active]).double() * (1 - torch.exp(-h["sigma"][:, 0] * torch.from_numpy(scale[na]).double()))
+            acc[na] += torch.cat([wa[:, None] * h["diffuse"], wa[:, None] * h["tint"] * h["specular"], wa[:, None]], 1).numpy()
+    if mode != "slot":
+        pos = wsum > 0
+        acc[pos] /= wsum[pos, None]
+    keep = ids[:, 0] < 0 if mode == "slot" else np.zeros(N, bool)
+    return acc[:, :3].reshape(B, S, 3), acc[:, 3:6].reshape(B, S, 3), acc[:, 6:].reshape(B, S, 1), keep.reshape(B, S), near.reshape(B, S)
+
+
+@pytest.mark.parametrize("nb,B,S", [(1, 64, 16), (1, 300, 7), (1, 37, 19), (3, 211, 7), (3, 1, 1), (2, 130, 128)])
+@pytest.mark.parametrize("mode", ["fore", "blend", "slot"])
+def test_pts_inference_against_cpu_restatement(mode, nb, B, S):
+    """pts_inference / bg_pts_inference / bg_pts_inference_v2 against field_restatement, per sample within 1e-4.
+    One scene tile takes the single-tile passes (decode with four tiles in flight for S >= 16, two below; blended
+    background excepted), several take the grouped path; B * S is not a multiple of the 128-row decode tile or the
+    256-row block.  Every sample row is written (over a sentinel) except those the op leaves alone, and
+    unassigned foreground samples give exact zeros."""
     ours, _ = _ops()
-    sc = make_scene(1, T=2 ** 12, seed=3)
-    B, S = 64, 16
-    g = torch.Generator().manual_seed(5)
-    o = sc["corners"][0] + sc["sizes"][0] * (0.2 + 0.6 * torch.rand(B, 3, generator=g))
-    d = torch.nn.functional.normalize(torch.randn(B, 3, generator=g), dim=-1) * 0.8
-    z = (torch.rand(B, S, generator=g) * 1.5).sort(-1)[0].contiguous()
-    dist = torch.full((B, S), 0.07)
-    bi = torch.full((B, S, 4), -1, dtype=torch.int16)
-    bi[..., 0] = 0
-    occ = torch.ones(sc["n_cells"], dtype=torch.bool)
-    outs = [torch.zeros(B, S, 3, device=DEV), torch.zeros(B, S, 3, device=DEV), torch.zeros(B, S, 1, device=DEV)]
-    ours.pts_inference(o.to(DEV), d.to(DEV), z.to(DEV), dist.to(DEV), bi.to(DEV), sc["tables"].to(DEV), sc["params"].to(DEV), sc["res"].to(DEV),
-                       occ.to(DEV), sc["starts"].to(DEV), sc["l2d"].to(DEV), sc["corners"].to(DEV), sc["sizes"].to(DEV), *outs)
-    p = o[:, None] + z[..., None] * d[:, None]
-    q = (p - sc["corners"][0]) / sc["sizes"][0]
-    inside = ((q > 0.02) & (q < 0.98)).all(-1)
-    cont = (2 * q - 1).reshape(-1, 3).numpy().astype(np.float32)           # (cont + 2) / 4 = q / 2 + 0.25
-    feats = on.hash_encode_fwd(cont, sc["tables"][0].float().numpy(), sc["res"][0].numpy())
-    dirs = d[:, None].expand(B, S, 3).reshape(-1, 3)
-    heads = tr.shallow_mlp(sc["mlps"][0], torch.from_numpy(feats).reshape(-1, 32), dirs, torch.ones(32))
-    alpha = 1 - torch.exp(-heads["sigma"][:, 0] * dist.reshape(-1) * dirs.norm(dim=-1))
-    want_d = (alpha[:, None] * heads["diffuse"]).reshape(B, S, 3)
-    want_s = (alpha[:, None] * heads["tint"] * heads["specular"]).reshape(B, S, 3)
-    m = inside
-    assert m.sum() > B * S // 2
-    assert float((outs[2].cpu()[..., 0][m] - alpha.reshape(B, S)[m]).abs().max()) < 1e-4
-    assert float((outs[0].cpu()[m] - want_d[m]).abs().max()) < 1e-4
-    assert float((outs[1].cpu()[m] - want_s[m]).abs().max()) < 1e-4
+    seed = 11 + nb + S
+    sc = make_scene(nb, seed=seed)
+    scd = dev(sc)
+    o, d = make_rays(B, seed)
+    g = torch.Generator().manual_seed(seed)
+    dist = blend = None
+    step = 1
+    if mode == "fore":
+        z = (torch.rand(B, S, generator=g) * 6.0).sort(-1)[0].contiguous()
+        dist = torch.rand(B, S, generator=g) * 0.1 + 0.01
+        isect = torch.full((B, nb, 2), MISS, device=DEV)
+        ours.ray_block_intersection(o.to(DEV), d.to(DEV), scd["corners"], scd["sizes"], isect)
+        bi = torch.full((B, S, 4), -1, dtype=torch.int16, device=DEV)
+        ours.prepare_points(z.to(DEV), torch.ones(B, 1, dtype=torch.bool, device=DEV), isect, bi)
+        slots = bi.cpu()
+        if nb > 1:                       # a tile behind a -1 slot is ignored
+            extra = (torch.rand(B, S, generator=g) < 0.1) & (slots[..., 0] >= 0) & (slots[..., 1] == -1)
+            slots[..., 2] = torch.where(extra, (slots[..., 0] + 1) % nb, slots[..., 2])
+    else:
+        z = (40 + torch.rand(B, S, generator=g).cumsum(-1)).contiguous()     # beyond every tile
+        slots = torch.randint(-1, nb, (B, 4), generator=g).to(torch.int16)      # with -1 gaps and repeated tiles
+        blend = torch.rand(B, 4, generator=g) + 0.05
+    outs = [torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 3), 7.0, device=DEV), torch.full((B, S, 1), 7.0, device=DEV)]
+    args = (o.to(DEV), d.to(DEV), z.to(DEV))
+    field = (scd["corners"], scd["sizes"], scd["res"], scd["tables"], scd["params"])
+    if mode == "fore":
+        ours.pts_inference(*args, dist.to(DEV), slots.to(DEV), scd["tables"], scd["params"], scd["res"], scd["occ"], scd["starts"],
+                           scd["l2d"], scd["corners"], scd["sizes"], *outs)
+    elif mode == "blend":
+        ours.bg_pts_inference(*args, slots.to(DEV), blend.to(DEV), *field, *outs)
+    else:
+        ours.bg_pts_inference_v2(*args, slots.to(DEV), step, *field, *outs)
+    torch.cuda.synchronize()
+    got = [t.cpu() for t in outs]
+    want_d, want_s, want_a, keep, near = field_restatement(mode, sc, o, d, z, dist, slots, blend, step)
+    keep = torch.from_numpy(keep)
+    for t in got:
+        assert bool((t[keep] == 7.0).all()), "rows of rays without a tile in this slot keep the caller's values"
+        assert bool((t[~keep] != 7.0).all()), "every other sample row is written"
+    if mode == "fore":
+        none = slots[..., 0] == -1
+        assert all(bool((t[none] == 0).all()) for t in got), "unassigned samples give zeros"
+    assert near.mean() < 0.01, f"{near.mean():.3%} of the samples lie within 1e-4 of a cell face"
+    m = torch.from_numpy(~near) & ~keep
+    if B * S > 1:
+        assert int((want_a[m.numpy()] != 0).sum()) > 0.05 * B * S, "too few samples evaluated to test anything"
+    for name, x, y in zip(("diffuse", "specular", "alpha"), got, (want_d, want_s, want_a)):
+        err = float((x.double()[m] - torch.from_numpy(y)[m]).abs().max()) if bool(m.any()) else 0.0
+        assert err < 1e-4, f"{mode} {name}: max abs err {err}"
 
 
 def _render_with(mod, sc, o, d, S, Sb):
@@ -282,7 +387,7 @@ def _render_with(mod, sc, o, d, S, Sb):
 
 
 @pytest.mark.parametrize("nb", [1, 3])
-def test_render_rays_driver_matches_reference_sequence(nb, infer_path):
+def test_render_rays_driver_matches_reference_sequence(nb):
     """render_frame.render_rays (our sync-free mirror of render_rays_base) against the reference's own
     operator sequence run on the rebuilt reference extension; composited colours within 1e-4."""
     ours, ref = _ops()

@@ -33,7 +33,6 @@ def main():
     for merged, fold in ((2, 1), (2, 0), (1, 0), (2, 1), (2, 0), (0, 0), (2, 1)):
         lib.snrf_decoder_set_bwd_merged(ctypes.c_int(merged))
         lib.snrf_decoder_set_fwd_fold(ctypes.c_int(fold))
-        lib.snrf_infer_set_fold(ctypes.c_int(fold))
         ms, loss = bench._time_steps(step, batches, 4)
         capi.time_calls(names)
         for b in batches[:8]:
@@ -43,14 +42,13 @@ def main():
         row = {"bwd_merged": merged, "fwd_fold": fold, "ms_per_step": ms, "loss": loss}
         for k in names:
             row[k + "_ms"] = sum(t.get(k, [])) / max(len(t.get(k, [])), 1)
-        if merged == 2:
+        if merged == 2 and fold == 1:               # the render's decode pass always folds layer 2
             r = bench.bench_render(step, cfg, dev, frames=3, warm=1)
             row["render_ms_per_frame"] = r["ms_per_frame"]
         rows.append(row)
         print(json.dumps(row), flush=True)
     lib.snrf_decoder_set_bwd_merged(ctypes.c_int(2))
     lib.snrf_decoder_set_fwd_fold(ctypes.c_int(1))
-    lib.snrf_infer_set_fold(ctypes.c_int(1))
     with open(args.out, "w") as fh:
         fh.write(json.dumps(rows) + "\n")
 
