@@ -83,6 +83,18 @@ int snrf_field_encode_bwd_adam(const float* rays_o, const float* rays_d, const f
                                float* table, float* exp_avg, float* exp_avg_sq, float lr, float beta1, float beta2, float eps,
                                int step, float* grad_scratch, long long scratch_entries, int small_levels, float* cpts_scratch,
                                const unsigned char* ray_valid, int split, int N, int S, int L, int T, void* stream);
+/* Surface normals of the density field at every sample, forward only: replaces the out_normal branch of
+ * HashGrid.render_batch_rays (hashgrid/__init__.py:547-556: torch.autograd.grad of sigma w.r.t. the samples, create_graph).
+ * feats_lm [16][N] float2 and jac_lm [16][3][N] float2 from snrf_field_encode_fwd of the same rays (mode 1 = fore, 2 =
+ * background; box_min, box_size, rays_o, rays_d [R,3], z_vals [R,S] as there); mask32 [32] (NULL = ones); params as
+ * snrf_decoder_fwd (only Spatial_MLP.mlp.0, .mlp.2 and sigma_layer are read).  g = d sigma / d x at x = o + z d:
+ * -> normal [N,3] = -g / (|g| + 1e-8), grad_x [N,3] = g (may be NULL).  fp32; softplus' as torch's (threshold 20); the
+ * background contraction's max is differentiated at its arg-max axis, as torch.max is.  ray_valid (optional, bytes [R]):
+ * rows of rays with a 0 flag are left untouched.  Grid-stride launch of min(ceil(N / 256), 2 x SMs) CTAs of 256 threads. */
+int snrf_field_normal(const float* feats_lm, const float* jac_lm, const float* mask32, const float* const* params, int mode,
+                      const float* box_min, const float* box_size, const float* rays_o, const float* rays_d,
+                      const float* z_vals, const unsigned char* ray_valid, float* normal, float* grad_x, int N, int S,
+                      void* stream);
 /* measurement hook: when on, snrf_field_encode_bwd_adam times its three kernel classes with CUDA events (and SYNCHRONISES
  * the stream); snrf_field_last_profile -> out4 = milliseconds {geometry + ray gradient, scatter slices, Adam slices, both} */
 void snrf_field_set_profile(int on);

@@ -1255,3 +1255,134 @@ SNRF_API int snrf_field_encode_bwd_adam_ert(const float* rays_o, const float* ra
     t_sample_live = nullptr;
     return rc;
 }
+
+// ---------------------------------------------------------------------------------------------------------------------------
+// Surface normals of the density field, forward only: the out_normal branch of HashGrid.render_batch_rays
+// (hashgrid/__init__.py:547-556), which the reference obtains from torch.autograd.grad of sigma w.r.t. the samples.
+// sigma = softplus(W_s H[:32] + b_s), H = W2 a1 + b2, a1 = exp(-50 z1^2), z1 = W1 (f m) + b1.  Layer 2 is linear, so its
+// sigma rows fold into u = W2[:32,:]^T w_s and c = w_s . b2[:32] + b_s once per CTA: sigma_pre = u . a1 + c and
+//   d sigma / d f = softplus'(sigma_pre) m (W1^T (-100 z1 a1 u)).
+// One pass over the 64 rows of W1 forms z1_j, sigma_pre and the W1^T accumulation together (softplus' is a common factor
+// applied at the end), so a thread holds 32 masked features and 32 gradient accumulators, nothing of width 64.  The gradient
+// w.r.t. the contracted point comes from the encode's Jacobians jac_lm, the one w.r.t. the sample from contract_bwd.
+// fp32 on the CUDA cores: ~4 k FMAs and 512 bytes of reads per sample, W1 broadcast from shared memory.
+// ---------------------------------------------------------------------------------------------------------------------------
+namespace {
+
+constexpr int kNormalThreads = 256;
+constexpr int kNormalCtasPerSm = 2;            // grid-stride: at most this many CTAs per SM (the register budget allows 2)
+
+__global__ void __launch_bounds__(kNormalThreads, kNormalCtasPerSm)
+field_normal_kernel(const float2* __restrict__ feats, const float2* __restrict__ jac, const float* __restrict__ mask32,
+                    const float* __restrict__ W1, const float* __restrict__ b1, const float* __restrict__ W2, const float* __restrict__ b2,
+                    const float* __restrict__ ws, const float* __restrict__ bs, const float* __restrict__ rays_o,
+                    const float* __restrict__ rays_d, const float* __restrict__ z_vals, const float* __restrict__ bmin_p,
+                    const float* __restrict__ bsize_p, const unsigned char* __restrict__ ray_valid, int back,
+                    float* __restrict__ normal, float* __restrict__ grad_x, int N, int S)
+{
+    __shared__ __align__(16) float s_w1[64 * 32];
+    __shared__ float s_b1[64], s_u[64], s_m[32];
+    __shared__ float s_c;
+    for (int i = threadIdx.x; i < 64 * 32; i += blockDim.x) s_w1[i] = W1[i];
+    if (threadIdx.x < 64) {
+        const int j = threadIdx.x;
+        float u = 0.0f;
+        for (int i = 0; i < 32; ++i) u = fmaf(W2[i * 64 + j], ws[i], u);
+        s_u[j] = u;
+        s_b1[j] = b1[j];
+    }
+    if (threadIdx.x < 32) s_m[threadIdx.x] = mask32 != nullptr ? mask32[threadIdx.x] : 1.0f;
+    if (threadIdx.x == 0) {
+        float c = bs[0];
+        for (int i = 0; i < 32; ++i) c = fmaf(ws[i], b2[i], c);
+        s_c = c;
+    }
+    __syncthreads();
+    const f3 bmin = ld3(bmin_p), bsize = ld3(bsize_p);
+    for (int n = blockIdx.x * blockDim.x + threadIdx.x; n < N; n += gridDim.x * blockDim.x) {
+        const int r = n / S;
+        if (ray_valid != nullptr && !ray_valid[r]) continue;          // masked-out ray: its rows are left untouched
+        float fm[32], g[32];
+#pragma unroll
+        for (int l = 0; l < 16; ++l) {
+            const float2 f = ldg2(feats + (size_t)l * N + n);
+            fm[2 * l] = f.x * s_m[2 * l];
+            fm[2 * l + 1] = f.y * s_m[2 * l + 1];
+            g[2 * l] = 0.0f;
+            g[2 * l + 1] = 0.0f;
+        }
+        float sp = s_c;
+        // rows in groups of 8: the eight t_j first, then the W1^T accumulation re-reads the rows from shared memory, so
+        // that no row is held in registers between the two uses.  ptxas (-O3, sm_100a): 128 registers (the cap of
+        // kNormalCtasPerSm), 8 bytes of stack: one 8-byte value stored and reloaded once per sample after this loop,
+        // where the 48 Jacobian loads are issued together; the loop itself has no local-memory traffic
+#pragma unroll 1
+        for (int j0 = 0; j0 < 64; j0 += 8) {
+            float t[8];
+#pragma unroll
+            for (int jj = 0; jj < 8; ++jj) {
+                const float4* w = reinterpret_cast<const float4*>(s_w1 + (j0 + jj) * 32);
+                float z = s_b1[j0 + jj];
+#pragma unroll
+                for (int q = 0; q < 8; ++q) {
+                    const float4 v = w[q];
+                    z = fmaf(v.x, fm[4 * q], z); z = fmaf(v.y, fm[4 * q + 1], z);
+                    z = fmaf(v.z, fm[4 * q + 2], z); z = fmaf(v.w, fm[4 * q + 3], z);
+                }
+                const float a = expf(-50.0f * z * z);
+                const float u = s_u[j0 + jj];
+                sp = fmaf(u, a, sp);
+                t[jj] = -100.0f * z * a * u;
+            }
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+#pragma unroll
+                for (int jj = 0; jj < 8; ++jj) {
+                    const float4 v = reinterpret_cast<const float4*>(s_w1 + (j0 + jj) * 32)[q];
+                    g[4 * q] = fmaf(v.x, t[jj], g[4 * q]); g[4 * q + 1] = fmaf(v.y, t[jj], g[4 * q + 1]);
+                    g[4 * q + 2] = fmaf(v.z, t[jj], g[4 * q + 2]); g[4 * q + 3] = fmaf(v.w, t[jj], g[4 * q + 3]);
+                }
+            }
+        }
+        // torch's softplus backward (beta 1, threshold 20): 1 above the threshold, e^x / (e^x + 1) below it
+        const float e = sp > 20.0f ? 0.0f : expf(sp);
+        const float dsp = sp > 20.0f ? 1.0f : e / (e + 1.0f);
+        f3 gc = mk3(0.0f, 0.0f, 0.0f);
+#pragma unroll
+        for (int l = 0; l < 16; ++l) {
+            const float g0 = dsp * s_m[2 * l] * g[2 * l], g1 = dsp * s_m[2 * l + 1] * g[2 * l + 1];
+            const float2* jl = jac + (size_t)l * 3 * N + n;
+            const float2 jx = __ldcs(jl), jy = __ldcs(jl + (size_t)N), jz = __ldcs(jl + 2 * (size_t)N);    // read once
+            gc.x = fmaf(g0, jx.x, fmaf(g1, jx.y, gc.x));
+            gc.y = fmaf(g0, jy.x, fmaf(g1, jy.y, gc.y));
+            gc.z = fmaf(g0, jz.x, fmaf(g1, jz.y, gc.z));
+        }
+        const Pt p = contract(back != 0, sample_pos(ld3(rays_o + 3 * (size_t)r), ld3(rays_d + 3 * (size_t)r), z_vals[n]), bmin, bsize);
+        const f3 gx = contract_bwd(back != 0, p, gc);
+        const float den = sqrtf(dot3(gx, gx)) + 1e-8f;
+        st3(normal + 3 * (size_t)n, mk3(-gx.x / den, -gx.y / den, -gx.z / den));
+        if (grad_x != nullptr) st3(grad_x + 3 * (size_t)n, gx);
+    }
+}
+
+}  // namespace
+
+// feats_lm [16][N] float2 and jac_lm [16][3][N] float2 from snrf_field_encode_fwd (mode 1 / 2, same rays and box);
+// params as snrf_decoder_fwd (host array of 16 device pointers, only the first six are read).  -> normal [N,3] =
+// -g / (|g| + 1e-8), grad_x [N,3] (optional) = g = d sigma / d sample.  Rows of masked-out rays are left untouched.
+SNRF_API int snrf_field_normal(const float* feats_lm, const float* jac_lm, const float* mask32, const float* const* params, int mode,
+                               const float* box_min, const float* box_size, const float* rays_o, const float* rays_d,
+                               const float* z_vals, const unsigned char* ray_valid, float* normal, float* grad_x, int N, int S,
+                               void* stream)
+{
+    SNRF_CHECK_ARG(N >= 0 && S > 0 && (mode == 1 || mode == 2), "snrf_field_normal: need N >= 0, S > 0, mode 1 or 2 (N=%d S=%d mode=%d)", N, S, mode);
+    SNRF_CHECK_ARG(feats_lm && jac_lm && params && box_min && box_size && rays_o && rays_d && z_vals && normal,
+                   "snrf_field_normal: a required pointer is NULL");
+    if (N == 0) return 0;
+    for (int i = 0; i < 6; ++i) SNRF_CHECK_ARG(params[i] != nullptr, "snrf_field_normal: decoder parameter %d is NULL", i);
+    const int want = snrf_div_up(N, kNormalThreads), cap = snrf_sm_count() * kNormalCtasPerSm;
+    field_normal_kernel<<<want < cap ? want : cap, kNormalThreads, 0, (cudaStream_t)stream>>>(
+        (const float2*)feats_lm, (const float2*)jac_lm, mask32, params[0], params[1], params[2], params[3], params[4], params[5],
+        rays_o, rays_d, z_vals, box_min, box_size, ray_valid, mode == 2 ? 1 : 0, normal, grad_x, N, S);
+    SNRF_RETURN_LAUNCH("snrf_field_normal");
+}

@@ -459,26 +459,35 @@ class HashGrid(nn.Module):
         R, S = z_vals.shape
         render_mode = mode
         mask16 = self.weight_feature(kwargs["global_step"])
-        # out_normal differentiates sigma w.r.t. the sample positions with create_graph (hashgrid/__init__.py:547-556 of the
-        # reference): that needs the torch decoder graph, so it takes the torch branch below (decided before any work)
-        params = _decoder.decoder_params(decoder) if (self.fused_decoder and not out_normal) else None
+        params = _decoder.decoder_params(decoder) if self.fused_decoder else None
         mode = 1 if contract_func == self.contract_fore else (2 if contract_func == self.contract_bg else 0)
-        if params is not None and mode != 0 and self.fused_encode and not out_normal and self.HE.features.is_cuda:
+        if params is not None and mode != 0 and self.fused_encode and self.HE.features.is_cuda:
             # fully fused path: sample position + contraction + hash encode in one kernel (level-major
             # features), the stock ShallowMLP on the tensor cores, packed head rows straight into compositing
+            jac = [] if out_normal else None
             feats = _field.field_encode(rays_o, rays_d, z_vals, self.HE.features, self.HE.resolution, self.min_bbox,
-                                        self.bbox_size, mode)
-            heads = _field.decoder_apply(feats, rays_d, mask16.repeat_interleave(2), S, params)
-            return _render.composite_packed(heads, z_vals, dists, rays_d, infinity, train=(render_mode is TRAIN)), True
+                                        self.bbox_size, mode, jac_out=jac)
+            mask32 = mask16.repeat_interleave(2)
+            if out_normal:
+                # the reference differentiates sigma w.r.t. the samples with torch.autograd.grad (hashgrid/__init__.py:547-556)
+                # and accumulates the normal detached: one forward kernel on the encode's features and Jacobians gives the
+                # same normal, and the Jacobians are released here unless the encode kept them for the ray gradient
+                n = _field.field_normal(feats, jac.pop(), mask32, params, rays_o.contiguous(), rays_d.contiguous(),
+                                        z_vals.contiguous(), self.min_bbox, self.bbox_size, mode)
+            heads = _field.decoder_apply(feats, rays_d, mask32, S, params)
+            out = _render.composite_packed(heads, z_vals, dists, rays_d, infinity, train=(render_mode is TRAIN))
+            if out_normal:
+                out["normal"] = self.accumulate(out["weights"], n.view(R, S, 3))
+            return out, True
         samples = rays_o[:, None, :] + z_vals[..., None] * rays_d[:, None, :]
         if contract_func is not None:
             cx, extra_w = contract_func(samples.reshape(-1, 3))
         else:
             cx, extra_w = samples.reshape(-1, 3), None
         feats = self.HE(cx)
-        if params is not None and extra_w is None:
+        if params is not None and extra_w is None and not out_normal:
             # stock ShallowMLP: the whole decoder runs on the tensor cores (csrc/decoder.cu) and
-            # hands packed head rows straight to the compositing kernel
+            # hands packed head rows straight to the compositing kernel; out_normal differentiates the torch decoder below
             heads = _field.decoder_apply(feats, rays_d, mask16.repeat_interleave(2), S, params)
             return _render.composite_packed(heads, z_vals, dists, rays_d, infinity, train=(render_mode is TRAIN)), True
         mask32 = mask16[None, None, :].repeat_interleave(2, dim=-1)

@@ -134,10 +134,12 @@ class FieldEncodeFn(torch.autograd.Function):
     Jacobians; the backward is a pure gradient scatter into `features.grad` (accumulated in place, no dense
     temporary) and returns d/d rays_o, d/d rays_d.  Where the table gradient goes is decided by
     `_gradmode`: returned densely (default, autograd-conformant), accumulated into `features.grad` ("direct"), or
-    consumed on the spot by the sparse Adam update ("fused": snrf_field_encode_bwd_adam)."""
+    consumed on the spot by the sparse Adam update ("fused": snrf_field_encode_bwd_adam).
+    `jac_out` (a list or None) receives the Jacobians [16, 3, R*S, 2], computed for it also when the rays need no gradient;
+    they are kept for the backward only when the rays do."""
 
     @staticmethod
-    def forward(ctx, rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid, split=0, ert=None):
+    def forward(ctx, rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid, split=0, ert=None, jac_out=None):
         R, S = z_vals.shape
         ctx.ert = ert
         N, L, T = R * S, int(features.shape[0]), int(features.shape[1])
@@ -147,7 +149,7 @@ class FieldEncodeFn(torch.autograd.Function):
                 raise RuntimeError("field encode: float32 CUDA tensors required (no CPU fallback)")
         need_pos = ctx.needs_input_grad[0] or ctx.needs_input_grad[1]
         out = torch.empty(L, N, 2, dtype=f32, device=z_vals.device)
-        jac = torch.empty(L, 3, N, 2, dtype=f32, device=z_vals.device) if need_pos else None
+        jac = torch.empty(L, 3, N, 2, dtype=f32, device=z_vals.device) if (need_pos or jac_out is not None) else None
         feats = features.detach().contiguous()
         box_min, box_size = box_min.contiguous(), box_size.contiguous()
         rc = capi.lib().snrf_field_encode_fwd(ptr(rays_o), ptr(rays_d), ptr(z_vals), c_void_p(0), ptr(box_min), ptr(box_size),
@@ -157,9 +159,11 @@ class FieldEncodeFn(torch.autograd.Function):
         ctx.mode, ctx.split, ctx.dims = int(mode), int(split), (N, S, L, T)
         ctx.small_levels = small_levels(resolution)
         ctx.features = features
-        ctx.save_for_backward(rays_o, rays_d, z_vals, resolution, box_min, box_size, jac if jac is not None else out.new_empty(0),
+        if jac_out is not None:
+            jac_out.append(jac)
+        ctx.save_for_backward(rays_o, rays_d, z_vals, resolution, box_min, box_size, jac if need_pos else out.new_empty(0),
                               valid if valid is not None else out.new_empty(0))
-        ctx.has_jac, ctx.has_valid = jac is not None, valid is not None
+        ctx.has_jac, ctx.has_valid = need_pos, valid is not None
         return out
 
     @staticmethod
@@ -188,7 +192,7 @@ class FieldEncodeFn(torch.autograd.Function):
                     ctypes.c_longlong(scratch.shape[0]), c_int(ctx.small_levels), ptr(cpts), *tail)
             capi.check(rc, "snrf_field_encode_bwd_adam")
             capi.launch_count += int(capi.lib().snrf_field_last_launch_count()) - 1     # one C call, many kernels
-            return g_o, g_d, None, None, None, None, None, None, None, None, None
+            return g_o, g_d, None, None, None, None, None, None, None, None, None, None
         direct = mode is not None
         if direct:
             # the training step's explicit opt-in (_gradmode.table_backward): accumulate in place, no dense temporary
@@ -200,11 +204,37 @@ class FieldEncodeFn(torch.autograd.Function):
             g_table, first = _gradmode.shared_table_grad(features)
         rc = getattr(capi.lib(), "snrf_field_encode_bwd" + sfx)(*common, ptr(g_table), *tail)
         capi.check(rc, "snrf_field_encode_bwd")
-        return g_o, g_d, None, (g_table if first else None), None, None, None, None, None, None, None
+        return g_o, g_d, None, (g_table if first else None), None, None, None, None, None, None, None, None
 
 
-def field_encode(rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid=None, split=0, ert=None):
+def field_encode(rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid=None, split=0, ert=None, jac_out=None):
     """valid (bool [R] or None): rays flagged False are skipped (their feature rows are left unwritten).
     mode 3: rays [0, split) are contracted with the fore map, rays [split, R) with the background map.
-    ert (_render.ErtState | None): early ray termination -- the backward skips the samples the compositing flagged dead."""
-    return FieldEncodeFn.apply(rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid, split, ert)
+    ert (_render.ErtState | None): early ray termination -- the backward skips the samples the compositing flagged dead.
+    jac_out (list | None): receives the forward's per-level Jacobians (see FieldEncodeFn), e.g. for field_normal."""
+    return FieldEncodeFn.apply(rays_o, rays_d, z_vals, features, resolution, box_min, box_size, mode, valid, split, ert, jac_out)
+
+
+def field_normal(feats, jac, mask32, params, rays_o, rays_d, z_vals, box_min, box_size, mode, valid=None, normal=None, grad=None):
+    """Surface normal -d sigma/dx / (|d sigma/dx| + 1e-8) at every sample of a field_encode call (snrf_field_normal): feats
+    [16, N, 2] and jac [16, 3, N, 2] from that call, mask32 [32] the level mask, params the 16 decoder tensors
+    (hashgrid._decoder.decoder_params), mode 1 (fore) or 2 (background) as there.  Forward only: nothing is differentiated.
+    Returns normal [N, 3]; `normal` / `grad` ([N, 3], optional) are buffers to write, grad receiving d sigma / dx itself.
+    Rows of rays flagged False in `valid` are left as they are."""
+    R, S = z_vals.shape
+    N = R * S
+    if tuple(feats.shape) != (16, N, 2) or tuple(jac.shape) != (16, 3, N, 2):
+        raise RuntimeError(f"field_normal: features [16, {N}, 2] and Jacobians [16, 3, {N}, 2] required, "
+                           f"got {tuple(feats.shape)} and {tuple(jac.shape)}")
+    for t in (feats, jac, rays_o, rays_d, z_vals):
+        if not t.is_cuda or t.dtype != f32 or not t.is_contiguous():
+            raise RuntimeError("field_normal: contiguous float32 CUDA tensors required (no CPU fallback)")
+    if normal is None:
+        normal = torch.empty(N, 3, dtype=f32, device=feats.device)
+    arr, keep = _param_array(params)
+    m = mask32.contiguous() if mask32 is not None else None
+    rc = capi.lib().snrf_field_normal(ptr(feats), ptr(jac), ptr(m), arr, c_int(int(mode)), ptr(box_min.contiguous()),
+                                      ptr(box_size.contiguous()), ptr(rays_o), ptr(rays_d), ptr(z_vals), ptr(valid), ptr(normal),
+                                      ptr(grad), c_int(N), c_int(S), capi.stream())
+    capi.check(rc, "snrf_field_normal")
+    return normal
