@@ -279,20 +279,11 @@ int snrf_decoder_fwd(const float* feats, const float* mask32, const float* rays_
 /* Operand precision of the decoder GEMMs: 1 (default) = error-compensated bf16x3 split operands in
  * every forward GEMM (~fp32 accuracy), 0 = plain bf16 operands (fastest). */
 void snrf_decoder_set_precision(int split);
-/* tuning hook: forward tiles in flight per CTA (4 = default: in-place operand tiles + per-ray SH term, S >= 16; 2 = round-1 kernel) */
-void snrf_decoder_set_inflight(int n);
-/* tuning hook: 1 (default) = the four-tile forward composes layer 2 (linear, no activation) into its consumers when it
- * stages the weights: z3 and the heads come straight from a1, four dependent stages per tile instead of five */
-void snrf_decoder_set_fwd_fold(int on);
-/* tuning hook: how snrf_decoder_bwd uses heads_fwd when given.  2 (default) = layer 2 (linear, no activation) folded into its
- * consumers: six dependent stages per tile, dW2 / dW3[:, :32] / dW_heads / db2 composed once per CTA from two accumulators;
- * 1 = the recompute skips the heads GEMM and layer 5 and layer 4 shares a commit group with the first backward stage;
- * 0 = recompute everything (the round-1 stage sequence) */
-void snrf_decoder_set_bwd_merged(int on);
-/* Backward of snrf_decoder_fwd (autograd of network.py:151-190).  grad_heads[N,10] (column order
- * of heads) -> grad_feats[N,32] WRITTEN; grad_rays_d[R,3] ACCUMULATED (may be NULL; the view
- * direction enters through the SH encoding only); grad_params = HOST array of 16 DEVICE pointers,
- * shapes/order of params, ACCUMULATED.  The forward is recomputed per 128-sample tile. */
+/* Backward of snrf_decoder_fwd (autograd of network.py:151-190).  heads_fwd[N,10] (REQUIRED, non-NULL) = the heads
+ * snrf_decoder_fwd returned for these inputs.  grad_heads[N,10] (column order of heads) -> grad_feats[N,32] WRITTEN;
+ * grad_rays_d[R,3] ACCUMULATED (may be NULL; the view direction enters through the SH encoding only); grad_params = HOST
+ * array of 16 DEVICE pointers, shapes/order of params, ACCUMULATED.  The forward is recomputed per 128-sample tile up to
+ * layer 4, with layer 2 (linear, no activation) folded into its consumers. */
 int snrf_decoder_bwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params,
                      const float* grad_heads, float* grad_feats, float* grad_rays_d, float* const* grad_params,
                      int N, int S, int level_major, const unsigned char* ray_valid, const float* heads_fwd, void* stream);

@@ -38,13 +38,6 @@ using namespace dec;
 
 namespace {
 
-// Weight-gradient GEMMs dW += dz^T a: the activation operand can only be read as its fp16 hi part (11 bits; its lo tile is
-// recycled by then).  With kWgradDzLo the dz operand is compensated (hi + lo: two MMA groups per layer); without it dz is
-// read as hi only as well -- the two roundings are then symmetric (both 2^-12, unbiased, independent per sample), the
-// weight-gradient error grows by ~sqrt(2) (measured: see tests/test_decoder_gpu.py) and half of the backward's
-// weight-gradient MMAs disappear, together with the one group that had to sit in front of a commit.
-constexpr bool kWgradDzLo = false;
-
 // ------------------------------- forward ------------------------------------
 // feats [N,32] f32, rays_d [R,3] (sample n belongs to ray n / S), out [N,10] f32 =
 // (sigma, tint3, diffuse3, specular3).
@@ -74,7 +67,7 @@ decoder_fwd_kernel(const float* __restrict__ feats, const float* __restrict__ ma
     unsigned char* T2 = T1 + kTile;
     unsigned char* LOa = SPLIT ? T2 + kTile : T1;      // never written when !SPLIT
     unsigned char* LOb = SPLIT ? LOa + kTile : T2;
-    const Tiles T{T0, T1, nullptr, T2, T1, nullptr, T2, nullptr, LOa, LOb};
+    const Tiles T{T0, T1, T2, T1, T2, LOa, LOb};
 
     for (int tile = 2 * blockIdx.x + c.group; tile < num_tiles; tile += 2 * gridDim.x) {
         const int n = tile * kRows + c.row;
@@ -83,7 +76,7 @@ decoder_fwd_kernel(const float* __restrict__ feats, const float* __restrict__ ma
         float head[10], zh[7];
         f3 d = mk3(0.f, 0.f, 1.f);
         float dn = 1.0f;
-        forward_tile<SPLIT, false, 2>(c, T, feats, rays_d, n, live, S, head, zh, d, dn, level_stride);
+        forward_tile<SPLIT, 2>(c, T, feats, rays_d, n, live, S, head, zh, d, dn, level_stride);
         if (c.cg == 0) {
             float z[16];
             umma::tmem_ld16(c.tmem + cDh + c.lane_addr, z);
@@ -107,7 +100,7 @@ decoder_fwd_kernel(const float* __restrict__ feats, const float* __restrict__ ma
 
 // ------------------------------- forward, four tiles in flight ---------------
 // (decoder_core.cuh: forward_layers4; same results as decoder_fwd_kernel, S >= kMinS4)
-template <bool SPLIT, bool FOLD>
+template <bool SPLIT>
 __global__ void __launch_bounds__(kThreadsDec, 1)
 decoder_fwd4_kernel(const float* __restrict__ feats, const float* __restrict__ mask32, const float* __restrict__ rays_d,
                     DecoderParams p, float* __restrict__ out, int N, int S, int num_tiles, long long level_stride,
@@ -122,7 +115,7 @@ decoder_fwd4_kernel(const float* __restrict__ feats, const float* __restrict__ m
     stage_all_weights<SPLIT>(smem, p, mask32, tid, kThreadsDec);
     float* w3sh = reinterpret_cast<float*>(smem + off_w3sh<SPLIT>());
     stage_w3sh(w3sh, p, tid, kThreadsDec);
-    if (FOLD) stage_fold_weights4<SPLIT>(smem, p, reinterpret_cast<float*>(smem + off_tiles4<SPLIT>()), tid, kThreadsDec);
+    stage_fold_weights4<SPLIT>(smem, p, reinterpret_cast<float*>(smem + off_tiles4<SPLIT>()), tid, kThreadsDec);
     if (warp == 0) umma::tmem_alloc<512>(&tmem_slot);
     if (tid == 0) {
         for (int g = 0; g < kGroups4; ++g) umma::mbar_init(&bars[g], 1);
@@ -184,8 +177,8 @@ decoder_fwd4_kernel(const float* __restrict__ feats, const float* __restrict__ m
         float head[10], zh[7];
         // the ray vectors are formed under the L1 MMAs: the first barrier of forward_layers4 has every thread of the group past
         // its last read of rb (the previous tile's z3 epilogue), two more barriers follow before the next read
-        forward_layers4<SPLIT, FOLD>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
-                                     [&]() { ray_vectors4<false>(rb, w3sh, rays_d, ray0, last - ray0 + 1, c.gtid); });
+        forward_layers4<SPLIT>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
+                               [&]() { ray_vectors4<false>(rb, w3sh, rays_d, ray0, last - ray0 + 1, c.gtid); });
         float z[16];
         umma::tmem_ld16(c.tmem + c4Dh + c.lane_addr, z);
         umma::tc_wait_ld();
@@ -202,498 +195,14 @@ decoder_fwd4_kernel(const float* __restrict__ feats, const float* __restrict__ m
     if (warp == 0) umma::tmem_free<512>(tmem_slot);
 }
 
-// ------------------------------- backward -----------------------------------
-// Per tile: recompute the forward keeping every intermediate in shared memory, then walk the
-// layers backwards.  Each backward stage is one commit group holding the input-gradient GEMM
-// (dA_{l-1} = dz_l W_l, weights read MN-major from the very tile the forward used K-major) and
-// the weight-gradient GEMMs (dW_l += dz_l^T A_{l-1}, both operands read MN-major, M = 64
-// accumulators that stay in TMEM for the whole kernel).  Bias gradients of the 64-wide layers
-// are one more GEMM against a column of ones.
+// ------------------------------- backward ------------------------------------------------------------------------------
+// Per tile: recompute the forward keeping the intermediates in shared memory, then walk the layers backwards.  Each stage
+// commits its input-gradient GEMM (dA = dz W, the weight tile read MN-major) first and issues its weight-gradient GEMMs
+// (dW += dz^T A, both operands MN-major, M = 64 accumulators that stay in TMEM for the whole kernel) behind the commit, so
+// that they execute under the epilogue; a tile ends with a commit on `bar_tail`, waited for before the next tile overwrites
+// the operand tiles.  The weight-gradient GEMMs read the hi parts of both operands: the two roundings are symmetric (2^-12,
+// unbiased, independent per sample) and average out over the batch.
 //
-// shared-memory tiles (16 KB each): A0 = [x | SH | SH_lo], a1, g1 -> dz1, H, a3, g3 -> dz4, a4,
-// g4 -> dz5, LOa (a1_lo / a3_lo in the forward, then the lo part of the current dz), LOb (x_lo / H_lo /
-// a4_lo in the forward, then [dz_heads | dz_spec | lo parts] and finally dH = dz2); a4 holds dH_lo after
-// B1; g = d(activation)/dz.
-// HEADS: the forward's head values are at hand (heads_fwd): the recompute skips the heads GEMM and layer 5, and layer 4
-// shares ONE commit group with the first backward stage (its epilogue forms dz5 = dA4 * g'(z4) straight from registers):
-// eight dependent stages per tile instead of ten.
-template <bool SPLIT, bool HEADS>
-__global__ void __launch_bounds__(kThreadsDec, 1)
-decoder_bwd_kernel(const float* __restrict__ feats, const float* __restrict__ mask32, const float* __restrict__ rays_d,
-                   DecoderParams p, const float* __restrict__ grad_heads, float* __restrict__ grad_feats,
-                   float* __restrict__ grad_rays_d, DecoderGrads gp, int N, int S, int num_tiles, long long level_stride,
-                   const unsigned char* __restrict__ ray_valid, const unsigned* __restrict__ gmax_bits,
-                   const float* __restrict__ heads_fwd, const unsigned char* __restrict__ sample_live)
-{
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    unsigned char* smem = (unsigned char*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    unsigned char* base = smem + off_tiles<SPLIT>();
-    const Tiles T{base, base + kTile, base + 2 * kTile, base + 3 * kTile, base + 4 * kTile, base + 5 * kTile,
-                  base + 6 * kTile, base + 7 * kTile, base + 8 * kTile, base + 9 * kTile};
-    // backward-phase aliases of tiles the forward no longer needs
-    unsigned char* Tdz = T.LOb;          // [dz_heads | dz_spec | their lo parts], then dH = dz2 (hi)
-    unsigned char* Tdzlo = T.LOa;        // lo part of the current layer's dz (dz5, dz4, dz1 in turn)
-    unsigned char* Tdhlo = T.a4;         // lo part of dH (a4 is dead once B1 has read it)
-    __shared__ uint64_t bar;
-    __shared__ uint64_t bar_tail;        // completion of the weight-gradient MMAs left in flight behind each stage's commit
-    __shared__ uint32_t tmem_slot;
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    uint32_t tail_phase = 0;
-    bool tail_pending = false;
-    // Power-of-two scale of the incoming gradient: max |grad_heads| (bits in *gmax_bits, from grad_absmax_kernel) is
-    // mapped into [0.5, 1), so that the fp16 dz operands keep 15 binary orders of headroom above it for the growth along
-    // the backward chain and 14 (24 with subnormals) below it.  Everything downstream is linear in the gradient:
-    // outputs are multiplied by ginv (exact).  A zero / non-finite maximum leaves the scale at 1.
-    float gscale = 1.0f, ginv = 1.0f;
-    if (kOpBf16 == 0 && gmax_bits != nullptr) {
-        const int e = (int)((*gmax_bits >> 23) & 0xffu);            // gmax = m 2^(e - 127), m in [1, 2)
-        if (e > 0 && e < 255) {
-            int se = 253 - e;                                        // exponent field of 2^(126 - e): gmax * scale in [0.5, 1)
-            se = se < 1 ? 1 : (se > 253 ? 253 : se);
-            gscale = __uint_as_float((uint32_t)se << 23);
-            ginv = __uint_as_float((uint32_t)(254 - se) << 23);
-        }
-    }
-
-    stage_all_weights<SPLIT>(smem, p, mask32, tid, kThreadsDec);
-    if (warp == 0) umma::tmem_alloc<512>(&tmem_slot);
-    if (tid == 0) { umma::mbar_init(&bar, 1); umma::mbar_init(&bar_tail, 1); umma::mbar_fence_init(); }
-    umma::fence_async_smem();
-    umma::tc_fence_before();
-    __syncthreads();
-    umma::tc_fence_after();
-    Ctx<SPLIT, 4> c;                                    // one tile per CTA, 4 column groups of 16
-    c.init(smem, &bar, tmem_slot);
-    const int row = c.row, cg = c.cg;
-    const uint32_t tmem = c.tmem, lane_addr = c.lane_addr;
-    const float* bias = c.bias;
-    const float* mask = c.mask;
-    const uint32_t aA0 = umma::smem_u32(T.A0), aa1 = umma::smem_u32(T.a1), ag1 = umma::smem_u32(T.g1), aH = umma::smem_u32(T.H),
-                   aa3 = umma::smem_u32(T.a3), ag3 = umma::smem_u32(T.g3), aa4 = umma::smem_u32(T.a4), ag4 = umma::smem_u32(T.g4),
-                   adz = umma::smem_u32(Tdz), adzlo = umma::smem_u32(Tdzlo), adhlo = umma::smem_u32(Tdhlo);
-    // Bias gradients of the 64-wide layers.  Layers 1 and 3 read A0, whose column 32 holds SH_0 = bf16(0.28209479)
-    // = 0.28125 in every live row: column 32 of dW1 (N widened to 48) and column 0 of the SH part of dW3 are
-    // c0 * sum_n dz_n, the flush divides by c0.  Layers 2 and 4 (inputs a1 / a3 have no constant column) are summed
-    // per thread in fp32 registers over all the tiles of this CTA and reduced once at the end.
-    float acc_b2[16], acc_b4[16], acc_small[10];       // acc_small: sigma, diffuse3, tint3, specular3 biases (column group 0)
-#pragma unroll
-    for (int j = 0; j < 16; ++j) { acc_b2[j] = 0.0f; acc_b4[j] = 0.0f; }
-#pragma unroll
-    for (int j = 0; j < 10; ++j) acc_small[j] = 0.0f;
-    const uint32_t aW1 = umma::smem_u32(smem + oW1), aW2 = umma::smem_u32(smem + oW2), aW3 = umma::smem_u32(smem + oW3),
-                   aW4 = umma::smem_u32(smem + oW4), aWh = umma::smem_u32(smem + oWh), aW5 = umma::smem_u32(smem + oW5);
-    constexpr uint32_t idf64 = umma::idesc_f16(128, 64, 0, 0, kOpBf16, kOpBf16);       // forward GEMM of layer 4 (HEADS path)
-    // input-gradient GEMMs: A K-major (dz rows), B MN-major (weight tile: rows = K = out, cols = N = in)
-    constexpr uint32_t idg64 = umma::idesc_f16(128, 64, 0, 1, kOpBf16, kOpBf16), idg32 = umma::idesc_f16(128, 32, 0, 1, kOpBf16, kOpBf16);
-    // weight-gradient GEMMs: both operands MN-major, M = 64
-    // (A = dz^T; B = the layer's input activations -- and the other way round for the transposed narrow layers)
-    constexpr uint32_t idw64 = umma::idesc_f16(64, 64, 1, 1, kOpBf16, kOpBf16), idw48 = umma::idesc_f16(64, 48, 1, 1, kOpBf16, kOpBf16),
-                       idw32 = umma::idesc_f16(64, 32, 1, 1, kOpBf16, kOpBf16), idw16 = umma::idesc_f16(64, 16, 1, 1, kOpBf16, kOpBf16),
-                       idwt16 = umma::idesc_f16(64, 16, 1, 1, kOpBf16, kOpBf16);
-    const uint32_t aW2l = umma::smem_u32(smem + oW2l), aW3l = umma::smem_u32(smem + oW3l), aW4l = umma::smem_u32(smem + oW4l),
-                   aW5l = umma::smem_u32(smem + oW5l);
-    // dA = dz W over `nk` k-steps; in SPLIT mode dz = dz_hi + dz_lo and W = W_hi + W_lo (the lo tile,
-    // or the lo half of a packed tile at a 64-byte column offset): dz_hi W_hi + dz_hi W_lo + dz_lo W_hi
-    auto dgrad = [&](int col, uint32_t dz_tile, int dz_k, uint32_t dzlo_tile, int dzlo_k, uint32_t w_hi, uint32_t w_lo, int nk,
-                     uint32_t idesc) {
-        for (int k = 0; k < nk; ++k)
-            umma::mma_bf16(tmem + col, umma::desc_kmajor(dz_tile, dz_k + k), umma::desc_mnmajor(w_hi, k), idesc, k > 0);
-        if (SPLIT) {
-            for (int k = 0; k < nk; ++k)
-                umma::mma_bf16(tmem + col, umma::desc_kmajor(dz_tile, dz_k + k), umma::desc_mnmajor(w_lo, k), idesc, 1);
-            for (int k = 0; k < nk; ++k)
-                umma::mma_bf16(tmem + col, umma::desc_kmajor(dzlo_tile, dzlo_k + k), umma::desc_mnmajor(w_hi, k), idesc, 1);
-        }
-    };
-    // dW += dz^T B over the 128 rows of the tile (8 k-steps), one operand part at a time; `init` = this is the first
-    // MMA group ever issued into that accumulator (first tile of the CTA, first part).  In SPLIT mode the dz operand
-    // is compensated (dz_hi + dz_lo = two parts); the activation operand B stays bf16 (its lo part is gone by now).
-    //
-    // Scheduling: a stage's epilogue needs only its input-gradient GEMM, so that one is committed first and the
-    // weight-gradient GEMMs are issued BEHIND the commit: they execute while the CTA runs the epilogue (ncu showed
-    // ~45 % of this kernel waiting for, or issuing, M = 64 weight-gradient MMAs when they sat in front of the commit).
-    // A part may be deferred like that only if the epilogue of its own stage does not overwrite a tile it reads
-    // (the next stage's commit covers every earlier MMA); the tile ends with a commit + wait on `bar_tail`.
-    auto wgrad_part = [&](int col, uint32_t a_tile, uint32_t b_tile_plus_off, uint32_t idesc, bool init) {
-        for (int k = 0; k < 8; ++k)
-            umma::mma_bf16(tmem + col, umma::desc_mnmajor(a_tile, k), umma::desc_mnmajor(b_tile_plus_off, k), idesc, (!init) || k > 0);
-    };
-    auto wgrad = [&](int col, uint32_t a_tile, uint32_t a_lo, uint32_t b_tile_plus_off, uint32_t idesc, bool first) {
-        wgrad_part(col, a_tile, b_tile_plus_off, idesc, first);
-        if (SPLIT && kWgradDzLo) wgrad_part(col, a_lo, b_tile_plus_off, idesc, false);
-    };
-    // transposed narrow layers (dW^T += A^T dz): the compensated operand is B
-    auto wgrad_t = [&](int col, uint32_t a_tile, uint32_t b_hi, uint32_t b_lo, uint32_t idesc, bool first) {
-        for (int k = 0; k < 8; ++k)
-            umma::mma_bf16(tmem + col, umma::desc_mnmajor(a_tile, k), umma::desc_mnmajor(b_hi, k), idesc, (!first) || k > 0);
-        if (SPLIT && kWgradDzLo)
-            for (int k = 0; k < 8; ++k)
-                umma::mma_bf16(tmem + col, umma::desc_mnmajor(a_tile, k), umma::desc_mnmajor(b_lo, k), idesc, 1);
-    };
-    float v[16];
-    // dz = dA * g on this thread's 16 columns: hi part in place over the g tile, lo part (SPLIT) into Tlo
-    auto mul_inplace = [&](int col, unsigned char* Tg, unsigned char* Tlo, float* bias_acc) {
-        umma::tmem_ld16(tmem + col + lane_addr + 16 * cg, v);
-        umma::tc_wait_ld();
-#pragma unroll
-        for (int q = 0; q < 2; ++q) {
-            const uint4 w4 = *reinterpret_cast<const uint4*>(Tg + umma::tile_chunk_off(row, 2 * cg + q));
-            const uint32_t w[4] = {w4.x, w4.y, w4.z, w4.w};
-            float o[8];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-                const __half2 h2 = *reinterpret_cast<const __half2*>(&w[e]);
-                o[2 * e] = v[8 * q + 2 * e] * __low2float(h2);
-                o[2 * e + 1] = v[8 * q + 2 * e + 1] * __high2float(h2);
-            }
-            if (bias_acc != nullptr) {
-#pragma unroll
-                for (int e = 0; e < 8; ++e) bias_acc[8 * q + e] += o[e];
-            }
-            store8_act<SPLIT>(Tg, 2 * cg + q, Tlo, 2 * cg + q, row, o);
-        }
-    };
-    // 32 accumulator columns (8 per column group) -> chunk (chunk0 + cg) of a hi / lo tile pair
-    auto store_quarter = [&](int col, unsigned char* Thi, unsigned char* Tlo, int chunk0, float* bias_acc) {
-        umma::tmem_ld8(tmem + col + lane_addr + 8 * cg, v);
-        umma::tc_wait_ld();
-#pragma unroll
-        for (int e = 0; e < 8; ++e) bias_acc[e] += v[e];
-        store8_act<SPLIT>(Thi, chunk0 + cg, Tlo, chunk0 + cg, row, v);
-    };
-
-    // the MMAs of this kernel are issued by one elected lane of warp 4 (column group 1): the warps of column group 0 also
-    // form the head gradients and those of column group 3 the SH backward, so a warp of group 1 / 2 reaches the issue first
-    const bool lead_warp = umma::warp_uniform() == 4;
-    bool first = true;      // no tile processed yet: the first one initialises the TMEM gradient accumulators
-    for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-        const int n = tile * kRows + row;
-        // (sample_live: the early-ray-termination flags of snrf_composite_fwd_ert -- a dead sample has a zero gradient row)
-        const bool live = n < N && (ray_valid == nullptr || ray_valid[n / S] != 0) && (sample_live == nullptr || sample_live[n] != 0);
-        if ((ray_valid != nullptr || sample_live != nullptr) && !c.any(live)) continue;     // tile of masked-out / terminated samples only
-        float head[10], zh[7];
-        f3 d = mk3(0.f, 0.f, 1.f);
-        float dn = 1.0f;
-        // with the forward's head values at hand (heads_fwd) the recompute stops after layer 3; layer 4 joins the first
-        // backward stage below
-        constexpr bool have_heads = HEADS;
-        // L2 prefetches: this tile's head gradients / head values (needed a few stages from now) and the next tile's features
-        if (cg == 0 && live) {
-            prefetch_l2(grad_heads + (size_t)n * 10);
-            prefetch_l2(grad_heads + (size_t)n * 10 + 8);
-            if (have_heads) { prefetch_l2(heads_fwd + (size_t)n * 10); prefetch_l2(heads_fwd + (size_t)n * 10 + 8); }
-        }
-        {
-            const long long nn = (long long)(tile + gridDim.x) * kRows + row;
-            if (nn < N) {
-                if (level_stride == 0) prefetch_l2(feats + (size_t)nn * 32 + 8 * cg);
-                else {
-#pragma unroll
-                    for (int l = 0; l < 4; ++l) if ((row & 3) == 0) prefetch_l2(reinterpret_cast<const float2*>(feats) + nn + (size_t)(4 * cg + l) * level_stride);
-                }
-            }
-        }
-        forward_tile<SPLIT, true, 4>(c, T, feats, rays_d, n, live, S, head, zh, d, dn, level_stride, have_heads ? 1 : 3,
-                                     tail_pending ? &bar_tail : nullptr, tail_phase);
-        if (tail_pending) { tail_phase ^= 1u; tail_pending = false; }
-
-        // ---- d(loss)/d(pre-activations) of the 7 heads and the 3 specular outputs (column group 0) -> Tdz (= LOb: H_lo /
-        // a4_lo, dead by now: with HEADS every MMA that read H_lo completed before the L3 epilogue and a4_lo is never formed)
-        if (cg == 0) {
-            float dzh[16], dzs[16];
-            float gh[10];
-            if (live) {
-                const float2* gsrc = reinterpret_cast<const float2*>(grad_heads + (size_t)n * 10);
-#pragma unroll
-                for (int j = 0; j < 5; ++j) { const float2 t = __ldg(gsrc + j); gh[2 * j] = t.x * gscale; gh[2 * j + 1] = t.y * gscale; }
-            } else {
-#pragma unroll
-                for (int j = 0; j < 10; ++j) gh[j] = 0.0f;
-            }
-            float spec[3], dsig;
-            if (have_heads) {
-                // activations as the forward stored them: sigma = softplus(z) -> softplus' = sigmoid(z) = 1 - exp(-sigma)
-                float hv[10];
-                if (live) {
-                    const float2* hsrc = reinterpret_cast<const float2*>(heads_fwd + (size_t)n * 10);
-#pragma unroll
-                    for (int j = 0; j < 5; ++j) { const float2 t = __ldg(hsrc + j); hv[2 * j] = t.x; hv[2 * j + 1] = t.y; }
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 10; ++j) hv[j] = 0.0f;
-                }
-                dsig = hv[0] > 20.0f ? 1.0f : -expm1f(-hv[0]);
-#pragma unroll
-                for (int j = 0; j < 3; ++j) { head[1 + j] = hv[1 + j]; head[4 + j] = hv[4 + j]; spec[j] = hv[7 + j]; }
-            } else {
-                float z[16];
-                umma::tmem_ld16(tmem + cDh + lane_addr, z);
-                umma::tc_wait_ld();
-                dsig = zh[0] > 20.0f ? 1.0f : sigmoidf(zh[0]);                  // softplus' = sigmoid
-#pragma unroll
-                for (int j = 0; j < 3; ++j) spec[j] = sigmoidf(z[j] + bias[oB5 + j]);
-            }
-#pragma unroll
-            for (int j = 0; j < 16; ++j) { dzh[j] = 0.0f; dzs[j] = 0.0f; }
-            dzh[0] = gh[0] * dsig;
-#pragma unroll
-            for (int j = 0; j < 3; ++j) {
-                dzh[1 + j] = gh[4 + j] * head[4 + j] * (1.0f - head[4 + j]);    // diffuse
-                dzh[4 + j] = gh[1 + j] * head[1 + j] * (1.0f - head[1 + j]);    // tint
-                dzs[j] = gh[7 + j] * spec[j] * (1.0f - spec[j]);                // specular
-            }
-            // Tdz = [dz_heads 0..15 | dz_spec 16..31 | dz_heads_lo 32..47 | dz_spec_lo 48..63]
-            store8_act<SPLIT>(Tdz, 0, Tdz, 4, row, dzh);
-            store8_act<SPLIT>(Tdz, 1, Tdz, 5, row, dzh + 8);
-            store8_act<SPLIT>(Tdz, 2, Tdz, 6, row, dzs);
-            store8_act<SPLIT>(Tdz, 3, Tdz, 7, row, dzs + 8);
-            // bias gradients of the narrow layers: summed per thread over the CTA's tiles, reduced once at the end
-#pragma unroll
-            for (int j = 0; j < 10; ++j) acc_small[j] += j < 7 ? dzh[j] : dzs[j - 7];
-        }
-        c.sync_operands();
-        if constexpr (HEADS) {
-            // ---- L4 + B1 in one commit group: Db = a3 W4^T ; dA4 = dz_spec W5 ; dH[0:32] = dz_heads Wh ; dWh^T += H^T dz_heads
-            if (lead_warp && umma::elect_one()) {
-                fwd_gemm<SPLIT>(tmem + cDb, aa3, 0, adzlo, 0, aW4, 0, aW4l, 0, 4, idf64, false);      // (adzlo = LOa holds a3_lo)
-                dgrad(cDa, adz, 1, adz, 3, aW5, aW5l, 1, idg64);
-                dgrad(cDc, adz, 0, adz, 2, aWh, aWh + 64, 1, idg32);     // dH[0:32] stays in TMEM until the B2 epilogue
-                umma::mma_commit(&bar);
-                wgrad_t(cGWhT, aH, adz, adz + 64, idwt16, first);        // behind the commit: this epilogue writes a4 / g4 / LOa only
-            }
-            c.wait_mma();
-            {   // a4 = g(z4) (hi part only: no layer reads a4_lo here), dz5 = dA4 * g'(z4) with g' still in registers
-                float z4[16];
-                umma::tmem_ld16(tmem + cDb + lane_addr + 16 * cg, z4);
-                umma::tmem_ld16(tmem + cDa + lane_addr + 16 * cg, v);
-                umma::tc_wait_ld();
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const float z = z4[j] + bias[oB4 + 16 * cg + j];
-                    const float a = gauss_act(z);
-                    z4[j] = a;
-                    v[j] *= -100.0f * z * a;
-                    acc_b4[j] += v[j];
-                }
-#pragma unroll
-                for (int q = 0; q < 2; ++q) {
-                    umma::tile_store8_f16(T.a4, row, 2 * cg + q, z4 + 8 * q);
-                    store8_act<SPLIT>(T.g4, 2 * cg + q, Tdzlo, 2 * cg + q, row, v + 8 * q);
-                }
-            }
-            c.sync_operands();
-            // ---- B2: dA3 = dz5 W4 ; dW4 += dz5^T a3 ; dW5^T += a4^T dz_spec
-            if (lead_warp && umma::elect_one()) {
-                dgrad(cDb, ag4, 0, adzlo, 0, aW4, aW4l, 4, idg64);
-                // in FRONT of the commit: the epilogue overwrites what they read (Tdz with dH, a4 with dH_lo / the dz lo tile)
-                wgrad_t(cGW5T, aa4, adz + 32, adz + 96, idwt16, first);
-                if (SPLIT && kWgradDzLo) wgrad_part(cGW4, adzlo, aa3, idw64, first);
-                umma::mma_commit(&bar);
-                wgrad_part(cGW4, ag4, aa3, idw64, (SPLIT && kWgradDzLo) ? false : first);
-            }
-        } else {
-            // ---- B1: dA4 = dz_spec W5 ; dH[0:32] = dz_heads Wh ; dW5^T += a4^T dz_spec ; dWh^T += H^T dz_heads
-            if (lead_warp && umma::elect_one()) {
-                dgrad(cDa, adz, 1, adz, 3, aW5, aW5l, 1, idg64);
-                dgrad(cDc, adz, 0, adz, 2, aWh, aWh + 64, 1, idg32);     // dH[0:32] stays in TMEM until the B2 epilogue
-                umma::mma_commit(&bar);
-                wgrad_t(cGW5T, aa4, adz + 32, adz + 96, idwt16, first);  // behind the commit: this epilogue writes g4 / dz lo only
-                wgrad_t(cGWhT, aH, adz, adz + 64, idwt16, first);
-            }
-            c.wait_mma();
-            mul_inplace(cDa, T.g4, Tdzlo, acc_b4);                   // dz5 (+ its column sums = d/d b4)
-            c.sync_operands();
-            // ---- B2: dA3 = dz5 W4 ; dW4 += dz5^T a3
-            if (lead_warp && umma::elect_one()) {
-                dgrad(cDb, ag4, 0, adzlo, 0, aW4, aW4l, 4, idg64);
-                // the epilogue overwrites the dz lo tile: its part goes in front of the commit, the hi part behind it
-                if (SPLIT && kWgradDzLo) wgrad_part(cGW4, adzlo, aa3, idw64, first);
-                umma::mma_commit(&bar);
-                wgrad_part(cGW4, ag4, aa3, idw64, (SPLIT && kWgradDzLo) ? false : first);
-            }
-        }
-        c.wait_mma();                                            // (covers the B1 weight-gradient MMAs that read Tdz and a4)
-        store_quarter(cDc, Tdz, Tdhlo, 0, acc_b2);               // dH[0:32] -> dz2 tile columns 0..31 (over the consumed dz_heads/spec)
-        mul_inplace(cDb, T.g3, Tdzlo, nullptr);                  // dz4
-        c.sync_operands();
-        // ---- B3: d[x2] = dz4 W3 ; dW3 += dz4^T [H[32:64] | SH] ; db3
-        if (lead_warp && umma::elect_one()) {
-            dgrad(cDa, ag3, 0, adzlo, 0, aW3, aW3l, 4, idg64);
-            umma::mma_commit(&bar);
-            wgrad(cGW3a, ag3, adzlo, aH + 64, idw32, first);        // behind the commit: the epilogue writes dH only
-            wgrad(cGW3b, ag3, adzlo, aA0 + 64, idw16, first);
-        }
-        c.wait_mma();
-        store_quarter(cDa, Tdz, Tdhlo, 4, acc_b2 + 8);           // dH[32:64]
-        c.sync_operands();
-        // ---- B4: dA1 = dH W2 ; dW2 += dH^T a1 ; db2
-        if (lead_warp && umma::elect_one()) {
-            dgrad(cDb, adz, 0, adhlo, 0, aW2, aW2l, 4, idg64);
-            umma::mma_commit(&bar);
-            wgrad(cGW2, adz, adhlo, aa1, idw64, first);             // behind the commit: the epilogue writes g1 / the dz lo tile
-        }
-        // (runs while the B4 MMAs execute: d[SH] sits in accumulator columns cDa + 32.. until B5 overwrites them)
-        if (grad_rays_d != nullptr && cg == 3) {                 // d/d(ray direction) through the SH encoding (one thread per row)
-            float dsh[16];
-            umma::tmem_ld16(tmem + cDa + lane_addr + 32, dsh);
-            umma::tc_wait_ld();
-            float gx = 0.f, gy = 0.f, gz = 0.f;
-            if (live) {
-                const float inv = 1.0f / (dn + 1e-8f);
-                const float x = d.x * inv, y = d.y * inv, z = d.z * inv;
-                const float xx = x * x, yy = y * y, zz = z * z, xy = x * y, yz = y * z, xz = x * z;
-                const float C1 = 0.4886025119029199f, C2a = 1.0925484305920792f, C2c = 0.31539156525252005f,
-                            C2e = 0.5462742152960396f, C3a = 0.5900435899266435f, C3b = 2.890611442640554f,
-                            C3c = 0.4570457994644658f, C3d = 0.3731763325901154f, C3e = 1.445305721320277f;
-                float vx = 0.f, vy = 0.f, vz = 0.f;
-                vy += dsh[1] * C1; vz += dsh[2] * C1; vx += dsh[3] * C1;
-                vx += dsh[4] * C2a * y; vy += dsh[4] * C2a * x;
-                vy += dsh[5] * -C2a * z; vz += dsh[5] * -C2a * y;
-                vx += dsh[6] * C2c * -2.f * x; vy += dsh[6] * C2c * -2.f * y; vz += dsh[6] * C2c * 4.f * z;
-                vx += dsh[7] * -C2a * z; vz += dsh[7] * -C2a * x;
-                vx += dsh[8] * C2e * 2.f * x; vy += dsh[8] * C2e * -2.f * y;
-                vx += dsh[9] * -C3a * 6.f * xy; vy += dsh[9] * -C3a * (3.f * xx - 3.f * yy);
-                vx += dsh[10] * C3b * yz; vy += dsh[10] * C3b * xz; vz += dsh[10] * C3b * xy;
-                vx += dsh[11] * -C3c * -2.f * xy; vy += dsh[11] * -C3c * (4.f * zz - xx - 3.f * yy); vz += dsh[11] * -C3c * 8.f * yz;
-                vx += dsh[12] * C3d * -6.f * xz; vy += dsh[12] * C3d * -6.f * yz; vz += dsh[12] * C3d * (6.f * zz - 3.f * xx - 3.f * yy);
-                vx += dsh[13] * -C3c * (4.f * zz - 3.f * xx - yy); vy += dsh[13] * -C3c * -2.f * xy; vz += dsh[13] * -C3c * 8.f * xz;
-                vx += dsh[14] * C3e * 2.f * xz; vy += dsh[14] * C3e * -2.f * yz; vz += dsh[14] * C3e * (xx - yy);
-                vx += dsh[15] * -C3a * (3.f * xx - 3.f * yy); vy += dsh[15] * -C3a * -6.f * xy;
-                // v = d / (|d| + eps):  dL/dd = dv / (n+eps) - d (d . dv) / (n (n+eps)^2)
-                const float ddv = d.x * vx + d.y * vy + d.z * vz;
-                const float k2 = dn > 0.f ? ddv * inv * inv / dn : 0.f;
-                gx = (vx * inv - d.x * k2) * ginv; gy = (vy * inv - d.y * k2) * ginv; gz = (vz * inv - d.z * k2) * ginv;
-            }
-            const int ray = live ? n / S : -1;
-            const int ray0 = __shfl_sync(0xffffffffu, ray, 0);
-            if (__all_sync(0xffffffffu, ray == ray0 || ray < 0)) {
-#pragma unroll
-                for (int off = 16; off > 0; off >>= 1) {
-                    gx += __shfl_xor_sync(0xffffffffu, gx, off);
-                    gy += __shfl_xor_sync(0xffffffffu, gy, off);
-                    gz += __shfl_xor_sync(0xffffffffu, gz, off);
-                }
-                if (lane == 0 && ray0 >= 0) {
-                    atomicAdd(grad_rays_d + 3 * (size_t)ray0 + 0, gx);
-                    atomicAdd(grad_rays_d + 3 * (size_t)ray0 + 1, gy);
-                    atomicAdd(grad_rays_d + 3 * (size_t)ray0 + 2, gz);
-                }
-            } else if (live) {
-                atomicAdd(grad_rays_d + 3 * (size_t)ray + 0, gx);
-                atomicAdd(grad_rays_d + 3 * (size_t)ray + 1, gy);
-                atomicAdd(grad_rays_d + 3 * (size_t)ray + 2, gz);
-            }
-        }
-        c.wait_mma();
-        mul_inplace(cDb, T.g1, Tdzlo, nullptr);                  // dz1
-        c.sync_operands();
-        // ---- B5: dx = dz1 W1 (32 columns) ; dW1 += dz1^T x ; db1
-        if (lead_warp && umma::elect_one()) {
-            dgrad(cDa, ag1, 0, adzlo, 0, aW1, aW1 + 64, 4, idg32);
-            umma::mma_commit(&bar);
-            wgrad(cGW1, ag1, adzlo, aA0, idw48, first);             // N = 48: x (32) | SH (16); column 32 -> d/d b1
-            umma::mma_commit(&bar_tail);                            // everything this tile issued
-        }
-        c.wait_mma();
-        umma::tmem_ld8(tmem + cDa + lane_addr + 8 * cg, v);     // d/d x, columns 8 cg .. 8 cg + 7 = levels 4 cg .. 4 cg + 3
-        umma::tc_wait_ld();
-        if (live) {
-#pragma unroll
-            for (int j = 0; j < 8; ++j) v[j] *= mask[8 * cg + j] * ginv;
-            if (level_stride == 0) {
-                float4* dst = reinterpret_cast<float4*>(grad_feats + (size_t)n * 32 + 8 * cg);
-                dst[0] = make_float4(v[0], v[1], v[2], v[3]);
-                dst[1] = make_float4(v[4], v[5], v[6], v[7]);
-            } else {            // level-major [16][N] float2: consecutive samples -> consecutive addresses
-                float2* dst = reinterpret_cast<float2*>(grad_feats) + n;
-#pragma unroll
-                for (int l = 0; l < 4; ++l) dst[(size_t)(4 * cg + l) * level_stride] = make_float2(v[2 * l], v[2 * l + 1]);
-            }
-        }
-        // the next tile overwrites the operand tiles the trailing weight-gradient MMAs read: they are waited for inside the
-        // next forward_tile (after its global loads), or right after the loop
-        tail_pending = true;
-        first = false;
-    }
-    if (tail_pending) {
-        umma::mbar_wait(&bar_tail, tail_phase);
-        umma::tc_fence_after();
-    }
-
-    // ================= flush the weight / bias gradients accumulated in TMEM =================
-    umma::tc_fence_after();
-    if (!first) {           // (a CTA whose tiles were all masked out never initialised its accumulators)
-        // M = 64 accumulators: row m lives in TMEM lane 32*(m/16) + m%16 -> warp q, lanes 0..15 hold rows 16q..16q+15
-        const int m = 16 * (warp & 3) + lane;
-        const bool own = lane < 16 && cg == 0;
-        float w[32];
-        auto flush = [&](int col, int ncols, float* dst, int ld, int col0) {
-            for (int c0 = 0; c0 < ncols; c0 += 32) {
-                const int nc = ncols - c0 >= 32 ? 32 : ncols - c0;
-                if (nc == 32) umma::tmem_ld32(tmem + col + c0 + lane_addr, w);
-                else umma::tmem_ld16(tmem + col + c0 + lane_addr, w);
-                umma::tc_wait_ld();
-                if (own)
-                    for (int j = 0; j < nc; ++j) atomicAdd(dst + (size_t)m * ld + col0 + c0 + j, w[j] * ginv);
-            }
-        };
-        flush(cGW1, 32, gp.W1, 32, 0);
-        flush(cGW2, 64, gp.W2, 64, 0);
-        flush(cGW3a, 32, gp.W3, 48, 0);
-        flush(cGW3b, 16, gp.W3, 48, 32);
-        flush(cGW4, 64, gp.W4, 64, 0);
-        float b8[16];
-        // d/d b1 = column 32 of the [64 x 48] dW1 accumulator, d/d b3 = column 0 of the SH part of dW3, both / SH_0
-        umma::tmem_ld16(tmem + cGW1 + 32 + lane_addr, b8);
-        umma::tc_wait_ld();
-        if (own) atomicAdd(gp.b1 + m, b8[0] * kInvSH0 * ginv);
-        umma::tmem_ld16(tmem + cGW3b + lane_addr, b8);
-        umma::tc_wait_ld();
-        if (own) atomicAdd(gp.b3 + m, b8[0] * kInvSH0 * ginv);
-        // transposed narrow layers: accumulator row = input feature k, column = output o
-        umma::tmem_ld16(tmem + cGWhT + lane_addr, b8);
-        umma::tc_wait_ld();
-        if (own && m < 32) {
-            atomicAdd(gp.Ws + m, b8[0] * ginv);
-            for (int o = 0; o < 3; ++o) { atomicAdd(gp.Wd + o * 32 + m, b8[1 + o] * ginv); atomicAdd(gp.Wt + o * 32 + m, b8[4 + o] * ginv); }
-        }
-        umma::tmem_ld16(tmem + cGW5T + lane_addr, b8);
-        umma::tc_wait_ld();
-        if (own)
-            for (int o = 0; o < 3; ++o) atomicAdd(gp.W5 + o * 64 + m, b8[o] * ginv);
-    }
-    // d/d b2, d/d b4: per-thread column sums -> sum over the 32 rows of the warp -> one atomic per warp and column
-#pragma unroll
-    for (int j = 0; j < 16; ++j) {
-        float t2 = acc_b2[j], t4 = acc_b4[j];
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            t2 += __shfl_xor_sync(0xffffffffu, t2, off);
-            t4 += __shfl_xor_sync(0xffffffffu, t4, off);
-        }
-        if (lane == 0 && !first) {
-            atomicAdd(gp.b2 + (j < 8 ? 8 * cg + j : 32 + 8 * cg + (j - 8)), t2 * ginv);      // store_quarter column mapping
-            atomicAdd(gp.b4 + 16 * cg + j, t4 * ginv);
-        }
-    }
-    if (cg == 0) {
-#pragma unroll
-        for (int j = 0; j < 10; ++j) {
-            float t = acc_small[j];
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) t += __shfl_xor_sync(0xffffffffu, t, off);
-            if (lane == 0 && !first) {
-                float* dst = j == 0 ? gp.bs : (j < 4 ? gp.bd + (j - 1) : (j < 7 ? gp.bt + (j - 4) : gp.b5 + (j - 7)));
-                atomicAdd(dst, t * ginv);
-            }
-        }
-    }
-    umma::tc_fence_before();
-    __syncthreads();
-    if (warp == 0) umma::tmem_free<512>(tmem);
-}
-
-// ------------------------------- backward with layer 2 folded away ------------------------------------------------------
 // Layer 2 of the decoder has NO activation (network.py:160-163: H = W2 h1 + b2 feeds the heads and the directional branch
 // linearly), so it composes with its consumers:
 //     z3 = H[32:64] W3a^T + SH W3b^T + b3 = a1 (W3a W2b)^T + SH W3b^T + (W3a b2b + b3)         W32 := W3a W2b   [64 x 64]
@@ -704,8 +213,8 @@ decoder_bwd_kernel(const float* __restrict__ feats, const float* __restrict__ ma
 //     G  := dz3^T a1 [64 x 64],  Gh := dzh^T a1 [7 x 64]       (the only weight-gradient GEMMs of layers 2 / 3a / heads)
 //     dW3a = G W2b^T + db3 (x) b2b      dWh = Gh W2a^T + dbh (x) b2a      dW2 = [Wh^T Gh ; W3a^T G]      db2 = [Wh^T dbh ; W3a^T db3]
 // where the second line is evaluated ONCE per CTA in fp32 after the last tile (0.3 M multiply-adds).  Per tile that leaves
-// SIX dependent stages (L1 | z3 | L4 + first backward stage | B2 | B3 | B5) instead of the ten of decoder_bwd_kernel<.,false>,
-// nine operand tiles instead of ten, 33 + 42 issue-side MMAs less, and no epilogue at all for H / dH.  W32 / Wh2 are formed in
+// SIX dependent stages (L1 | z3 | L4 + first backward stage | B2 | B3 | B5) instead of the ten of a layer-by-layer recompute
+// and backward, nine operand tiles instead of ten, 33 + 42 issue-side MMAs less, and no epilogue at all for H / dH.  W32 / Wh2 are formed in
 // fp32 from the fp32 parameters when the CTA stages its weights and split hi + lo like every other operand.
 namespace fold {
 constexpr int oW1 = 0, oW32 = 8192, oW32l = 16384, oW3b = 24576, oW4 = 32768, oW4l = 40960, oWh2 = 49152, oWh2l = 51200,
@@ -740,11 +249,15 @@ decoder_bwd_fold_kernel(const float* __restrict__ feats, const float* __restrict
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     uint32_t tail_phase = 0, phase = 0;
     bool tail_pending = false;
-    float gscale = 1.0f, ginv = 1.0f;              // power-of-two scale of the incoming gradient (see decoder_bwd_kernel)
+    // Power-of-two scale of the incoming gradient: max |grad_heads| (bits in *gmax_bits, from grad_absmax_kernel) is
+    // mapped into [0.5, 1), so that the fp16 dz operands keep 15 binary orders of headroom above it for the growth along
+    // the backward chain and 14 (24 with subnormals) below it.  Everything downstream is linear in the gradient:
+    // outputs are multiplied by ginv (exact).  A zero / non-finite maximum leaves the scale at 1.
+    float gscale = 1.0f, ginv = 1.0f;
     if (kOpBf16 == 0 && gmax_bits != nullptr) {
-        const int e = (int)((*gmax_bits >> 23) & 0xffu);
+        const int e = (int)((*gmax_bits >> 23) & 0xffu);            // gmax = m 2^(e - 127), m in [1, 2)
         if (e > 0 && e < 255) {
-            int se = 253 - e;
+            int se = 253 - e;                                        // exponent field of 2^(126 - e): gmax * scale in [0.5, 1)
             se = se < 1 ? 1 : (se > 253 ? 253 : se);
             gscale = __uint_as_float((uint32_t)se << 23);
             ginv = __uint_as_float((uint32_t)(254 - se) << 23);
@@ -1303,10 +816,6 @@ grad_absmax_kernel(const float* __restrict__ g, int N, int S, const unsigned cha
 __device__ unsigned g_gmax_slots[64];      // a ring: concurrent backward launches on different streams use different slots
 int g_gmax_next = 0;
 
-int g_fwd_inflight = 4; // forward tiles in flight per CTA: 4 (in-place operands, per-ray SH term; S >= kMinS4) or 2
-thread_local const unsigned char* t_sample_live = nullptr;     // set by snrf_decoder_bwd_ert around its call of snrf_decoder_bwd
-int g_fwd_fold = 1;     // four-tile forward: layer 2 folded into its consumers (four dependent stages per tile instead of five)
-int g_bwd_merged = 2;   // backward with heads_fwd: 2 = layer 2 folded away (decoder_bwd_fold_kernel), 1 = layer 4 merged with the first backward stage, 0 = everything recomputed
 int g_split = 1;       // 1 = error-compensated bf16x3 operands in the forward GEMMs (default), 0 = plain bf16
 
 template <typename K>
@@ -1317,69 +826,14 @@ int set_smem(K kernel, int bytes, const char* name)
     return 0;
 }
 
-}  // namespace
-
-// ------------------------------- C ABI --------------------------------------
-// 0 = plain bf16 operands (fastest), 1 = bf16x3 split operands in the forward GEMMs (default)
-SNRF_API void snrf_decoder_set_precision(int split) { g_split = split ? 1 : 0; }
-// tuning hook: 1 (default) = the backward uses heads_fwd when given (no heads GEMM / layer 5 in the recompute, layer 4 merged
-// with the first backward stage); 0 = ignore heads_fwd and recompute everything (the round-1 stage sequence)
-SNRF_API void snrf_decoder_set_bwd_merged(int on) { g_bwd_merged = on < 0 ? 0 : (on > 2 ? 2 : on); }
-// tuning hook: 1 (default) = the four-tile forward folds layer 2 into its consumers (decoder_core.cuh: forward_layers4<., FOLD>)
-SNRF_API void snrf_decoder_set_fwd_fold(int on) { g_fwd_fold = on ? 1 : 0; }
-// tuning hook: forward tiles in flight per CTA (4 = default, 2 = the round-1 kernel)
-SNRF_API void snrf_decoder_set_inflight(int n) { g_fwd_inflight = n == 2 ? 2 : 4; }
-
-// params: HOST array of 16 DEVICE pointers in network.ShallowMLP state_dict order
-SNRF_API int snrf_decoder_fwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params,
-                              float* heads_out, int N, int S, int level_major, const unsigned char* ray_valid, void* stream)
-{
-    SNRF_CHECK_ARG(N >= 0 && S > 0, "snrf_decoder_fwd: need N >= 0, S > 0 (N=%d S=%d)", N, S);
-    SNRF_CHECK_ARG(params != nullptr, "snrf_decoder_fwd: params is required");
-    if (N == 0) return 0;
-    DecoderParams p{params[0], params[1], params[2], params[3], params[4], params[5], params[6], params[7],
-                    params[8], params[9], params[10], params[11], params[12], params[13], params[14], params[15]};
-    static bool configured = false;
-    if (!configured) {
-        int rc = set_smem(decoder_fwd_kernel<true>, fwd_smem<true>(), "snrf_decoder_fwd");
-        if (rc == 0) rc = set_smem(decoder_fwd_kernel<false>, fwd_smem<false>(), "snrf_decoder_fwd");
-        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<true, true>, fwd4_smem<true>(), "snrf_decoder_fwd");
-        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<true, false>, fwd4_smem<true>(), "snrf_decoder_fwd");
-        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<false, true>, fwd4_smem<false>(), "snrf_decoder_fwd");
-        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<false, false>, fwd4_smem<false>(), "snrf_decoder_fwd");
-        if (rc) return rc;
-        configured = true;
-    }
-    const int num_tiles = snrf_div_up(N, kRows);
-    cudaStream_t s = (cudaStream_t)stream;
-    int grid = snrf_sm_count();                     // one 16-warp CTA per SM
-    if (g_fwd_inflight == 4 && S >= kMinS4) {       // four tiles in flight each
-        if (grid > (num_tiles + 3) / 4) grid = (num_tiles + 3) / 4;
-#define SNRF_DEC_FWD4(SPLIT, FOLD) decoder_fwd4_kernel<SPLIT, FOLD><<<grid, kThreadsDec, fwd4_smem<SPLIT>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid)
-        if (g_split) { if (g_fwd_fold) SNRF_DEC_FWD4(true, true); else SNRF_DEC_FWD4(true, false); }
-        else         { if (g_fwd_fold) SNRF_DEC_FWD4(false, true); else SNRF_DEC_FWD4(false, false); }
-#undef SNRF_DEC_FWD4
-        SNRF_RETURN_LAUNCH("snrf_decoder_fwd");
-    }
-    if (grid > (num_tiles + 1) / 2) grid = (num_tiles + 1) / 2;   // two tiles in flight each
-    if (g_split)
-        decoder_fwd_kernel<true><<<grid, kThreadsDec, fwd_smem<true>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid);
-    else
-        decoder_fwd_kernel<false><<<grid, kThreadsDec, fwd_smem<false>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid);
-    SNRF_RETURN_LAUNCH("snrf_decoder_fwd");
-}
-
-// Backward of snrf_decoder_fwd.  heads_fwd: the [N,10] output of the forward (NULL: recomputed; with it the per-tile
-// recompute skips the last layer).  grad_heads[N,10] (same column order as heads) ->
-// grad_feats[N,32] (WRITTEN), grad_rays_d[R,3] (ACCUMULATED; may be NULL: the view direction
-// only enters through the SH encoding), grad_params = HOST array of 16 DEVICE pointers,
-// same order and shapes as params (ACCUMULATED).
-SNRF_API int snrf_decoder_bwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params,
-                              const float* grad_heads, float* grad_feats, float* grad_rays_d, float* const* grad_params,
-                              int N, int S, int level_major, const unsigned char* ray_valid, const float* heads_fwd, void* stream)
+// snrf_decoder_bwd / snrf_decoder_bwd_ert; sample_live (may be NULL): the early-ray-termination flags of snrf_composite_fwd_ert
+int decoder_bwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params, const float* grad_heads,
+                float* grad_feats, float* grad_rays_d, float* const* grad_params, int N, int S, int level_major,
+                const unsigned char* ray_valid, const float* heads_fwd, const unsigned char* sample_live, void* stream)
 {
     SNRF_CHECK_ARG(N >= 0 && S > 0, "snrf_decoder_bwd: need N >= 0, S > 0 (N=%d S=%d)", N, S);
     SNRF_CHECK_ARG(params != nullptr && grad_params != nullptr, "snrf_decoder_bwd: params and grad_params are required");
+    SNRF_CHECK_ARG(heads_fwd != nullptr, "snrf_decoder_bwd: heads_fwd (the output of snrf_decoder_fwd) is required");
     if (N == 0) return 0;
     DecoderParams p{params[0], params[1], params[2], params[3], params[4], params[5], params[6], params[7],
                     params[8], params[9], params[10], params[11], params[12], params[13], params[14], params[15]};
@@ -1388,11 +842,7 @@ SNRF_API int snrf_decoder_bwd(const float* feats, const float* mask32, const flo
                    grad_params[12], grad_params[13], grad_params[14], grad_params[15]};
     static bool configured = false;
     if (!configured) {
-        int rc = set_smem(decoder_bwd_kernel<true, true>, bwd_smem<true>(), "snrf_decoder_bwd");
-        if (rc == 0) rc = set_smem(decoder_bwd_kernel<true, false>, bwd_smem<true>(), "snrf_decoder_bwd");
-        if (rc == 0) rc = set_smem(decoder_bwd_kernel<false, true>, bwd_smem<false>(), "snrf_decoder_bwd");
-        if (rc == 0) rc = set_smem(decoder_bwd_kernel<false, false>, bwd_smem<false>(), "snrf_decoder_bwd");
-        if (rc == 0) rc = set_smem(decoder_bwd_fold_kernel<true>, fold::smem_bytes, "snrf_decoder_bwd");
+        int rc = set_smem(decoder_bwd_fold_kernel<true>, fold::smem_bytes, "snrf_decoder_bwd");
         if (rc == 0) rc = set_smem(decoder_bwd_fold_kernel<false>, fold::smem_bytes, "snrf_decoder_bwd");
         if (rc) return rc;
         configured = true;
@@ -1412,19 +862,68 @@ SNRF_API int snrf_decoder_bwd(const float* feats, const float* mask32, const flo
         if (gx > snrf_sm_count() * 8) gx = snrf_sm_count() * 8;
         grad_absmax_kernel<<<gx > 0 ? gx : 1, 256, 0, s>>>(grad_heads, N, S, ray_valid, slot);
     }
-    if (heads_fwd != nullptr && g_bwd_merged == 2) {
-        if (g_split)
-            decoder_bwd_fold_kernel<true><<<grid, kThreadsDec, fold::smem_bytes, s>>>(feats, mask32, rays_d, p, grad_heads, grad_feats, grad_rays_d, g, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid, slot, heads_fwd, t_sample_live);
-        else
-            decoder_bwd_fold_kernel<false><<<grid, kThreadsDec, fold::smem_bytes, s>>>(feats, mask32, rays_d, p, grad_heads, grad_feats, grad_rays_d, g, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid, slot, heads_fwd, t_sample_live);
-        SNRF_RETURN_LAUNCH("snrf_decoder_bwd");
-    }
-    const bool merged = heads_fwd != nullptr && g_bwd_merged;
-#define SNRF_DEC_BWD(SPLIT, HEADS) decoder_bwd_kernel<SPLIT, HEADS><<<grid, kThreadsDec, bwd_smem<SPLIT>(), s>>>(feats, mask32, rays_d, p, grad_heads, grad_feats, grad_rays_d, g, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid, slot, merged ? heads_fwd : nullptr, t_sample_live)
-    if (g_split) { if (merged) SNRF_DEC_BWD(true, true); else SNRF_DEC_BWD(true, false); }
-    else         { if (merged) SNRF_DEC_BWD(false, true); else SNRF_DEC_BWD(false, false); }
-#undef SNRF_DEC_BWD
+    if (g_split)
+        decoder_bwd_fold_kernel<true><<<grid, kThreadsDec, fold::smem_bytes, s>>>(feats, mask32, rays_d, p, grad_heads, grad_feats, grad_rays_d, g, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid, slot, heads_fwd, sample_live);
+    else
+        decoder_bwd_fold_kernel<false><<<grid, kThreadsDec, fold::smem_bytes, s>>>(feats, mask32, rays_d, p, grad_heads, grad_feats, grad_rays_d, g, N, S, num_tiles, level_major ? (long long)N : 0ll, ray_valid, slot, heads_fwd, sample_live);
     SNRF_RETURN_LAUNCH("snrf_decoder_bwd");
+}
+
+}  // namespace
+
+// ------------------------------- C ABI --------------------------------------
+// 0 = plain bf16 operands (fastest), 1 = bf16x3 split operands in the forward GEMMs (default)
+SNRF_API void snrf_decoder_set_precision(int split) { g_split = split ? 1 : 0; }
+
+// params: HOST array of 16 DEVICE pointers in network.ShallowMLP state_dict order
+SNRF_API int snrf_decoder_fwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params,
+                              float* heads_out, int N, int S, int level_major, const unsigned char* ray_valid, void* stream)
+{
+    SNRF_CHECK_ARG(N >= 0 && S > 0, "snrf_decoder_fwd: need N >= 0, S > 0 (N=%d S=%d)", N, S);
+    SNRF_CHECK_ARG(params != nullptr, "snrf_decoder_fwd: params is required");
+    if (N == 0) return 0;
+    DecoderParams p{params[0], params[1], params[2], params[3], params[4], params[5], params[6], params[7],
+                    params[8], params[9], params[10], params[11], params[12], params[13], params[14], params[15]};
+    static bool configured = false;
+    if (!configured) {
+        int rc = set_smem(decoder_fwd_kernel<true>, fwd_smem<true>(), "snrf_decoder_fwd");
+        if (rc == 0) rc = set_smem(decoder_fwd_kernel<false>, fwd_smem<false>(), "snrf_decoder_fwd");
+        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<true>, fwd4_smem<true>(), "snrf_decoder_fwd");
+        if (rc == 0) rc = set_smem(decoder_fwd4_kernel<false>, fwd4_smem<false>(), "snrf_decoder_fwd");
+        if (rc) return rc;
+        configured = true;
+    }
+    const int num_tiles = snrf_div_up(N, kRows);
+    const long long level_stride = level_major ? (long long)N : 0ll;
+    cudaStream_t s = (cudaStream_t)stream;
+    int grid = snrf_sm_count();                     // one 16-warp CTA per SM
+    if (S >= kMinS4) {                              // four tiles in flight each (a tile spans at most kMaxRays4 rays)
+        if (grid > (num_tiles + 3) / 4) grid = (num_tiles + 3) / 4;
+        if (g_split)
+            decoder_fwd4_kernel<true><<<grid, kThreadsDec, fwd4_smem<true>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_stride, ray_valid);
+        else
+            decoder_fwd4_kernel<false><<<grid, kThreadsDec, fwd4_smem<false>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_stride, ray_valid);
+        SNRF_RETURN_LAUNCH("snrf_decoder_fwd");
+    }
+    if (grid > (num_tiles + 1) / 2) grid = (num_tiles + 1) / 2;   // two tiles in flight each
+    if (g_split)
+        decoder_fwd_kernel<true><<<grid, kThreadsDec, fwd_smem<true>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_stride, ray_valid);
+    else
+        decoder_fwd_kernel<false><<<grid, kThreadsDec, fwd_smem<false>(), s>>>(feats, mask32, rays_d, p, heads_out, N, S, num_tiles, level_stride, ray_valid);
+    SNRF_RETURN_LAUNCH("snrf_decoder_fwd");
+}
+
+// Backward of snrf_decoder_fwd.  heads_fwd: the [N,10] output of the forward (required: the backward takes the head
+// activations from it instead of recomputing the last layers).  grad_heads[N,10] (same column order as heads) ->
+// grad_feats[N,32] (WRITTEN), grad_rays_d[R,3] (ACCUMULATED; may be NULL: the view direction
+// only enters through the SH encoding), grad_params = HOST array of 16 DEVICE pointers,
+// same order and shapes as params (ACCUMULATED).
+SNRF_API int snrf_decoder_bwd(const float* feats, const float* mask32, const float* rays_d, const float* const* params,
+                              const float* grad_heads, float* grad_feats, float* grad_rays_d, float* const* grad_params,
+                              int N, int S, int level_major, const unsigned char* ray_valid, const float* heads_fwd, void* stream)
+{
+    return decoder_bwd(feats, mask32, rays_d, params, grad_heads, grad_feats, grad_rays_d, grad_params, N, S, level_major, ray_valid,
+                       heads_fwd, nullptr, stream);
 }
 
 // snrf_decoder_bwd with the per-sample early-ray-termination flags of snrf_composite_fwd_ert (sample_live [N], may be NULL):
@@ -1435,9 +934,6 @@ SNRF_API int snrf_decoder_bwd_ert(const float* feats, const float* mask32, const
                                   int N, int S, int level_major, const unsigned char* ray_valid, const float* heads_fwd,
                                   const unsigned char* sample_live, void* stream)
 {
-    t_sample_live = sample_live;
-    const int rc = snrf_decoder_bwd(feats, mask32, rays_d, params, grad_heads, grad_feats, grad_rays_d, grad_params, N, S, level_major,
-                                    ray_valid, heads_fwd, stream);
-    t_sample_live = nullptr;
-    return rc;
+    return decoder_bwd(feats, mask32, rays_d, params, grad_heads, grad_feats, grad_rays_d, grad_params, N, S, level_major, ray_valid,
+                       heads_fwd, sample_live, stream);
 }

@@ -64,14 +64,9 @@ template <bool SPLIT> constexpr int off_small() { return off_mask<SPLIT>() + 128
 template <bool SPLIT> constexpr int off_tiles() { return ((off_small<SPLIT>() + 64 + 1023) / 1024) * 1024; }
 template <bool SPLIT> constexpr int fwd_tiles() { return SPLIT ? 5 : 3; }     // operand tiles of one in-flight forward tile
 template <bool SPLIT> constexpr int fwd_smem() { return off_tiles<SPLIT>() + 2 * fwd_tiles<SPLIT>() * kTile + 1024; }   // two tiles in flight
-template <bool SPLIT> constexpr int bwd_smem() { return off_tiles<SPLIT>() + 10 * kTile + 1024; }
 
-// TMEM columns: working accumulators, then (backward only) the persistent gradient accumulators
+// TMEM columns of the working accumulators
 constexpr int cDa = 0, cDb = 64, cDh = 128;
-// (cGW1 is 48 wide: x (32) | SH (16) -- its column 32 = SH_0 carries the bias gradient of layer 1, as column 0 of
-// cGW3b does for layer 3)
-constexpr int cGW1 = 144, cGW2 = 192, cGW3a = 256, cGW3b = 288, cGW4 = 304, cGWhT = 368, cGW5T = 384;   // ends at 400
-constexpr int cDc = 416;       // backward: dH[0:32], parked until the B2 epilogue (32 columns)
 
 __device__ __forceinline__ float gauss_act(float v) { return exp2f(v * v * kGaussLog2); }
 __device__ __forceinline__ float sigmoidf(float v) { return 1.0f / (1.0f + __expf(-v)); }
@@ -227,19 +222,17 @@ __device__ __forceinline__ void fwd_gemm(uint32_t d, uint32_t a_hi, int a_hi_k, 
     }
 }
 
-// The tiles one forward pass writes.  Forward kernel: a1 == a3, H == a4, g* unused.
+// The tiles one forward pass writes (a1 and a3 may share a tile, H and a4 likewise).
 struct Tiles {
-    unsigned char *A0, *a1, *g1, *H, *a3, *g3, *a4, *g4, *LOa, *LOb;
+    unsigned char *A0, *a1, *H, *a3, *a4, *LOa, *LOb;
 };
 
-// Thread layout of the decoder kernels: kThreadsDec = 512 threads = 16 warps per CTA, in one of two shapes.
-//   NCG = 4 (backward): ONE 128-row tile per CTA; thread (row, cg), row = 32 (warp & 3) + lane is the sample / TMEM lane
-//            (a warp can only read the TMEM lane quadrant warp % 4), cg = warp >> 2 is the column group: in every
-//            64-wide layer the thread owns columns [16 cg, 16 cg + 16).
-//   NCG = 2 (forward, inference): TWO tiles in flight per CTA; group = warp >> 3 owns a tile (own operand tiles, TMEM
-//            columns, mbarrier and named barrier), its 8 warps form 2 column groups of 32 columns.  While one group
-//            waits for its MMAs the other runs its epilogue (and, in the inference kernel, its table gathers).
-// Either way four warps per scheduler hide the latency a one-thread-per-row layout leaves exposed.
+// Thread layout of the two-tile decoder kernels: kThreadsDec = 512 threads = 16 warps per CTA, TWO tiles in flight per CTA
+// (NCG = 2).  group = warp >> 3 owns a tile (own operand tiles, TMEM columns, mbarrier and named barrier); thread (row, cg),
+// row = 32 (warp & 3) + lane is the sample / TMEM lane (a warp can only read the TMEM lane quadrant warp % 4), the group's
+// 8 warps form 2 column groups cg of 32 columns.  While one group waits for its MMAs the other runs its epilogue (and, in
+// the inference kernel, its table gathers).  Four warps per scheduler hide the latency a one-thread-per-row layout leaves
+// exposed.
 constexpr int kThreadsDec = 512;
 constexpr int kTmemGroup = 160;           // TMEM columns of one in-flight forward tile (cDa, cDb, cDh = 144, padded)
 
@@ -277,12 +270,11 @@ struct Ctx {
         tid = threadIdx.x;
         const int warp = tid >> 5;
         row = 32 * (warp & 3) + (tid & 31);
-        if (NCG == 4) { group = 0; cg = warp >> 2; nthr = kThreadsDec; }
-        else { group = warp >> 3; cg = (warp >> 2) & 1; nthr = kThreadsDec / 2; }
+        group = warp >> 3; cg = (warp >> 2) & 1; nthr = kThreadsDec / 2;
         bar = bars + group;
         bar_id = 1 + group;
         leader_warp = umma::warp_uniform() == group * (kThreadsDec / 64);
-        tmem = tmem_base + (NCG == 4 ? 0 : group * kTmemGroup);
+        tmem = tmem_base + group * kTmemGroup;
         lane_addr = (uint32_t)(32 * (warp & 3)) << 16;
         bias = reinterpret_cast<const float*>(smem + off_bias<SPLIT>());
         mask = reinterpret_cast<const float*>(smem + off_mask<SPLIT>());
@@ -306,37 +298,30 @@ struct Ctx {
     // this thread's W accumulator columns [W cg, W cg + W) of the 64-wide accumulator at `col`
     __device__ __forceinline__ void load_cols(int col, float* v)
     {
-        if (W == 16) umma::tmem_ld16(tmem + col + lane_addr + 16 * cg, v);
-        else umma::tmem_ld32(tmem + col + lane_addr + 32 * cg, v);
+        umma::tmem_ld32(tmem + col + lane_addr + 32 * cg, v);
         umma::tc_wait_ld();
     }
 };
 
 // Operand row of one sample: A0 = [x_hi (0..31) | SH_hi (32..47) | SH_lo (48..63)], LOb = [x_lo (0..31)].
-// Thread (row, cg) stores its 32 / NCG (already masked) features x (chunks (4 / NCG) cg ...) and one SH chunk:
-// NCG = 4: the threads with cg >= 2 store SH chunk cg - 2; NCG = 2: cg stores SH chunk cg.  sh8 = that chunk's 8 values.
+// Thread (row, cg) stores its 32 / NCG (already masked) features x (chunks (4 / NCG) cg ...) and SH chunk cg
+// (sh8 = that chunk's 8 values).
 template <bool SPLIT, int NCG>
 __device__ __forceinline__ void store_input_row(const Tiles& T, int row, int cg, const float* x, const float* sh8)
 {
     constexpr int XC = 4 / NCG;
 #pragma unroll
     for (int q = 0; q < XC; ++q) store8_act<SPLIT>(T.A0, XC * cg + q, T.LOb, XC * cg + q, row, x + 8 * q);
-    const int shc = NCG == 4 ? cg - 2 : cg;
-    if (shc >= 0) {
-        store8_act<SPLIT>(T.A0, 4 + shc, T.A0, 6 + shc, row, sh8);
-        if (!SPLIT) umma::tile_zero8(T.A0, row, 6 + shc);
-    }
+    store8_act<SPLIT>(T.A0, 4 + cg, T.A0, 6 + cg, row, sh8);
+    if (!SPLIT) umma::tile_zero8(T.A0, row, 6 + cg);
 }
 
 // The decoder layers of one tile up to (and including) the L5 GEMM, from operand rows already in
 // A0 / LOb.  Writes the operand tiles; the threads with cg == 0 return sigma/diffuse/tint activated in
 // head[0..6] (torch semantics) and their pre-activations in zh[0..6]; the specular pre-activations are
 // left in TMEM columns cDh..cDh+2.
-// stages = 3: everything; 2: stop after the L4 epilogue; 1 (backward, when the forward's head values are at hand): stop after
-// the L3 epilogue and skip the heads GEMM -- the caller runs layer 4 together with the first backward stage, the last layer's
-// output is only needed for the specular sigmoid, whose derivative follows from the saved head value.
-template <bool SPLIT, bool TRAIN, int NCG>
-__device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& T, float* head, float* zh, int stages = 3)
+template <bool SPLIT, int NCG>
+__device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& T, float* head, float* zh)
 {
     constexpr int W = 64 / NCG, CH = W / 8;
     unsigned char* smem = c.smem;
@@ -359,25 +344,16 @@ __device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& 
         umma::mma_commit(c.bar);
     }
     c.wait_mma();
-    float v[W], g[TRAIN ? W : 1];
-    // Gaussian layer epilogue on this thread's W columns: a = exp(-50 z^2) -> (Ta, lo in Tlo);
-    // TRAIN: g = da/dz = -100 z a -> Tg
-    auto gauss_epilogue = [&](int col, int boff, unsigned char* Ta, unsigned char* Tlo, unsigned char* Tg) {
+    float v[W];
+    // Gaussian layer epilogue on this thread's W columns: a = exp(-50 z^2) -> (Ta, lo in Tlo)
+    auto gauss_epilogue = [&](int col, int boff, unsigned char* Ta, unsigned char* Tlo) {
         c.load_cols(col, v);
 #pragma unroll
-        for (int j = 0; j < W; ++j) {
-            const float z = v[j] + bias[boff + W * cg + j];
-            const float a = gauss_act(z);
-            v[j] = a;
-            if (TRAIN) g[j] = -100.0f * z * a;
-        }
+        for (int j = 0; j < W; ++j) v[j] = gauss_act(v[j] + bias[boff + W * cg + j]);
 #pragma unroll
-        for (int q = 0; q < CH; ++q) {
-            store8_act<SPLIT>(Ta, CH * cg + q, Tlo, CH * cg + q, row, v + 8 * q);
-            if (TRAIN) umma::tile_store8_f16(Tg, row, CH * cg + q, g + 8 * q);   // fp16: |g| <= 6.1, read back element-wise only
-        }
+        for (int q = 0; q < CH; ++q) store8_act<SPLIT>(Ta, CH * cg + q, Tlo, CH * cg + q, row, v + 8 * q);
     };
-    gauss_epilogue(cDa, oB1, T.a1, T.LOa, T.g1);
+    gauss_epilogue(cDa, oB1, T.a1, T.LOa);
     c.sync_operands();
     // ---- L2: Db = h1 W2^T (K = 64)
     if (c.leader()) {
@@ -393,13 +369,13 @@ __device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& 
     c.sync_operands();
     // ---- heads: Dh = H[0:32] Wh^T (K = 32, N = 16);   L3: Da = [H[32:64] | SH] W3^T (K = 48)
     if (c.leader()) {
-        if (stages != 1) fwd_gemm<SPLIT>(tmem + cDh, aH, 0, aLOb, 0, aWh, 0, aWh, 2, 2, id16, false);
+        fwd_gemm<SPLIT>(tmem + cDh, aH, 0, aLOb, 0, aWh, 0, aWh, 2, 2, id16, false);
         fwd_gemm<SPLIT>(tmem + cDa, aH, 2, aLOb, 2, aW3, 0, aW3l, 0, 2, id64, false);
         fwd_gemm<SPLIT>(tmem + cDa, aA0, 2, aA0, 3, aW3, 2, aW3l, 2, 1, id64, true);
         umma::mma_commit(c.bar);
     }
     c.wait_mma();
-    if (cg == 0 && stages != 1) {
+    if (cg == 0) {
         float z[16];
         umma::tmem_ld16(tmem + cDh + lane_addr, z);
         umma::tc_wait_ld();
@@ -412,8 +388,7 @@ __device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& 
             head[1 + j] = sigmoidf(zh[4 + j]);     // tint
         }
     }
-    gauss_epilogue(cDa, oB3, T.a3, T.LOa, T.g3);
-    if (stages == 1) return;
+    gauss_epilogue(cDa, oB3, T.a3, T.LOa);
     c.sync_operands();
     // ---- L4: Db = a3 W4^T (K = 64)
     if (c.leader()) {
@@ -421,8 +396,7 @@ __device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& 
         umma::mma_commit(c.bar);
     }
     c.wait_mma();
-    gauss_epilogue(cDb, oB4, T.a4, T.LOb, T.g4);
-    if (stages == 2) return;
+    gauss_epilogue(cDb, oB4, T.a4, T.LOb);
     c.sync_operands();
     // ---- L5: Dh = a4 W5^T (K = 64, N = 16)
     if (c.leader()) {
@@ -435,16 +409,14 @@ __device__ __forceinline__ void forward_layers(Ctx<SPLIT, NCG>& c, const Tiles& 
 // Training-side input: features from HBM times the level mask, SH of d / (|d| + 1e-8) (network.py:172-190).
 // feats: [N,32] row-major (level_stride = 0) or level-major [16][N] float2 (level_stride = N).
 // d / dn (the ray direction and its norm) are returned to the threads that hold an SH chunk.
-template <bool SPLIT, bool TRAIN, int NCG>
+template <bool SPLIT, int NCG>
 __device__ __forceinline__ void forward_tile(Ctx<SPLIT, NCG>& c, const Tiles& T, const float* __restrict__ feats,
                                              const float* __restrict__ rays_d, int n, bool live, int S, float* head, float* zh,
-                                             f3& d, float& dn, long long level_stride, int stages = 3,
-                                             uint64_t* pending_bar = nullptr, uint32_t pending_phase = 0)
+                                             f3& d, float& dn, long long level_stride)
 {
     constexpr int NX = 32 / NCG;                // features per thread
     const float* mask = c.mask;
     const int cg = c.cg;
-    const int shc = NCG == 4 ? cg - 2 : cg;
     float x[NX], sh[16];
 #pragma unroll
     for (int j = 0; j < NX; ++j) x[j] = 0.0f;
@@ -467,21 +439,13 @@ __device__ __forceinline__ void forward_tile(Ctx<SPLIT, NCG>& c, const Tiles& T,
         }
 #pragma unroll
         for (int j = 0; j < NX; ++j) x[j] *= mask[NX * cg + j];
-        if (shc >= 0) {
-            d = ld3(rays_d + 3 * (size_t)(n / S));
-            dn = sqrtf(d.x * d.x + d.y * d.y + d.z * d.z);
-            const float inv = 1.0f / (dn + 1e-8f);
-            sh16(d.x * inv, d.y * inv, d.z * inv, sh);
-        }
+        d = ld3(rays_d + 3 * (size_t)(n / S));
+        dn = sqrtf(d.x * d.x + d.y * d.y + d.z * d.z);
+        const float inv = 1.0f / (dn + 1e-8f);
+        sh16(d.x * inv, d.y * inv, d.z * inv, sh);
     }
-    // (backward: the previous tile's trailing weight-gradient MMAs still read the operand tiles; they are waited for HERE,
-    // after this tile's global loads have been issued, so the two latencies overlap)
-    if (pending_bar != nullptr) {
-        umma::mbar_wait(pending_bar, pending_phase);
-        umma::tc_fence_after();
-    }
-    store_input_row<SPLIT, NCG>(T, c.row, cg, x, sh + 8 * (shc & 1));
-    forward_layers<SPLIT, TRAIN, NCG>(c, T, head, zh, stages);
+    store_input_row<SPLIT, NCG>(T, c.row, cg, x, sh + 8 * (cg & 1));
+    forward_layers<SPLIT, NCG>(c, T, head, zh);
 }
 
 // =====================================================================================================================
@@ -623,14 +587,14 @@ __device__ void stage_fold_weights4(unsigned char* smem, const DecoderParams& p,
 // The layers of one tile, operands in place in (P, Q) = (hi, lo).  x (already masked) is this thread's whole input row;
 // rb = this row's ray vector W3_sh SH(d) (64 floats in shared memory).  Returns sigma / diffuse / tint activated in
 // head[0..6] and leaves the specular pre-activations in TMEM columns c4Dh .. c4Dh + 2 (after the last wait).
-// FOLD: layer 2 (linear, no activation) is composed into its consumers when the weights are staged (stage_fold_weights4):
+// Layer 2 (linear, no activation) is composed into its consumers when the weights are staged (stage_fold_weights4):
 // the W2 tiles hold W32 = W3[:, 0:32] W2[32:64, :], the Wh tile / the first rows of the W3-lo tile hold Wh2 = Wh W2[0:32, :]
 // (hi / lo), the b3 / head bias slots the composed biases -- z3 and the heads come straight from a1 in ONE stage, H is never
 // formed: four dependent stages per tile instead of five, 12 MMAs and one 64-column epilogue less.
 struct NoHook4 { __device__ __forceinline__ void operator()() const {} };
 // under_l1(): called by every thread of the group right after the L1 MMAs have been issued -- work that is not needed before
 // the z3 epilogue (the per-ray SH vectors rb) runs there instead of in front of the tile's first barrier.
-template <bool SPLIT, bool FOLD = false, class Hook = NoHook4>
+template <bool SPLIT, class Hook = NoHook4>
 __device__ __forceinline__ void forward_layers4(Ctx4& c, unsigned char* smem, unsigned char* P, unsigned char* Q, const float* x,
                                                 const float* rb, float* head, float* zh, Hook under_l1 = Hook())
 {
@@ -638,10 +602,9 @@ __device__ __forceinline__ void forward_layers4(Ctx4& c, unsigned char* smem, un
     const uint32_t tmem = c.tmem, lane_addr = c.lane_addr;
     const float* bias = reinterpret_cast<const float*>(smem + off_bias<SPLIT>());
     const uint32_t aP = umma::smem_u32(P), aQ = umma::smem_u32(Q);
-    const uint32_t aW1 = umma::smem_u32(smem + oW1), aW2 = umma::smem_u32(smem + oW2), aW3 = umma::smem_u32(smem + oW3),
-                   aW4 = umma::smem_u32(smem + oW4), aWh = umma::smem_u32(smem + oWh), aW5 = umma::smem_u32(smem + oW5),
-                   aW2l = umma::smem_u32(smem + oW2l), aW3l = umma::smem_u32(smem + oW3l), aW4l = umma::smem_u32(smem + oW4l),
-                   aW5l = umma::smem_u32(smem + oW5l);
+    const uint32_t aW1 = umma::smem_u32(smem + oW1), aW2 = umma::smem_u32(smem + oW2), aW4 = umma::smem_u32(smem + oW4),
+                   aWh = umma::smem_u32(smem + oWh), aW5 = umma::smem_u32(smem + oW5), aW2l = umma::smem_u32(smem + oW2l),
+                   aW3l = umma::smem_u32(smem + oW3l), aW4l = umma::smem_u32(smem + oW4l), aW5l = umma::smem_u32(smem + oW5l);
     constexpr uint32_t id64 = umma::idesc_f16(128, 64, 0, 0, kOpBf16, kOpBf16), id16 = umma::idesc_f16(128, 16, 0, 0, kOpBf16, kOpBf16);
     // input row, packed: x_hi in columns 0..31 of P, x_lo in columns 32..63 of P
 #pragma unroll
@@ -657,8 +620,8 @@ __device__ __forceinline__ void forward_layers4(Ctx4& c, unsigned char* smem, un
     under_l1();
     c.wait_mma();
     float v[32];
-    // epilogue of a 64-wide layer on this thread's row, 32 columns at a time: v = D + bias (+ extra) -> f(v) -> (P, Q)
-    auto epilogue = [&](int boff, const float* extra, bool gaussian) {
+    // Gaussian epilogue of a 64-wide layer on this thread's row, 32 columns at a time: v = g(D + bias (+ extra)) -> (P, Q)
+    auto epilogue = [&](int boff, const float* extra) {
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
             umma::tmem_ld32(tmem + c4D + lane_addr + 32 * half, v);
@@ -667,33 +630,18 @@ __device__ __forceinline__ void forward_layers4(Ctx4& c, unsigned char* smem, un
             for (int j = 0; j < 32; ++j) {
                 float z = v[j] + bias[boff + 32 * half + j];
                 if (extra != nullptr) z += extra[32 * half + j];
-                v[j] = gaussian ? gauss_act(z) : z;
+                v[j] = gauss_act(z);
             }
 #pragma unroll
             for (int q = 0; q < 4; ++q) store8_act<SPLIT>(P, 4 * half + q, Q, 4 * half + q, row, v + 8 * q);
         }
     };
-    epilogue(oB1, nullptr, true);                                         // a1
+    epilogue(oB1, nullptr);                                               // a1
     c.sync_operands();
-    if (FOLD) {
-        if (c.leader()) {      // heads: Dh = a1 Wh2^T (K = 64, N = 16);  z3: D = a1 W32^T (K = 64)
-            fwd_gemm<SPLIT>(tmem + c4Dh, aP, 0, aQ, 0, aWh, 0, aW3l, 0, 4, id16, false);
-            fwd_gemm<SPLIT>(tmem + c4D, aP, 0, aQ, 0, aW2, 0, aW2l, 0, 4, id64, false);
-            umma::mma_commit(c.bar);
-        }
-    } else {
-        if (c.leader()) {          // L2: D = a1 W2^T (K = 64)
-            fwd_gemm<SPLIT>(tmem + c4D, aP, 0, aQ, 0, aW2, 0, aW2l, 0, 4, id64, false);
-            umma::mma_commit(c.bar);
-        }
-        c.wait_mma();
-        epilogue(oB2, nullptr, false);                                        // H
-        c.sync_operands();
-        if (c.leader()) {          // heads: Dh = H[0:32] Wh^T (K = 32, N = 16);  L3: D = H[32:64] W3[:, 0:32]^T (K = 32)
-            fwd_gemm<SPLIT>(tmem + c4Dh, aP, 0, aQ, 0, aWh, 0, aWh, 2, 2, id16, false);
-            fwd_gemm<SPLIT>(tmem + c4D, aP, 2, aQ, 2, aW3, 0, aW3l, 0, 2, id64, false);
-            umma::mma_commit(c.bar);
-        }
+    if (c.leader()) {          // heads: Dh = a1 Wh2^T (K = 64, N = 16);  z3: D = a1 W32^T (K = 64)
+        fwd_gemm<SPLIT>(tmem + c4Dh, aP, 0, aQ, 0, aWh, 0, aW3l, 0, 4, id16, false);
+        fwd_gemm<SPLIT>(tmem + c4D, aP, 0, aQ, 0, aW2, 0, aW2l, 0, 4, id64, false);
+        umma::mma_commit(c.bar);
     }
     c.wait_mma();
     {
@@ -709,14 +657,14 @@ __device__ __forceinline__ void forward_layers4(Ctx4& c, unsigned char* smem, un
             head[1 + j] = sigmoidf(zh[4 + j]);      // tint
         }
     }
-    epilogue(oB3, rb, true);                                              // a3 (+ the ray's SH term)
+    epilogue(oB3, rb);                                                    // a3 (+ the ray's SH term)
     c.sync_operands();
     if (c.leader()) {          // L4: D = a3 W4^T (K = 64)
         fwd_gemm<SPLIT>(tmem + c4D, aP, 0, aQ, 0, aW4, 0, aW4l, 0, 4, id64, false);
         umma::mma_commit(c.bar);
     }
     c.wait_mma();
-    epilogue(oB4, nullptr, true);                                         // a4
+    epilogue(oB4, nullptr);                                               // a4
     c.sync_operands();
     if (c.leader()) {          // L5: Dh = a4 W5^T (K = 64, N = 16)
         fwd_gemm<SPLIT>(tmem + c4Dh, aP, 0, aQ, 0, aW5, 0, aW5l, 0, 4, id16, false);

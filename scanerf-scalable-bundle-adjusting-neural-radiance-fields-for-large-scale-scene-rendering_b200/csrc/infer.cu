@@ -169,7 +169,7 @@ __device__ __forceinline__ bool eval_tile(Ctx<true, 2>& c, const Tiles& Tl, bool
     }
     store_input_row<true, 2>(Tl, c.row, cg, x, sh + 8 * cg);
     float head[10], zh[7];
-    forward_layers<true, false, 2>(c, Tl, head, zh);
+    forward_layers<true, 2>(c, Tl, head, zh);
     if (cg == 0) {
         float zs[16];
         umma::tmem_ld16(c.tmem + cDh + c.lane_addr, zs);
@@ -206,7 +206,7 @@ __device__ __forceinline__ bool eval_tile(Ctx<true, 2>& c, const Tiles& Tl, bool
     unsigned char* T2 = T1 + kTile;                                                                              \
     unsigned char* LOa = T2 + kTile;                                                                             \
     unsigned char* LOb = LOa + kTile;                                                                            \
-    const Tiles Tl{T0, T1, nullptr, T2, T1, nullptr, T2, nullptr, LOa, LOb};                                     \
+    const Tiles Tl{T0, T1, T2, T1, T2, LOa, LOb};                                                                \
     (void)row; (void)cg;
 
 template <int MODE>
@@ -313,8 +313,8 @@ infer_decode4_kernel(InferArgs a, long long n0, int Nc, const float2* __restrict
             const int nrays = (int)(last_n / a.S) - ray0 + 1;
             const int my_ray = active ? (int)(n / a.S) - ray0 : 0;
             float head[10], zh[7];
-            forward_layers4<true, true>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
-                                        [&]() { ray_vectors4<true>(rb, w3sh, a.rays_d, ray0, nrays, c.gtid); });   // under the L1 MMAs
+            forward_layers4<true>(c, smem, P, Q, x, rb + my_ray * 64, head, zh,
+                                  [&]() { ray_vectors4<true>(rb, w3sh, a.rays_d, ray0, nrays, c.gtid); });   // under the L1 MMAs
             float zs[16];
             umma::tmem_ld16(c.tmem + c4Dh + c.lane_addr, zs);
             umma::tc_wait_ld();

@@ -26,7 +26,7 @@ _timed_events = []          # [(start_event, end_event, units)]
 _UNITS_ARG = {"snrf_hash_fwd": 7, "snrf_hash_bwd": 8, "snrf_field_encode_fwd": 13, "snrf_field_encode_bwd": 16,
               "snrf_field_encode_bwd_adam": 27, "snrf_field_encode_bwd_ert": 16, "snrf_field_encode_bwd_adam_ert": 27}
 _HOST_ONLY = {"snrf_last_error", "snrf_version", "snrf_device_sm_count", "snrf_l2_fetch_granularity", "snrf_hash_set_levels_per_block",
-              "snrf_decoder_set_precision", "snrf_decoder_set_inflight", "snrf_composite_set_fwd_packed", "snrf_decoder_set_fwd_fold", "snrf_decoder_set_bwd_merged", "snrf_infer_set_chunk_log2", "snrf_infer_release_scratch", "snrf_field_set_passes_log2", "snrf_field_set_aggregate_levels", "snrf_field_set_run_length", "snrf_field_set_bwd_impl", "snrf_field_set_fwd_pairing", "snrf_field_set_fwd_l2_policy", "snrf_field_set_fwd_pair_loads", "snrf_field_set_fwd_split_levels", "snrf_field_set_levels_per_group", "snrf_field_set_profile", "snrf_field_last_profile", "snrf_field_last_launch_count", "snrf_field_set_overlap", "snrf_field_set_coarse_concurrent", "snrf_field_set_l2_hints", "snrf_field_set_pdl", "snrf_field_set_persist_mib", "snrf_field_set_occupancy_smem", "snrf_field_set_slice_log2",
+              "snrf_decoder_set_precision", "snrf_composite_set_fwd_packed", "snrf_infer_set_chunk_log2", "snrf_infer_release_scratch", "snrf_field_set_passes_log2", "snrf_field_set_aggregate_levels", "snrf_field_set_run_length", "snrf_field_set_bwd_impl", "snrf_field_set_fwd_pairing", "snrf_field_set_fwd_l2_policy", "snrf_field_set_fwd_pair_loads", "snrf_field_set_fwd_split_levels", "snrf_field_set_levels_per_group", "snrf_field_set_profile", "snrf_field_last_profile", "snrf_field_last_launch_count", "snrf_field_set_overlap", "snrf_field_set_coarse_concurrent", "snrf_field_set_l2_hints", "snrf_field_set_pdl", "snrf_field_set_persist_mib", "snrf_field_set_occupancy_smem", "snrf_field_set_slice_log2",
               "snrf_voxelize_mesh_host"}
 
 

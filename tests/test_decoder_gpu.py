@@ -50,38 +50,32 @@ def _decoder_and_inputs(N, S, seed):
 
 @pytest.mark.parametrize("N,S,masked", [(128, 128, False), (128 * 37 + 5, 64, True), (4096 * 5 + 77, 16, True), (128 * 9, 100, False),
                                         (128 * 700 + 3, 128, False)])
-def test_four_tiles_in_flight_forward_equals_two_tile_forward(N, S, masked):
-    """The forward with four tiles in flight (in-place operand tiles, the SH term of layer 3 added per ray in fp32; with and
-    without layer 2 folded into its consumers) against the round-1 two-tile kernel: same heads (the SH term is exact instead of split-compensated, everything else is the same
-    arithmetic), level-major and row-major inputs, ragged last tile, rays masked out, tiles that straddle many rays."""
+def test_four_tiles_in_flight_forward_equals_one_sample_per_ray_forward(N, S, masked):
+    """The forward with four tiles in flight (in-place operand tiles, layer 2 folded into its consumers, the SH term of layer 3
+    added per ray in fp32) against the same samples restated one per ray (S = 1 < kMinS4: each sample gets its ray's direction
+    and flag), which snrf_decoder_fwd runs on the two-tile kernel.  Both kernels normalise the direction per sample, so the
+    heads agree (the SH term is exact instead of split-compensated, everything else is the same arithmetic): level-major and
+    row-major inputs, ragged last tile, rays masked out, tiles that straddle many rays."""
     load_pkg()
-    import scanerf_b200_capi as capi
     from hashgrid import _field
     dec, params, feats, mask, rays_d = _decoder_and_inputs(N, S, N + 3)
     dev = "cuda:0"
     valid = (torch.rand(rays_d.shape[0], generator=torch.Generator().manual_seed(1)) < 0.7).to(dev) if masked else None
     pd = [p.to(dev) for p in params]
+    d, m = rays_d.to(dev), mask.to(dev)
+    d1 = d.repeat_interleave(S, 0)[:N]
+    valid1 = valid.repeat_interleave(S)[:N] if masked else None
     for lm in (False, True):
         f = feats.to(dev)
         if lm:
             f = f.reshape(N, 16, 2).permute(1, 0, 2).contiguous()
-        outs = []
-        for inflight, fold in ((2, 0), (4, 0), (4, 1)):
-            capi.lib().snrf_decoder_set_inflight(capi.c_int(inflight))
-            capi.lib().snrf_decoder_set_fwd_fold(capi.c_int(fold))
-            outs.append(_field.decoder_forward(f, mask.to(dev), rays_d.to(dev), S, pd, valid))
-        capi.lib().snrf_decoder_set_inflight(capi.c_int(4))
-        capi.lib().snrf_decoder_set_fwd_fold(capi.c_int(1))
+        a = _field.decoder_forward(f, m, d1, 1, pd, valid1)
+        b = _field.decoder_forward(f, m, d, S, pd, valid)
         torch.cuda.synchronize()
-        a = outs[0]
-        for b in outs[1:]:
-            if valid is not None:
-                keep = valid.repeat_interleave(S)[:N]
-                aa, b = a[keep], b[keep]
-            else:
-                aa = a
-            assert bool(torch.isfinite(b).all())
-            assert float((aa - b).abs().max()) < 2e-5, (lm, float((aa - b).abs().max()))
+        if valid is not None:
+            a, b = a[valid1], b[valid1]
+        assert bool(torch.isfinite(b).all())
+        assert float((a - b).abs().max()) < 2e-5, (lm, float((a - b).abs().max()))
 
 
 @pytest.mark.parametrize("split", [True, False])
@@ -111,50 +105,57 @@ def test_decoder_forward_matches_torch(N, S, split):
         assert mean_rel < rel_tol, f"{k}: mean relative err {mean_rel}"
 
 
-@pytest.mark.parametrize("merged", [2, 1, 0])
+@pytest.mark.parametrize("inputs", ["row_major", "level_major", "masked"])
 @pytest.mark.parametrize("split", [True, False])
 @pytest.mark.parametrize("N,S", [(128, 128), (128 * 5 + 17, 32), (4096 * 3, 128)])
-def test_decoder_backward_matches_torch(N, S, split, merged):
-    """merged = 2 (default): layer 2 folded into its consumers (six dependent stages, dW2 / dW3a / dW_heads / db2 composed per
-    CTA); 1: the backward uses the forward's head values (no heads GEMM / layer 5 in the recompute, layer 4 in one commit group
-    with the first backward stage); 0: everything recomputed, the round-1 stage sequence."""
-    import ctypes
+def test_decoder_backward_matches_torch(N, S, split, inputs):
+    """The backward (layer 2 folded into its consumers: six dependent stages per tile, dW2 / dW3a / dW_heads / db2 composed
+    per CTA) against fp32 torch autograd.  inputs: row-major features [N,32]; level-major features [16,N,2] (the layout of the
+    field encode); row-major with every third ray masked out (its samples get no gradient, their grad_feats rows are not
+    compared; at S = 128 such a tile has no live sample)."""
     load_pkg()
-    import scanerf_b200_capi as capi
     from hashgrid import _field
-    capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(merged))
     dec, params, feats, mask, rays_d = _decoder_and_inputs(N, S, N + 1)
     g = torch.Generator().manual_seed(3)
     cot = torch.randn(N, 10, generator=g)
+    valid = live = None
+    if inputs == "masked":
+        valid = torch.arange(rays_d.shape[0]) % 3 != 1
+        live = valid.repeat_interleave(S)[:N]
     # torch reference (fp32, CPU)
     f_ref = feats.clone().requires_grad_(True)
     d_ref = rays_d.clone().requires_grad_(True)
     o = dec(torch.cat([f_ref, d_ref.repeat_interleave(S, 0)[:N]], -1), weight_feature=mask)
     ref_heads = torch.cat([o["sigma"], o["tint"], o["diffuse"], o["specular"]], -1)
-    (ref_heads * cot).sum().backward()
+    (ref_heads * (cot if live is None else cot * live[:, None])).sum().backward()
     # tensor-core path
     dev = "cuda:0"
-    f_gpu = feats.to(dev).requires_grad_(True)
+    f_in = feats.reshape(N, 16, 2).permute(1, 0, 2).contiguous() if inputs == "level_major" else feats
+    f_gpu = f_in.to(dev).requires_grad_(True)
     d_gpu = rays_d.to(dev).requires_grad_(True)
     p_gpu = [p.detach().to(dev).requires_grad_(True) for p in params]
     _field.set_precision(split)
     try:
-        heads = _field.decoder_apply(f_gpu, d_gpu, mask.to(dev), S, p_gpu)
+        heads = _field.decoder_apply(f_gpu, d_gpu, mask.to(dev), S, p_gpu, None if valid is None else valid.to(dev))
         (heads * cot.to(dev)).sum().backward()
         torch.cuda.synchronize()
     finally:
         _field.set_precision(True)
-        capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(2))
 
     def rel(a, b):      # relative error in the L2 sense
         return float((a.cpu() - b).norm() / b.norm().clamp_min(1e-20))
-    errs = {"feats": rel(f_gpu.grad, f_ref.grad), "rays_d": rel(d_gpu.grad, d_ref.grad)}
+    g_feats = f_gpu.grad.permute(1, 0, 2).reshape(N, 32) if inputs == "level_major" else f_gpu.grad
+    if live is None:
+        errs = {"feats": rel(g_feats, f_ref.grad)}
+    else:
+        errs = {"feats": rel(g_feats[live.to(dev)], f_ref.grad[live])}
+    errs["rays_d"] = rel(d_gpu.grad, d_ref.grad)
     for q, p in zip(p_gpu, params):
         errs[f"param{tuple(p.shape)}"] = rel(q.grad, p.grad)
     print(f"decoder bwd split={split} rel L2 errs:", {k: f"{v:.2e}" for k, v in errs.items()})
     # split: every gradient within 2e-3 (the north star's tolerance for the 16-bit operand path): the input-gradient
-    # chain is error-compensated (hi + lo operands), the weight-gradient GEMMs read compensated dz against the fp16 hi
-    # part of the activations (2^-12 operand rounding; round 1's bf16 activations needed a 5e-3 bar here).
+    # chain is error-compensated (hi + lo operands), the weight-gradient GEMMs read the fp16 hi parts of dz and of the
+    # activations (2^-12 operand rounding each; round 1's bf16 activations needed a 5e-3 bar here).
     # plain (hi only) operands: the Gaussian activations amplify operand rounding.
     for k, v in errs.items():
         tol = 2e-3 if split else 2e-1

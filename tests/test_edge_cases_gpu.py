@@ -113,3 +113,19 @@ def test_argument_validation():
     with pytest.raises(RuntimeError):                                # slot out of range
         H.bg_pts_inference_v2(z(1, 3), z(1, 3), z(1, 8), z(1, 4, dtype=torch.int16), 4, sc["corners"], sc["sizes"], sc["res"], sc["tables"],
                               sc["params"], z(1, 8, 3), z(1, 8, 3), z(1, 8, 1))
+    # the decoder backward takes the head activations from the forward's output: heads_fwd = NULL is rejected
+    import ctypes
+    import scanerf_b200_capi as capi
+    from hashgrid._decoder import ShallowMLP, decoder_params
+    from scanerf_b200_capi import c_int, c_void_p, ptr
+    params = [p.detach().to(DEV) for p in decoder_params(ShallowMLP(32))]
+    grads = [torch.zeros_like(p) for p in params]
+    arr = (ctypes.c_void_p * 16)(*[p.data_ptr() for p in params])
+    garr = (ctypes.c_void_p * 16)(*[g.data_ptr() for g in grads])
+    N, S = 256, 128
+    feats, rays_d, g_heads, g_feats = z(N, 32), z(N // S, 3), torch.ones(N, 10, device=DEV), z(N, 32)
+    rc = capi.lib().snrf_decoder_bwd(ptr(feats), c_void_p(0), ptr(rays_d), arr, ptr(g_heads), ptr(g_feats), c_void_p(0), garr,
+                                     c_int(N), c_int(S), c_int(0), c_void_p(0), c_void_p(0), capi.stream())
+    torch.cuda.synchronize()
+    assert rc != 0 and b"heads_fwd" in capi.lib().snrf_last_error()
+    assert all(float(g.abs().max()) == 0.0 for g in grads)

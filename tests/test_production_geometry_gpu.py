@@ -211,34 +211,6 @@ def test_decoder_backward_ert_dead_tiles():
     _check_grads("decoder bwd ert", g_rm, g_d, g_params, want, live)
 
 
-@pytest.mark.parametrize("merged", [1, 0])
-def test_decoder_backward_selectable_arms_at_several_tiles_per_cta(merged):
-    """The backward arms kept selectable (1: forward heads reused, layer 4 merged with the first backward stage; 0: everything
-    recomputed) at about three tiles per CTA, ragged last tile, masked rays."""
-    capi = _capi()
-    from hashgrid import _field
-    N, S_ = N_RAGGED, S_RAGGED
-    tiles, grid = _bwd_geometry(N)
-    assert 3 <= tiles / grid < 4
-    params, feats, mask32, rays_d = _decoder_case(N, S_, 6 + merged)
-    nr = rays_d.shape[0]
-    gd = torch.Generator(device=DEV).manual_seed(7)
-    valid = (torch.arange(nr, device=DEV) * S_ // ROWS % 7 != 3) & (torch.rand(nr, device=DEV, generator=gd) > 0.1)
-    live = valid.repeat_interleave(S_)[:N]
-    cot = torch.randn(N, 10, device=DEV, generator=gd)
-    f = feats.clone().requires_grad_(True)
-    d = rays_d.clone().requires_grad_(True)
-    p = [q.clone().requires_grad_(True) for q in params]
-    capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(merged))
-    try:
-        _field.decoder_apply(f, d, mask32, S_, p, valid).backward(cot)
-        torch.cuda.synchronize()
-    finally:
-        capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(2))
-    want = _reference_decoder(params, feats, mask32, rays_d, S_, cot * live[:, None])
-    _check_grads(f"decoder bwd merged={merged}", f.grad.permute(1, 0, 2).reshape(N, 32), d.grad, [q.grad for q in p], want, live)
-
-
 # ------------------------------------------------------------------------------------------------------------------------
 # B. scatter + Adam at T = 2^24
 # ------------------------------------------------------------------------------------------------------------------------

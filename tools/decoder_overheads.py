@@ -29,10 +29,7 @@ def main():
     params = [p.detach().requires_grad_(True) for p in _decoder.decoder_params(dec)]
     S = 128
     rows = []
-    import ctypes
-    import scanerf_b200_capi as capi
-    for k, merged in ((1, 2), (1, 1), (1, 0), (4, 2), (4, 1), (16, 2), (64, 2), (221, 2)):
-        capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(merged))
+    for k in (1, 4, 16, 64, 221):
         N = 148 * 128 * k
         feats = (torch.randn(16, N, 2, device=dev) * 0.3).requires_grad_(True)
         rays_d = torch.randn(N // S, 3, device=dev)
@@ -64,10 +61,9 @@ def main():
             e = run()
             torch.cuda.synchronize()
             fw.append(f0.elapsed_time(f1)); bw.append(e[0].elapsed_time(e[1]))
-        row = {"bwd_variant": merged, "tiles_per_cta": k, "samples": N, "fwd_ms": sorted(fw)[len(fw) // 2], "bwd_ms_incl_absmax": sorted(bw)[len(bw) // 2]}
+        row = {"tiles_per_cta": k, "samples": N, "fwd_ms": sorted(fw)[len(fw) // 2], "bwd_ms_incl_absmax": sorted(bw)[len(bw) // 2]}
         rows.append(row)
         print(json.dumps(row), flush=True)
-    capi.lib().snrf_decoder_set_bwd_merged(ctypes.c_int(2))
     with open(args.out, "w") as fh:
         fh.write(json.dumps(rows) + "\n")
 
