@@ -135,3 +135,51 @@ def adam_step(params, grads, exp_avg, exp_avg_sq, lr, beta1, beta2, eps, step, r
                            ctypes.c_int(int(half_state)), ctypes.c_float(lr), ctypes.c_float(beta1),
                            ctypes.c_float(beta2), ctypes.c_float(eps), ctypes.c_int(step))
     return p, m, v
+
+
+def _i64(a):
+    return np.ascontiguousarray(a, dtype=np.int64)
+
+
+def _scene(corners, sizes, occupied, starts, log2dim):
+    return _f32(corners), _f32(sizes), _u8(occupied), _i64(starts), _i32(log2dim)
+
+
+def render_sample(rays_o, rays_d, corners, sizes, occupied, starts, log2dim, order, isect, tracing_idx, z_start, z_vals, dists):
+    """One call of the multi-tile render sampler; tracing_idx [B], z_start [B], z_vals / dists [B,S] are updated in place
+    (they must be contiguous int32 / float32 arrays)."""
+    rays_o, rays_d, order, isect = _f32(rays_o), _f32(rays_d), _i32(order), _f32(isect)
+    c, s, occ, st, l2 = _scene(corners, sizes, occupied, starts, log2dim)
+    for a, t in ((tracing_idx, np.int32), (z_start, np.float32), (z_vals, np.float32), (dists, np.float32)):
+        assert a.dtype == t and a.flags.c_contiguous
+    B, nb, S = rays_o.shape[0], c.shape[0], z_vals.shape[1]
+    lib().oracle_render_sample(_p(rays_o), _p(rays_d), _p(c), _p(s), _p(occ), _p(st), _p(l2), _p(order), _p(isect), _p(tracing_idx),
+                               _p(z_start), _p(z_vals), _p(dists), ctypes.c_int(B), ctypes.c_int(nb), ctypes.c_int(S))
+
+
+def firsthit_block(rays_o, rays_d, corners, sizes, occupied, starts, log2dim, order, isect, hit_init=-1):
+    rays_o, rays_d, order, isect = _f32(rays_o), _f32(rays_d), _i32(order), _f32(isect)
+    c, s, occ, st, l2 = _scene(corners, sizes, occupied, starts, log2dim)
+    B, nb = rays_o.shape[0], c.shape[0]
+    hit = np.full(B, hit_init, np.int16)
+    lib().oracle_firsthit_block(_p(rays_o), _p(rays_d), _p(c), _p(s), _p(occ), _p(st), _p(l2), _p(order), _p(isect), _p(hit),
+                                ctypes.c_int(B), ctypes.c_int(nb))
+    return hit
+
+
+def process_occupied(bidx, total_grid, corners, sizes, occupied, starts, log2dim, target):
+    """Returns a copy of `target` (the concatenated grids) with tile bidx's occupied cells dilated into the other tiles."""
+    c, s, occ, st, l2 = _scene(corners, sizes, occupied, starts, log2dim)
+    tgt = _u8(target).copy()
+    lib().oracle_process_occupied(ctypes.c_int(bidx), ctypes.c_int(total_grid), _p(c), _p(s), _p(occ), _p(st), _p(l2), _p(tgt),
+                                  ctypes.c_int(c.shape[0]))
+    return tgt
+
+
+def outgoing_bidx(rays_o, rays_d, corners, sizes, order, isect, skip=False):
+    rays_o, rays_d, corners, sizes, order, isect = _f32(rays_o), _f32(rays_d), _f32(corners), _f32(sizes), _i32(order), _f32(isect)
+    B, nb = order.shape
+    ids, w = np.full((B, 4), -1, np.int16), np.zeros((B, 4), np.float32)
+    lib().oracle_outgoing_bidx(_p(rays_o), _p(rays_d), _p(corners), _p(sizes), _p(order), _p(isect), _p(ids), _p(w),
+                               ctypes.c_int(int(skip)), ctypes.c_int(B), ctypes.c_int(nb))
+    return ids, w

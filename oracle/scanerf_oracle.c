@@ -436,6 +436,251 @@ ORACLE_API void oracle_sample_points_grid(const float *rays_o, const float *rays
     }
 }
 
+/* ------------------------------------------------------------------------- */
+/* 3. multi-tile render tracing (hashgrid/src/rendering_kernel.cu)            */
+/* ------------------------------------------------------------------------- */
+
+#define RENDER_MISS 10000000.0f
+
+/* The scene of the multi-tile renderer: nb tiles (corner, size), their occupancy grids
+ * concatenated at starts[b] with (2^lx, 2^ly, 2^lz) cells; isect[B, nb, 2] = (near, far), 1e7 on a
+ * miss; order[B, nb] = the tiles of each ray near to far. */
+typedef struct {
+    const float *rays_o, *rays_d, *corners, *sizes, *isect;
+    const unsigned char *occ; const long long *starts; const int *log2dim, *order;
+    int *tracing_idx; float *z_start, *z_vals, *dists; short *hit, *ids; float *w;
+    unsigned char *tgt; int nb, S, bidx, skip;
+} trace_ctx_t;
+
+typedef struct { float corner[3], cell[3]; int n[3], ly, lz; const unsigned char *occ; } tile_grid_t;
+
+static void tile_grid(const trace_ctx_t *x, int b, tile_grid_t *g)
+{
+    for (int a = 0; a < 3; ++a) {
+        g->n[a] = 1 << x->log2dim[3 * b + a];
+        g->corner[a] = x->corners[3 * b + a];
+        g->cell[a] = x->sizes[3 * b + a] / (float)g->n[a];
+    }
+    g->ly = x->log2dim[3 * b + 1]; g->lz = x->log2dim[3 * b + 2];
+    g->occ = x->occ + x->starts[b];
+}
+static void tile_walk(const tile_grid_t *g, walk_t *w, const float *o, const float *d, float t_near, float t_far)
+{
+    float ol[3] = {o[0] - g->corner[0], o[1] - g->corner[1], o[2] - g->corner[2]};
+    walk_init(w, ol, d, t_near, t_far, g->n, g->cell);
+}
+static int tile_on(const tile_grid_t *g, const walk_t *w)
+{
+    return g->occ[((uint32_t)w->c[0] << (g->ly + g->lz)) | ((uint32_t)w->c[1] << g->lz) | (uint32_t)w->c[2]] != 0;
+}
+
+/* rendering_kernel.cu:178-382 (sample_points): one call advances every ray to the next tile of its order
+ * that has occupied segments beyond z_start and places S samples there, n = (int)(len / total * S) per
+ * segment, the last segment taking the rest.  The walk starts at the tile's near on a ray's first tile
+ * and at z_start (the previous tile's far) after it.  z_vals / dists keep the caller's fill elsewhere. */
+static void render_sample_range(int i0, int i1, void *vctx)
+{
+    const trace_ctx_t *x = (const trace_ctx_t *)vctx;
+    const int nb = x->nb, S = x->S;
+    for (int i = i0; i < i1; ++i) {
+        const float *o = x->rays_o + 3 * (size_t)i, *d = x->rays_d + 3 * (size_t)i;
+        const int *order = x->order + (size_t)i * nb;
+        const float *isect = x->isect + (size_t)i * nb * 2;
+        float *zr = x->z_vals + (size_t)i * S, *dr = x->dists + (size_t)i * S;
+        int step = x->tracing_idx[i];
+        float t = x->z_start[i];
+        while (step < nb) {
+            const int b = order[step];
+            const float near = isect[2 * b], far = isect[2 * b + 1];
+            if (near == RENDER_MISS) break;
+            if (t >= far) { ++step; continue; }
+            if (step == 0) t = near;
+            tile_grid_t g; walk_t w;
+            tile_grid(x, b, &g);
+            tile_walk(&g, &w, o, d, t, 0.0f);
+            int num_seg = 0; float total = 0.0f;
+            while (!walk_done(&w)) {
+                walk_next(&w);
+                if (tile_on(&g, &w)) { float len = w.t1 - w.t0; if (len > 0) { total += len; ++num_seg; } }
+                walk_step(&w);
+            }
+            if (num_seg == 0) { t = far; ++step; continue; }
+            tile_walk(&g, &w, o, d, t, 0.0f);
+            int num = 0, count = 0;
+            while (!walk_done(&w)) {
+                walk_next(&w);
+                if (tile_on(&g, &w)) {
+                    float len = w.t1 - w.t0;
+                    if (len > 0) {
+                        int n = imin(imax((int)(len / total * (float)S), 1), S - num);
+                        if (count == num_seg - 1) n = S - num;
+                        if (n > 0) {
+                            float interval = (w.t1 - w.t0) / (float)n;        /* uniform_sample_bound_v3 */
+                            for (int k = 0; k < n; ++k) { zr[num + k] = fmaf((float)k, interval, w.t0); dr[num + k] = interval; }
+                        }
+                        num += n; ++count;
+                    }
+                }
+                walk_step(&w);
+            }
+            t = far; ++step;
+            break;
+        }
+        x->tracing_idx[i] = step;
+        x->z_start[i] = t;
+    }
+}
+
+ORACLE_API void oracle_render_sample(const float *rays_o, const float *rays_d, const float *corners, const float *sizes,
+                                     const unsigned char *occ, const long long *starts, const int *log2dim,
+                                     const int *order, const float *isect, int *tracing_idx, float *z_start,
+                                     float *z_vals, float *dists, int B, int nb, int S)
+{
+    trace_ctx_t x; memset(&x, 0, sizeof(x));
+    x.rays_o = rays_o; x.rays_d = rays_d; x.corners = corners; x.sizes = sizes; x.occ = occ; x.starts = starts;
+    x.log2dim = log2dim; x.order = order; x.isect = isect; x.tracing_idx = tracing_idx; x.z_start = z_start;
+    x.z_vals = z_vals; x.dists = dists; x.nb = nb; x.S = S;
+    parallel_for(B, render_sample_range, &x);
+}
+
+/* rendering_kernel.cu:704-812 (ray_firsthit_block): the tile with the nearest far among the tiles whose
+ * walk from near meets an occupied cell; else, where hit[i] is still -1, the last tile the ray enters. */
+static void firsthit_range(int i0, int i1, void *vctx)
+{
+    const trace_ctx_t *x = (const trace_ctx_t *)vctx;
+    const int nb = x->nb;
+    for (int i = i0; i < i1; ++i) {
+        const float *o = x->rays_o + 3 * (size_t)i, *d = x->rays_d + 3 * (size_t)i;
+        const int *order = x->order + (size_t)i * nb;
+        const float *isect = x->isect + (size_t)i * nb * 2;
+        float dis = RENDER_MISS;
+        int last = -1;
+        for (int s = 0; s < nb; ++s) {
+            const int b = order[s];
+            const float near = isect[2 * b], far = isect[2 * b + 1];
+            if (near == RENDER_MISS) break;
+            tile_grid_t g; walk_t w;
+            tile_grid(x, b, &g);
+            tile_walk(&g, &w, o, d, near, far);
+            int any = 0;
+            while (!walk_done(&w)) {
+                walk_next(&w);
+                if (tile_on(&g, &w)) { any = 1; break; }
+                walk_step(&w);
+            }
+            if (any && dis > far) { x->hit[i] = (short)b; dis = far; }
+            last = b;
+        }
+        if (last != -1 && x->hit[i] == -1) x->hit[i] = (short)last;
+    }
+}
+
+ORACLE_API void oracle_firsthit_block(const float *rays_o, const float *rays_d, const float *corners, const float *sizes,
+                                      const unsigned char *occ, const long long *starts, const int *log2dim,
+                                      const int *order, const float *isect, short *hit, int B, int nb)
+{
+    trace_ctx_t x; memset(&x, 0, sizeof(x));
+    x.rays_o = rays_o; x.rays_d = rays_d; x.corners = corners; x.sizes = sizes; x.occ = occ; x.starts = starts;
+    x.log2dim = log2dim; x.order = order; x.isect = isect; x.hit = hit; x.nb = nb;
+    parallel_for(B, firsthit_range, &x);
+}
+
+/* rendering_kernel.cu:1478-1565 (process_occupied_grid): each occupied cell of tile bidx (cell index t in
+ * [0, total_grid), decomposed with bidx's own grid) marks, in every other tile b, the cell of b's grid that
+ * holds each of its eight corners, if that corner lies in [0, 1)^3 of b.  The cell origin float(i) * cell +
+ * corner is one FMA under nvcc's contraction.  Runs over the target tiles so that no two threads write
+ * the same grid. */
+static void occupied_range(int b0, int b1, void *vctx)
+{
+    const trace_ctx_t *x = (const trace_ctx_t *)vctx;
+    const int bidx = x->bidx;
+    tile_grid_t src;
+    tile_grid(x, bidx, &src);
+    const int ry = src.n[1], rz = src.n[2], total = x->S;
+    for (int b = b0; b < b1; ++b) {
+        if (b == bidx) continue;
+        const float *c = x->corners + 3 * b, *sz = x->sizes + 3 * b;
+        const int *l = x->log2dim + 3 * b;
+        unsigned char *tg = x->tgt + x->starts[b];
+        for (int t = 0; t < total; ++t) {
+            if (!src.occ[t]) continue;
+            const int ix0 = t / (ry * rz), rem = t - ix0 * (ry * rz), iy0 = rem / rz, iz0 = rem % rz;
+            const float p0[3] = {fmaf((float)ix0, src.cell[0], src.corner[0]), fmaf((float)iy0, src.cell[1], src.corner[1]),
+                                 fmaf((float)iz0, src.cell[2], src.corner[2])};
+            for (int j = 0; j < 8; ++j) {
+                const int v[3] = {(j >> 2) & 1, (j >> 1) & 1, j & 1};
+                float q[3]; int inside = 1, id[3];
+                for (int a = 0; a < 3; ++a) {
+                    q[a] = (fmaf((float)v[a], src.cell[a], p0[a]) - c[a]) / sz[a];
+                    inside &= q[a] >= 0 && q[a] < 1;
+                }
+                if (!inside) continue;
+                for (int a = 0; a < 3; ++a) id[a] = (int)(q[a] * (float)(1 << l[a]));
+                tg[(id[0] << (l[1] + l[2])) | (id[1] << l[2]) | id[2]] = 1;
+            }
+        }
+    }
+}
+
+ORACLE_API void oracle_process_occupied(int bidx, int total_grid, const float *corners, const float *sizes,
+                                        const unsigned char *occ, const long long *starts, const int *log2dim,
+                                        unsigned char *tgt, int nb)
+{
+    trace_ctx_t x; memset(&x, 0, sizeof(x));
+    x.corners = corners; x.sizes = sizes; x.occ = occ; x.starts = starts; x.log2dim = log2dim; x.tgt = tgt;
+    x.bidx = bidx; x.S = total_grid; x.nb = nb;
+    parallel_for(nb, occupied_range, &x);
+}
+
+/* rendering_kernel.cu:1262-1401 (update_outgoing_bidx): the tiles sharing the largest far among those the
+ * ray enters (without skip: up to the first tile that starts beyond the current far), at most 4; one tile
+ * gets weight 1, several get the x / z face distances of the exit point o + far d (one FMA) in each. */
+static void outgoing_range(int i0, int i1, void *vctx)
+{
+    const trace_ctx_t *x = (const trace_ctx_t *)vctx;
+    const int nb = x->nb;
+    for (int i = i0; i < i1; ++i) {
+        const int *order = x->order + (size_t)i * nb;
+        const float *isect = x->isect + (size_t)i * nb * 2;
+        float far = -1.0f;
+        int index = 0, cur[4] = {-1, -1, -1, -1};
+        for (int s = 0; s < nb; ++s) {
+            const int b = order[s];
+            const float n = isect[2 * b], f = isect[2 * b + 1];
+            if (n == RENDER_MISS) break;
+            if (!x->skip && (n > far && far != -1.0f)) break;
+            if (f > far) { far = f; cur[0] = b; cur[1] = cur[2] = cur[3] = -1; index = 1; }
+            else if (f == far && index < 4) cur[index++] = b;
+        }
+        if (far == -1.0f) continue;
+        short *ob = x->ids + (size_t)i * 4;
+        float *ow = x->w + (size_t)i * 4;
+        if (index == 1) { ow[0] = 1.0f; ob[0] = (short)cur[0]; continue; }
+        const float *o = x->rays_o + 3 * (size_t)i, *d = x->rays_d + 3 * (size_t)i;
+        const float p[3] = {fmaf(far, d[0], o[0]), fmaf(far, d[1], o[1]), fmaf(far, d[2], o[2])};
+        for (int k = 0; k < 4 && cur[k] != -1; ++k) {
+            const int b = cur[k];
+            float dis[3];
+            for (int a = 0; a < 3; ++a) {
+                const float sz = x->sizes[3 * b + a];
+                const float q = clampf((p[a] - x->corners[3 * b + a]) / sz, 0.0f, 1.0f);
+                dis[a] = (0.5f - fabsf(q - 0.5f)) * sz;
+            }
+            ow[k] = dis[0] != 0 && dis[2] != 0 ? dis[0] * dis[2] : (dis[0] != 0 ? dis[0] : (dis[2] != 0 ? dis[2] : 0.0f));
+            ob[k] = (short)b;
+        }
+    }
+}
+
+ORACLE_API void oracle_outgoing_bidx(const float *rays_o, const float *rays_d, const float *corners, const float *sizes,
+                                     const int *order, const float *isect, short *ids, float *w, int skip, int B, int nb)
+{
+    trace_ctx_t x; memset(&x, 0, sizeof(x));
+    x.rays_o = rays_o; x.rays_d = rays_d; x.corners = corners; x.sizes = sizes; x.order = order; x.isect = isect;
+    x.ids = ids; x.w = w; x.skip = skip; x.nb = nb;
+    parallel_for(B, outgoing_range, &x);
+}
+
 /* cuda/sample_kernel.cu:17-44 + uniform_sample_bound (cuda_utils.h:77-87) */
 ORACLE_API void oracle_background_sampling(const float *starts, const float *bg_depth, float *z_vals,
                                            int B, int S, float range)

@@ -363,7 +363,7 @@ struct Work {
     float4* row_uw;                                // [max_rows] table coordinate u, blend weight w
     float* row_scale;                              // [max_rows] alpha scale (step length x |d|, or the bg step)
     int* pair_row;                                 // [Nc][4] row of the pair in slot s (-1: none)
-    float* wsum;                                   // [Nc] sum of the member weights (< 0: leave the caller's rows alone)
+    float* wsum;                                   // [Nc] sum of the member weights (slot mode, -1: leave the caller's rows alone)
     float2* feats;                                 // [16][max_rows]
     float4* rowout;                                // [max_rows][2] w * alpha * (diffuse, specular), w * alpha
     int max_rows;
@@ -551,7 +551,9 @@ work_combine_kernel(InferArgs a, long long n0, int Nc, Work w)
 {
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < Nc; i += gridDim.x * blockDim.x) {
         const float wsum = w.wsum[i];
-        if (wsum < 0.0f) continue;                             // background ray without a tile in this slot
+        // background ray without a tile in this slot.  Only the slot mode marks that with a negative sum: a foreground sample
+        // a rounding error outside its tile has a negative face weight, and its row is written like any other.
+        if (MODE == kBackSlot && wsum < 0.0f) continue;
         const int4 rows4 = *reinterpret_cast<const int4*>(w.pair_row + (size_t)i * kMaxPts);
         const int rows[kMaxPts] = {rows4.x, rows4.y, rows4.z, rows4.w};
         f3 acc_d = mk3(0, 0, 0), acc_s = mk3(0, 0, 0);

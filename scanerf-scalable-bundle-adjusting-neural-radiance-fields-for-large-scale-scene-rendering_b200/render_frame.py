@@ -101,7 +101,9 @@ def render_rays(ts, rays_o, rays_d, num_sample=128, num_bg_sample=128, sample_ra
     adaptive (scenes of several tiles): read the number of tracing rounds (the most tiles any ray crosses) and of
     background slots in use back from the device, as the reference does (rendering.py:318-320, 470) -- two host
     synchronisations per call that save the empty rounds.  adaptive=False runs the worst-case counts and never
-    synchronises (for callers that pipeline frames or capture the call in a CUDA graph)."""
+    synchronises (for callers that pipeline frames or capture the call in a CUDA graph); both give the same image.
+    The slots in use are counted by tile id, not by positive weight as at rendering.py:470: an exit tile whose exit
+    point lies on one of its x-z edges has weight 0 and can precede a weighted slot, which that count would drop."""
     dev, B, nb = rays_o.device, rays_o.shape[0], ts.num_tiles
     f32 = torch.float32
     intersections = torch.full((B, nb, 2), MISS, dtype=f32, device=dev)
@@ -140,7 +142,7 @@ def render_rays(ts, rays_o, rays_d, num_sample=128, num_bg_sample=128, sample_ra
     bg_zv = torch.empty(B, num_bg_sample, dtype=f32, device=dev)
     n_bg = min(4, nb)                     # at most min(4, tiles) exit tiles share the farthest face
     if adaptive and nb > 1:
-        n_bg = int((bg_w > 0).sum(-1).max())
+        n_bg = int((bg_bidxs >= 0).sum(-1).max())      # the exit tiles fill the slots from 0
     for i in range(n_bg):
         bg_zv.fill_(-1.0); pts_d.zero_(); pts_s.zero_(); pts_a.zero_()
         ops.inverse_z_sampling(intersections, bg_bidxs[..., i].contiguous(), bg_zv, sample_range)

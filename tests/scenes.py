@@ -38,6 +38,21 @@ def occupancy(log2dim, gen, p=0.3):
     return torch.rand(shape, generator=gen) < p
 
 
+def tracing_layout(gen):
+    """Four renderer tiles (foreground boxes, corner + size) along x with one grid resolution each, so that the grid
+    offsets are uneven: 0 and 1 overlap on x in [6, 8], 1 and 2 share the face x = 14, and 3 lies beyond a gap
+    (x in [22, 26]).  Occupancy: tile 1 all set, tile 2 all empty, tiles 0 and 3 about 45 % random.  Returns
+    corners [4,3], sizes [4,3], log2dim [4,3] (int32), the concatenated grids (bool), their starts (int64)."""
+    corners = torch.tensor([[0.0, 0.0, 0.0], [6.0, 0.0, 2.0], [14.0, 0.0, 2.0], [26.0, 0.0, -1.0]])
+    sizes = torch.tensor([[8.0, 6.0, 8.0], [8.0, 6.0, 8.0], [8.0, 6.0, 8.0], [8.0, 6.0, 12.0]])
+    log2dim = torch.tensor([[3, 2, 3], [4, 2, 3], [3, 3, 4], [2, 2, 2]], dtype=torch.int32)
+    grids = [occupancy(l, gen, p=0.45).reshape(-1) for l in log2dim]
+    grids[1][:] = True
+    grids[2][:] = False
+    n = [int(g.numel()) for g in grids]
+    return corners, sizes, log2dim, torch.cat(grids), torch.tensor(np.cumsum([0] + n)[:-1], dtype=torch.int64)
+
+
 def write_proxy_mesh_ply(path, corner, size, seed=0, n_boxes=20, ground_res=64):
     """Procedural proxy mesh for a tile: a gently rolling heightfield ground over the tile
     footprint (y is up, ground near the tile floor) plus `n_boxes` axis-aligned boxes standing

@@ -118,3 +118,55 @@ def test_render_oracle_invariants():
     ids, w = rr.update_outgoing_bidx(np.zeros((1, 3), np.float32), np.array([[1.0, 0, 0]], np.float32), np.zeros((2, 3), np.float32),
                                      np.ones((2, 3), np.float32), np.array([[0, 1]], np.int32), np.array([[[0, 2.0], [1.0, 3.0]]], np.float32))
     assert ids[0, 0] == 1 and w[0, 0] == 1.0
+
+
+def test_tracing_restatements_agree():
+    """The C restatements of the multi-tile render tracing stages (sampler, first hit, occupancy dilation, exit tiles)
+    and the vectorised forms of the simple stages against the loop forms of oracle/render_ref.py, on the tiles of
+    scenes.tracing_layout (overlap, shared face, gap, uneven grids) and a few hundred rays from inside, outside and
+    beyond the tiles.  Tile ids and tracing state bit-exact; depths within 1e-6 relative."""
+    from oracle import render_ref as rr
+    g = torch.Generator().manual_seed(5)
+    corners, sizes, l2d, occ, starts = (t.numpy() for t in scenes.tracing_layout(g))
+    B, S, nb = 300, 16, 4
+    o, d = scenes.random_rays(B, g, [-4.0, -1.0, -3.0], [40.0, 8.0, 16.0], inside=True)
+    o, d = o.numpy(), d.numpy()
+    isect = np.where(on.ray_aabb(o, d, corners + sizes / 2, sizes) == -1, np.float32(1e7), on.ray_aabb(o, d, corners + sizes / 2, sizes))
+    assert np.array_equal(isect, rr.ray_block_intersection(o, d, corners, sizes))
+    order = np.argsort(isect[..., 0], -1, kind="stable").astype(np.int32)
+    assert (isect[..., 0] != 1e7).sum(-1).max() >= 3 and (isect[..., 0] == 1e7).all(-1).any()
+    fake = occ.astype(np.uint8)
+    for b in range(nb):
+        got = on.process_occupied(b, int(2 ** l2d[b].sum()), corners, sizes, occ, starts, l2d, fake)
+        want = rr.process_occupied_grid(b, corners, sizes, occ, starts, l2d, fake)
+        assert np.array_equal(got, want), f"process_occupied tile {b}"
+        fake = got
+    assert fake[starts[2]:starts[3]].any() and (fake >= occ).all()
+    ti, zs = np.zeros(B, np.int32), np.zeros(B, np.float32)
+    for _ in range(nb):
+        z, di = np.full((B, S), -1, np.float32), np.full((B, S), -1, np.float32)
+        wti, wzs, wz, wdi = rr.sample_points(o, d, corners, sizes, fake, starts, l2d, order, isect, ti, zs, S)
+        on.render_sample(o, d, corners, sizes, fake, starts, l2d, order, isect, ti, zs, z, di)
+        assert np.array_equal(ti, wti) and np.array_equal(z == -1, wz == -1)
+        for x, y in ((zs, wzs), (z, wz), (di, wdi)):
+            assert np.allclose(x, y, rtol=1e-6, atol=0)
+        running = ti < nb
+        assert np.array_equal(rr.prepare_points_vec(z, running, isect), rr.prepare_points(z, running, isect))
+    assert np.array_equal(ti, (isect[..., 0] != 1e7).sum(-1)), "after nb calls every ray stops at its first missed tile"
+    assert np.array_equal(on.firsthit_block(o, d, corners, sizes, fake, starts, l2d, order, isect),
+                          rr.ray_firsthit_block(o, d, corners, sizes, fake, starts, l2d, order, isect))
+    assert np.array_equal(rr.get_last_block_vec(order, isect), rr.get_last_block(order, isect))
+    ids, w = on.outgoing_bidx(o, d, corners, sizes, order, isect)
+    wids, ww = rr.update_outgoing_bidx(o, d, corners, sizes, order, isect)
+    assert np.array_equal(ids, wids) and np.allclose(w, ww, rtol=1e-4, atol=1e-5)      # the loop form rounds o + far d twice
+    assert (ids[:, 1] >= 0).any()
+    z = rr.inverse_z_vec(isect, ids[:, 0], 12, 1e6, np.full((B, 12), -1, np.float32))
+    wz = rr.inverse_z_sampling(isect, ids[:, 0], 12, 1e6)
+    assert np.array_equal(z == -1, wz == -1) and np.allclose(z, wz, rtol=1e-5)
+    rng = np.random.default_rng(0)
+    pd, ps, pa = rng.random((B, S, 3), np.float32), rng.random((B, S, 3), np.float32), rng.random((B, S, 1), np.float32) * 0.3
+    init = [rng.random((B, 1), np.float32), rng.random((B, 3), np.float32), rng.random((B, 3), np.float32), rng.random((B, 1), np.float32)]
+    init[0][::7] = 1e-6
+    zz = np.repeat(z, 2, 1)[:, :S]
+    for x, y in zip(rr.accumulate64(pd, ps, pa, init[0], zz, *init[1:]), rr.accumulate_color(pd, ps, pa, init[0], zz, *init[1:])):
+        assert np.allclose(x.reshape(y.shape), y, rtol=1e-5, atol=1e-5)

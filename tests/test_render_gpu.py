@@ -266,7 +266,8 @@ def field_restatement(mode, sc, o, d, z, dist, slots, blend=None, step=0):
             else:
                 q = np.float32(2) * (p[n] - bc) / bs - np.float32(1)
                 nrm = np.abs(q).max(-1, keepdims=True)
-                assert (nrm > 1).all(), "background samples lie outside the tile (u in [0, 1])"
+                # the first inverse-z sample sits on the exit face: nrm = 1 up to the rounding of 1 / (1 / far) and o + z d
+                assert (nrm >= 1 - 1e-5).all(), "background samples lie on or outside the tile (u in [0, 1])"
                 u = _fma(q, (np.float32(2) - np.float32(1) / nrm) / nrm, 2) * np.float32(0.25)
                 w = blend.numpy()[ray[n], s] if mode == "blend" else np.ones(len(n), np.float32)
                 active = np.ones(len(n), bool)
@@ -345,6 +346,35 @@ def test_pts_inference_against_cpu_restatement(mode, nb, B, S):
     for name, x, y in zip(("diffuse", "specular", "alpha"), got, (want_d, want_s, want_a)):
         err = float((x.double()[m] - torch.from_numpy(y)[m]).abs().max()) if bool(m.any()) else 0.0
         assert err < 1e-4, f"{mode} {name}: max abs err {err}"
+
+
+@pytest.mark.parametrize("nb", [1, 3])
+def test_pts_inference_writes_samples_with_a_negative_weight_sum(nb):
+    """Foreground samples a rounding error outside their tile's x = 0 face have a negative face weight (dis.x < 0 < dis.z)
+    and so a negative weight sum, which the reference leaves unnormalised.  Their rows are written like any other, on the
+    single-tile path (nb = 1) and the multi-tile work list (nb = 3), and equal field_restatement within 1e-4."""
+    ours, _ = _ops()
+    sc = make_scene(nb, seed=31)
+    scd = dev(sc)
+    B = 512
+    g = torch.Generator().manual_seed(31)
+    o = torch.stack([torch.full((B,), -1.0), 0.5 + 5 * torch.rand(B, generator=g), 0.5 + 11 * torch.rand(B, generator=g)], -1).contiguous()
+    d = torch.tensor([[1.0, 0.0, 0.0]]).expand(B, 3).contiguous()
+    z = torch.tensor([1 - 2e-6, 1 - 1e-6, 1 - 5e-7, 1.0, 1 + 1e-6, 3.3, 6.1, 9.7]).expand(B, 8).contiguous()
+    dist = torch.full((B, 8), 0.05)
+    slots = torch.full((B, 8, 4), -1, dtype=torch.int16)
+    slots[..., 0] = 0
+    outs = [torch.full((B, 8, 3), 7.0, device=DEV), torch.full((B, 8, 3), 7.0, device=DEV), torch.full((B, 8, 1), 7.0, device=DEV)]
+    ours.pts_inference(o.to(DEV), d.to(DEV), z.to(DEV), dist.to(DEV), slots.to(DEV), scd["tables"], scd["params"], scd["res"], scd["occ"],
+                       scd["starts"], scd["l2d"], scd["corners"], scd["sizes"], *outs)
+    torch.cuda.synchronize()
+    got = [t.cpu() for t in outs]
+    want = field_restatement("fore", sc, o, d, z, dist, slots)[:3]
+    assert (want[2][:, :3] < 0).any(), "some evaluated samples outside the face carry a negative weight"
+    for name, x, y in zip(("diffuse", "specular", "alpha"), got, want):
+        assert bool((x != 7.0).all()), f"{name}: every sample row is written"
+        err = float((x.double() - torch.from_numpy(y)).abs().max())
+        assert err < 1e-4, f"{name}: max abs err {err}"
 
 
 def _render_with(mod, sc, o, d, S, Sb):
