@@ -18,6 +18,8 @@
 #ifndef SCANERF_B200_H
 #define SCANERF_B200_H
 
+#include <stddef.h>
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -393,6 +395,17 @@ int snrf_adam_step(float* params, float* grads, void* exp_avg, void* exp_avg_sq,
                    long long rows, int dim, int row_stride, int half_state,
                    float lr, float beta1, float beta2, float eps, int step, int zero_grad,
                    void* stream);
+
+/* ---- image-quality metrics ---------------------------------------------------------- */
+/* tile.py:810-864 / rendering.py val mode score held-out views on the host (tools/ssim.py); here on the device.
+ * pred[N,H,W,3] f32; gt[N,H,W,3] u8 (gt_is_u8=1, read as (float)v / 255.0f) or f32 (gt_is_u8=0);
+ * mask[N,H,W] bytes, non-zero = score the pixel (NULL = every pixel).
+ * -> out_mse[N], out_ssim[N]: means over the masked pixels and the 3 channels (NaN when no pixel is masked in),
+ *    out_count[N]: masked pixels.  SSIM: 11x11 Gaussian window (sigma 1.5), zero padding, C1 = 0.01^2, C2 = 0.03^2
+ *    (pytorch-ssim; the mask selects map values, it does not change the local statistics).
+ * scratch: N * ceil(H/16) * ceil(W/32) * 3 doubles of device memory.  Deterministic: the same inputs give the same bits. */
+int snrf_image_metrics(const float* pred, const void* gt, int gt_is_u8, const unsigned char* mask, int N, int H, int W,
+                       float* out_mse, float* out_ssim, float* out_count, void* scratch, size_t scratch_bytes, void* stream);
 
 /* ---- ray <-> proxy mesh (fastMesh) --------------------------------------------- */
 /* fastMesh/include/fastMesh.h:11-57 (class fastMesh).  The handle owns one device allocation on

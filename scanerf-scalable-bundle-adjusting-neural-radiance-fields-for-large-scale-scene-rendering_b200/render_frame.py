@@ -164,3 +164,18 @@ def render_frame(ts, H, W, K, c2w, **kw):
     rays_o, rays_d = pinhole_rays(H, W, K, c2w, ts.device)
     d, s, z, t = render_rays(ts, rays_o, rays_d, **kw)
     return d.reshape(H, W, 3), s.reshape(H, W, 3), z.reshape(H, W, 1), t.reshape(H, W, 1)
+
+
+@torch.no_grad()
+def evaluate_frames(ts, Ks, c2ws, images, H, W, masks=None, **render_kw):
+    """rendering.py's `val` mode over a TileSet: each camera (Ks [V,3,3], c2ws [V,3,4] on the device) rendered with
+    render_frame(**render_kw), rgb = clamp(diffuse + specular, 0, 1) as the training path composes it, and scored against
+    `images` [V,H,W,3] (uint8 or float32 in [0, 1]) within `masks` [V,H,W(,1)] bool or None.
+    -> metrics.image_metrics' per-view {"mse", "psnr", "ssim", "count"} [V] plus "mean_mse", "mean_psnr", "mean_ssim", all
+    device tensors.  With adaptive=False nothing synchronises with the host."""
+    from metrics import image_metrics, with_means
+    pred = torch.empty(len(c2ws), H, W, 3, dtype=torch.float32, device=ts.device)
+    for k in range(len(c2ws)):
+        d, s, _, _ = render_frame(ts, H, W, Ks[k], c2ws[k], **render_kw)
+        torch.clamp(d + s, 0, 1, out=pred[k])
+    return with_means(image_metrics(pred, images, masks))

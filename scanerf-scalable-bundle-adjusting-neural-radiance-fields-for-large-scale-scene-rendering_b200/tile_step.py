@@ -217,24 +217,50 @@ class TileStep:
             return self.poses.rays(locs)
 
     @torch.no_grad()
+    def render_image(self, view, H, W, stride=1, chunk=1 << 16):
+        """TILE.render_image_rays (tile.py:724-756): every `stride`-th pixel of camera `view` rendered in chunks of `chunk`
+        rays with the inference path.  -> (color [h, w, 3], depth [h, w, 1]), h = ceil(H / stride), w = ceil(W / stride).
+        No host synchronisation."""
+        rays_o, rays_d = self.full_image_rays(view, H, W, stride)
+        n = rays_o.shape[0]
+        color = torch.zeros(n, 3, device=self.device)
+        depth = torch.zeros(n, 1, device=self.device)
+        for b in range(0, n, chunk):
+            out, ok = self.render_rays(rays_o[b:b + chunk].contiguous(), rays_d[b:b + chunk].contiguous(), None, INFERENCE)
+            if ok:
+                color[b:b + chunk] = out["pred_color"]
+                depth[b:b + chunk] = out["pred_depth"]
+        h, w = (H + stride - 1) // stride, (W + stride - 1) // stride
+        return color.reshape(h, w, 3), depth.reshape(h, w, 1)
+
+    @torch.no_grad()
+    def evaluate(self, views, images, masks=None, H=None, W=None):
+        """Held-out view evaluation (tile.py:810-864): renders each camera of `views` (ints) at H x W (default: the images'
+        size) and scores it against `images` [V,H,W,3] (uint8 or float32 in [0, 1], on the device) within `masks`
+        [V,H,W(,1)] bool or None.  -> metrics.image_metrics' per-view {"mse", "psnr", "ssim", "count"} [V] plus their
+        means "mean_mse", "mean_psnr", "mean_ssim", all device tensors; nothing synchronises until a value is read."""
+        from metrics import image_metrics, with_means
+        H = images.shape[-3] if H is None else H
+        W = images.shape[-2] if W is None else W
+        pred = torch.empty(len(views), H, W, 3, device=self.device)
+        for k, v in enumerate(views):
+            pred[k] = self.render_image(int(v), H, W)[0]
+        return with_means(image_metrics(pred, images, masks))
+
+    @torch.no_grad()
     def render_shared_depth(self, H, W, batch=1 << 16):
         """TILE.render_shared_depth: for every overlap camera of this tile whose centre lies INSIDE the tile's (doubled) box,
         the half-resolution depth map of the tile's current field.  -> (global camera ids [k], maps [k, H//2, W//2])."""
         if self.consensus is None:
             raise RuntimeError("render_shared_depth: enable_consensus() first (the overlap cameras come from the exchange)")
         center, half = self.featureGrid.bbox_center, self.featureGrid.bbox_size / 2.0
+        cam_centres = self.poses.c2w()[:, :, 3]                                            # = the rays' origin
         ids, maps = [], []
         for i in torch.nonzero(self.consensus.overlap_flags)[:, 0].tolist():
-            rays_o, rays_d = self.full_image_rays(i, H, W, stride=2)
-            if not bool(torch.all(torch.abs(rays_o[0] - center) < half / 2.0)):           # tile.py:445-448
+            if not bool(torch.all(torch.abs(cam_centres[i] - center) < half / 2.0)):       # tile.py:445-448
                 continue
-            depth = torch.zeros(rays_o.shape[0], 1, device=self.device)
-            for b in range(0, rays_o.shape[0], batch):                                     # TILE.render_depth_rays, tile.py:714-722
-                out, ok = self.render_rays(rays_o[b:b + batch].contiguous(), rays_d[b:b + batch].contiguous(), None, INFERENCE)
-                if ok:
-                    depth[b:b + batch] = out["pred_depth"]
             ids.append(int(self.camera_ids[i]))
-            maps.append(depth.reshape((H + 1) // 2, (W + 1) // 2))
+            maps.append(self.render_image(i, H, W, stride=2, chunk=batch)[1][..., 0])      # TILE.render_depth_rays, tile.py:714-722
         if not ids:
             return torch.zeros(0, dtype=torch.long, device=self.device), torch.zeros(0, (H + 1) // 2, (W + 1) // 2, device=self.device)
         return torch.tensor(ids, dtype=torch.long, device=self.device), torch.stack(maps)
